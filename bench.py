@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path through the C ABI
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                   # also saves the last timed step's field and markers as .npy
 
 A "step" is one full timestep input_dt of the reference time loop (src/pic1dp.F90:79-93): 2 RK substeps, each
 = gather + push(x, w, v) + wrap + deposit, plus 2 field solves and 2 density all-reduces.  1 particle-step = 1 marker
@@ -31,11 +32,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (no __pycache__ from the imports below)
 
 BYTES_IRK1 = 56   # read x,v,w,p; write x',v',w'            (SURVEY.md 8d / DESIGN.md)
 BYTES_IRK2 = 80   # read mid x,v,w + start x,v,w + p; write x,v,w
 BYTES_STEP = BYTES_IRK1 + BYTES_IRK2
 OUTPUT_EVERY = 10  # input_output_interval / input_dt = 0.5 / 0.05
+DUMP_MARKERS = 1 << 20  # --dump-outputs marker sample: x, v, p, w x 8 B x 2^20 = 32 MiB
 
 
 def parse():
@@ -71,6 +74,10 @@ def parse():
     ap.add_argument("--cpu-markers", type=float, default=2e7, help="markers of the bounded CPU sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed on rank 0 to DIR/<name>.npy (float64): the "
+                         "field arrays and a fixed sample of %d markers -- to compare two builds output for output"
+                         % DUMP_MARKERS)
     args = ap.parse_args()
     if args.nx is None:
         args.nx = 8192 if args.scaling == "strong" else 1024
@@ -177,6 +184,19 @@ def measured_peak():
         return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def dump_outputs(g, out_dir):
+    """What a caller of the timed path receives after its last step: the field (get_field) and the markers
+    (get_markers).  Markers beyond DUMP_MARKERS are sampled at fixed seeded indices, the same ones for the same marker
+    count, so that two builds run with the same arguments compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in g.get_field().items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    n = g.get_markers_ptr(0)
+    idx = slice(None) if n <= DUMP_MARKERS else np.sort(np.random.default_rng(0).choice(n, DUMP_MARKERS, replace=False))
+    for k in ("x", "v", "p", "w"):   # one array at a time: the whole set is 32 B per marker of host memory
+        np.save(os.path.join(out_dir, k + ".npy"), g.get_markers(0, want=(k,))[k][idx])
 
 
 def cpu_reference_run(nx, n_markers, steps, warmup, nthreads, repeats=1):
@@ -486,6 +506,8 @@ def main():
         dist.all_gather_object(rows, (stamps.astype(np.int64), int(last)))
         if rank == 0:
             p2p_trace = analyse_trace(rows, 2 * args.steps, cap)
+    if args.dump_outputs and rank == 0:   # before the regions below reload and advance the markers
+        dump_outputs(g, args.dump_outputs)
 
     # ---- sustained: the same loop for >= 500 further steps (graph replay, no per-launch events).  Runs AFTER the
     # driver-length e2e region below, so that `value` and `e2e` are both measured from the same (cool) state and

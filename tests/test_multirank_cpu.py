@@ -162,6 +162,42 @@ def test_bench_trace_analysis_separates_skew_from_exchange_floor():
     assert abs(t["per_step_cost_us"]["skew_worst_rank"] - 2 * skews[1:].max(axis=1).mean() / 1e3) < 1e-9
 
 
+def test_bench_dump_outputs_writes_field_and_a_fixed_marker_sample(tmp_path):
+    """bench.py --dump-outputs: the field arrays whole, the markers at the same seeded indices on every run, in float64,
+    within 64 MB; a marker set no larger than the sample is written whole."""
+    sys.path.insert(0, ROOT)
+    import bench
+
+    class FakeGpu:   # the Pic1dGpu calls dump_outputs makes
+        def __init__(self, n):
+            self.mk = {k: np.arange(n, dtype=np.float64) + i for i, k in enumerate("xvpw")}
+
+        def get_field(self):
+            return dict(electric=np.full(16, 1.0), chargeden=np.full(16, 2.0), mode_re=np.ones(1), mode_im=np.zeros(1))
+
+        def get_markers_ptr(self, isp):
+            return self.mk["x"].size
+
+        def get_markers(self, isp, want):
+            return {k: self.mk[k].copy() for k in want}
+
+    n = 3 * bench.DUMP_MARKERS + 7
+    bench.dump_outputs(FakeGpu(n), str(tmp_path / "a"))
+    bench.dump_outputs(FakeGpu(n), str(tmp_path / "b"))
+    names = ("electric", "chargeden", "mode_re", "mode_im", "x", "v", "p", "w")
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(k + ".npy" for k in names)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 << 20
+    a = {k: np.load(tmp_path / "a" / (k + ".npy")) for k in names}
+    b = {k: np.load(tmp_path / "b" / (k + ".npy")) for k in names}
+    assert all(a[k].dtype == np.float64 and np.array_equal(a[k], b[k]) for k in names)
+    assert np.array_equal(a["electric"], np.full(16, 1.0))
+    x = a["x"]
+    assert x.size == bench.DUMP_MARKERS and np.all(np.diff(x) > 0) and x[-1] < n   # distinct indices, in order
+    assert all(np.array_equal(a[k], x + i) for i, k in enumerate("xvpw"))            # one index set for all four
+    bench.dump_outputs(FakeGpu(1000), str(tmp_path / "c"))
+    assert np.array_equal(np.load(tmp_path / "c" / "w.npy"), np.arange(1000) + 3.0)
+
+
 def test_bench_rank_seeds_are_valid_kiss64_states_and_rank_dependent():
     sys.path.insert(0, ROOT)
     import bench
