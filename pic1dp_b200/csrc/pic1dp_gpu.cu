@@ -116,6 +116,7 @@ struct pic1dp_gpu {
   std::vector<int> lt_irk;          // irk of each recorded pair
   Species sp[PIC1DP_MAX_SPECIES];
   double *d_E = nullptr, *d_rho = nullptr, *d_mre = nullptr, *d_mim = nullptr;
+  double *d_E_start = nullptr;   // field of step()'s first substep, kept for the recomputed midpoint (ParticleArgs::E_start)
   double *d_Fre = nullptr, *d_Fim = nullptr, *d_ginv = nullptr;
   double *d_partial = nullptr, *d_red = nullptr, *d_energy = nullptr;
   void *d_kiss_tab = nullptr;   // KissTables: jump-ahead tables of the device KISS64 (allocated on first use)
@@ -148,6 +149,10 @@ struct pic1dp_gpu {
   int tma_smem[2] = {0, 0};  // dynamic shared memory of the TMA kernels, irk = 1, 2
   bool use_cpa[2] = {false, false};  // cp.async-staged kernel per substep
   int cpa_smem[2] = {0, 0};
+  // step() runs the recomputed-midpoint kernel pair (k_push with RC = true): substep 1 stores only w', substep 2 rebuilds
+  // x' and v' from the start-of-step state and E_start.  40 + 64 instead of 56 + 80 bytes per marker and step.
+  bool recompute = false;
+  int smem_rc = 0;   // dynamic shared memory of the RC irk = 2 kernel (second field table)
   bool partial_valid = false;  // a fused push has already deposited into d_partial
   int nred = 1;
   ncclComm_t comm = nullptr;
@@ -356,7 +361,7 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
     }
     if (S.p) cudaFree(S.p);
   }
-  double *bufs[] = {h->d_E, h->d_rho, h->d_mre, h->d_mim, h->d_Fre, h->d_Fim, h->d_ginv, h->d_partial, h->d_red, h->d_energy,
+  double *bufs[] = {h->d_E, h->d_E_start, h->d_rho, h->d_mre, h->d_mim, h->d_Fre, h->d_Fim, h->d_ginv, h->d_partial, h->d_red, h->d_energy,
                     h->d_diag_part, h->d_diag_sums, h->d_hist, h->d_hist_out, h->d_dist_part, h->d_hist_all};
   for (double *b : bufs)
     if (b) cudaFree(b);
@@ -481,15 +486,28 @@ static int create_impl(pic1dp_gpu_t *h) {
   h->cfg = (p.deltaf == 1 && p.linear == 0 && p.iptclshape >= 3) ? 1 : -1;
   {
     int per_sm_min = 1 << 30;
+    // recomputed-midpoint pair of step(): its irk = 2 kernel holds the field of both substeps.  Used where the rest of the
+    // substep is as in the reference's shape-4 loop (no compute_shape_x between the substeps reads the midpoint x) and
+    // where the second table keeps the residency of the stored-midpoint kernels (not at nx = 8192 with the pair grid).
+    h->smem_rc = h->smem_push + 8 * ((nx + 1) & ~1);
+    bool rc_ok = p.fuse != 0 && p.iptclshape == 4 && (size_t)h->smem_rc <= max_smem;
+    int per_sm_rc = 1 << 30;
     const int cfgs[6] = {-1, 1, 9, 25, 33, 57};
     for (int irk2 = 0; irk2 < 2; irk2++)
       for (int fused = 0; fused < 2; fused++)
         for (int ci = 0; ci < 6; ci++) {
-          PushKernel k = pick_push(p.iptcldist, dep, irk2 == 1, fused == 1, cfgs[ci]);
+          PushKernel k = pick_push(p.iptcldist, dep, irk2 == 1, fused == 1, cfgs[ci], false);
           CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, h->smem_push));
           int per_sm = 0;
           CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, h->threads, h->smem_push));
           if (fused && per_sm < per_sm_min) per_sm_min = per_sm;
+          if (fused && rc_ok) {
+            const int sm = irk2 ? h->smem_rc : h->smem_push;
+            k = pick_push(p.iptcldist, dep, irk2 == 1, true, cfgs[ci], true);
+            CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
+            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, h->threads, sm));
+            if (per_sm < per_sm_rc) per_sm_rc = per_sm;
+          }
         }
     if (per_sm_min < 1) per_sm_min = 1;
     // TMA-pipelined variant (2-stage ring of 2*threads markers): usable when it reaches the same residency.
@@ -549,6 +567,8 @@ static int create_impl(pic1dp_gpu_t *h) {
       return PIC1DP_EUNSUPPORTED;
     }
     h->grid = h->nsm * per_sm_min;  // persistent grid: every CTA resident, private grid per CTA
+    // the RC pair replaces the direct kernels only (the TMA / cp.async rings keep the stored midpoint)
+    h->recompute = rc_ok && per_sm_rc >= per_sm_min && !h->use_tma[0] && !h->use_tma[1] && !h->use_cpa[0] && !h->use_cpa[1];
   }
   CK(cudaFuncSetAttribute(pick_deposit(dep, true), cudaFuncAttributeMaxDynamicSharedMemorySize,
                           h->smem_dep > 0 ? h->smem_dep : 8));
@@ -573,6 +593,7 @@ static int create_impl(pic1dp_gpu_t *h) {
   // ---- grid ----
   h->nred = (p.iptclshape <= 2) ? p.nspecies : 1;
   CK(cudaMalloc(&h->d_E, (size_t)nx * 8));
+  CK(cudaMalloc(&h->d_E_start, (size_t)nx * 8));
   CK(cudaMalloc(&h->d_rho, (size_t)nx * 8));
   CK(cudaMalloc(&h->d_mre, (size_t)M * 8));
   CK(cudaMalloc(&h->d_mim, (size_t)M * 8));
@@ -1009,6 +1030,8 @@ static void fill_particle_args(pic1dp_gpu_t *h, int s, ParticleArgs &a) {
   memset(&a, 0, sizeof(a));
   a.p = S.p;
   a.E = h->d_E;
+  a.E_start = h->d_E_start;
+  a.dth = 0.5 * p.dt;
   a.partial = h->d_partial + (size_t)s * h->grid * p.nx;
   a.noob = h->d_noob;
   a.dep_wmax_hi = h->d_wmax_hi + s;
@@ -1173,8 +1196,9 @@ int pic1dp_gpu_solve_field(pic1dp_gpu_t *h) {
   return solve_field_impl(h, false);
 }
 
-int pic1dp_gpu_push(pic1dp_gpu_t *h, int32_t irk) {
-  if (!h || (irk != 1 && irk != 2)) { if (h) h->err = "push: irk must be 1 or 2"; return PIC1DP_EINVAL; }
+// recompute: the RC kernel pair of step() (h->recompute).  Its irk = 1 leaves the midpoint set's x and v unwritten, so
+// it must be followed by the RC irk = 2 before anything reads the markers; the public per-substep push stores them.
+static int push_impl(pic1dp_gpu_t *h, int32_t irk, bool recompute) {
   int rc = check_loaded(h, "push");
   if (rc) return rc;
   CK(cudaSetDevice(h->p.device));
@@ -1191,7 +1215,7 @@ int pic1dp_gpu_push(pic1dp_gpu_t *h, int32_t irk) {
     if (irk == 1) {
       S.bak = S.cur;       // VecCopy x,v,w -> *_bak (:181-187) without moving a byte
       out = S.cur ^ 1;
-      a.dt = 0.5 * p.dt;   // :179
+      a.dt = a.dth;        // 0.5 * dt, :179
     } else {
       out = S.bak;         // overwrite the start-of-step set
       a.dt = p.dt;         // :192
@@ -1226,8 +1250,11 @@ int pic1dp_gpu_push(pic1dp_gpu_t *h, int32_t irk) {
     } else if (fused && h->use_tma[irk - 1] && cfg > 0) {
       PushKernel k = pick_tma(p.iptcldist, h->dep, irk == 2, cfg);
       k<<<h->grid, 512, h->tma_smem[irk - 1], h->stream>>>(a);
+    } else if (recompute) {
+      PushKernel k = pick_push(p.iptcldist, h->dep, irk == 2, true, cfg, true);
+      k<<<h->grid, h->threads, irk == 2 ? h->smem_rc : h->smem_push, h->stream>>>(a);
     } else {
-      PushKernel k = pick_push(p.iptcldist, h->dep, irk == 2, fused, cfg);
+      PushKernel k = pick_push(p.iptcldist, h->dep, irk == 2, fused, cfg, false);
       k<<<h->grid, h->threads, h->smem_push, h->stream>>>(a);
     }
     CKL(h);
@@ -1239,6 +1266,11 @@ int pic1dp_gpu_push(pic1dp_gpu_t *h, int32_t irk) {
   }
   h->partial_valid = fused;
   return PIC1DP_OK;
+}
+
+int pic1dp_gpu_push(pic1dp_gpu_t *h, int32_t irk) {
+  if (!h || (irk != 1 && irk != 2)) { if (h) h->err = "push: irk must be 1 or 2"; return PIC1DP_EINVAL; }
+  return push_impl(h, irk, false);
 }
 
 int pic1dp_gpu_launch_timing_start(pic1dp_gpu_t *h) {
@@ -1268,7 +1300,7 @@ int pic1dp_gpu_launch_timing_stop(pic1dp_gpu_t *h, double ms_sum[2], int64_t lau
 // one timestep with individual launches: src/pic1dp.F90:79-90
 static int step_direct(pic1dp_gpu_t *h) {
   for (int irk = 1; irk <= 2; irk++) {
-    int rc = pic1dp_gpu_push(h, irk);
+    int rc = push_impl(h, irk, h->recompute);
     if (rc) return rc;
     if (h->p.iptclshape < 4) {
       rc = pic1dp_gpu_compute_shape_x(h);
@@ -1364,7 +1396,7 @@ int pic1dp_gpu_profile_step(pic1dp_gpu_t *h, float ms[6]) {
   int e = 0;
   CK(cudaEventRecord(h->pev[e++], h->stream));
   for (int irk = 1; irk <= 2; irk++) {
-    int rc = pic1dp_gpu_push(h, irk);
+    int rc = push_impl(h, irk, h->recompute);   // the kernels of step()
     if (rc) return rc;
     CK(cudaEventRecord(h->pev[e++], h->stream));
     if (h->p.iptclshape < 4) {

@@ -10,26 +10,25 @@ namespace pic1dp {
 namespace {
 constexpr int DIST = PIC1DP_DIST;
 
-template <bool IRK2, int CFG>
+template <bool IRK2, int CFG, bool RC>
 PushKernel pick_dep(int dep) {
   switch (dep) {
-    case DEP_SMEM_ATOMIC: return k_push<DIST, IRK2, DEP_SMEM_ATOMIC, true, CFG>;
-    case DEP_GLOBAL_RED: return k_push<DIST, IRK2, DEP_GLOBAL_RED, true, CFG>;
-    case DEP_FIXED: return k_push<DIST, IRK2, DEP_FIXED, true, CFG>;
-    default: return k_push<DIST, IRK2, DEP_WARP_PRIVATE, true, CFG>;
+    case DEP_SMEM_ATOMIC: return k_push<DIST, IRK2, DEP_SMEM_ATOMIC, true, CFG, RC>;
+    case DEP_GLOBAL_RED: return k_push<DIST, IRK2, DEP_GLOBAL_RED, true, CFG, RC>;
+    case DEP_FIXED: return k_push<DIST, IRK2, DEP_FIXED, true, CFG, RC>;
+    default: return k_push<DIST, IRK2, DEP_WARP_PRIVATE, true, CFG, RC>;
   }
 }
-template <bool IRK2>
-PushKernel pick_cfg(int dep, bool fused, int cfg) {
-  if (!fused) return k_push<DIST, IRK2, DEP_SMEM_ATOMIC, false, -1>;
-  if (cfg == 1) return pick_dep<IRK2, 1>(dep);
-  if (cfg == 9) return pick_dep<IRK2, 9>(dep);
-  if (cfg == 25) return pick_dep<IRK2, 25>(dep);
+template <bool IRK2, bool RC>
+PushKernel pick_cfg(int dep, int cfg) {
+  if (cfg == 1) return pick_dep<IRK2, 1, RC>(dep);
+  if (cfg == 9) return pick_dep<IRK2, 9, RC>(dep);
+  if (cfg == 25) return pick_dep<IRK2, 25, RC>(dep);
 #if PIC1DP_DIST == 2 || PIC1DP_DIST == 3
-  if (cfg == 33) return pick_dep<IRK2, 33>(dep);   // PIC1DP_ARITH_TOLERANCE
-  if (cfg == 57) return pick_dep<IRK2, 57>(dep);
+  if (cfg == 33) return pick_dep<IRK2, 33, RC>(dep);   // PIC1DP_ARITH_TOLERANCE
+  if (cfg == 57) return pick_dep<IRK2, 57, RC>(dep);
 #endif
-  return pick_dep<IRK2, -1>(dep);
+  return pick_dep<IRK2, -1, RC>(dep);
 }
 template <bool IRK2, int CFG>
 PushKernel pick_tma_dep(int dep) {
@@ -52,8 +51,10 @@ PushKernel pick_cpa_dep(int dep) {
 #define PIC1DP_CAT2(a, b) a##b
 #define PIC1DP_CAT(a, b) PIC1DP_CAT2(a, b)
 
-PushKernel PIC1DP_CAT(pick_push_dist, PIC1DP_DIST)(int dep, bool irk2, bool fused, int cfg) {
-  return irk2 ? pick_cfg<true>(dep, fused, cfg) : pick_cfg<false>(dep, fused, cfg);
+PushKernel PIC1DP_CAT(pick_push_dist, PIC1DP_DIST)(int dep, bool irk2, bool fused, int cfg, bool rc) {
+  if (!fused) return irk2 ? k_push<DIST, true, DEP_SMEM_ATOMIC, false, -1> : k_push<DIST, false, DEP_SMEM_ATOMIC, false, -1>;
+  if (rc) return irk2 ? pick_cfg<true, true>(dep, cfg) : pick_cfg<false, true>(dep, cfg);
+  return irk2 ? pick_cfg<true, false>(dep, cfg) : pick_cfg<false, false>(dep, cfg);
 }
 PushKernel PIC1DP_CAT(pick_tma_dist, PIC1DP_DIST)(int dep, bool irk2, int cfg) {
   if (cfg == 25) return irk2 ? pick_tma_dep<true, 25>(dep) : pick_tma_dep<false, 25>(dep);

@@ -11,9 +11,10 @@ namespace pic1dp {
 typedef void (*PushKernel)(const ParticleArgs);
 
 // cfg: -1 generic (switches read at run time), 1 = delta-f nonlinear shape 3/4, 9 = same with power-of-two
-// divisors, 25 = same with T = T2 = m = 1 (the reference default input); + 32 = TOLERANCE arithmetic (w path only)
-#define PIC1DP_DECLARE_DIST(D)                                              \
-  PushKernel pick_push_dist##D(int dep, bool irk2, bool fused, int cfg);    \
+// divisors, 25 = same with T = T2 = m = 1 (the reference default input); + 32 = TOLERANCE arithmetic (w path only).
+// rc: the recomputed-midpoint forms of step() (fused only; k_push with RC = true)
+#define PIC1DP_DECLARE_DIST(D)                                                       \
+  PushKernel pick_push_dist##D(int dep, bool irk2, bool fused, int cfg, bool rc);    \
   PushKernel pick_tma_dist##D(int dep, bool irk2, int cfg);                 \
   PushKernel pick_cpa_dist##D(int dep, bool irk2, int cfg);
 PIC1DP_DECLARE_DIST(0)
@@ -22,12 +23,12 @@ PIC1DP_DECLARE_DIST(2)
 PIC1DP_DECLARE_DIST(3)
 #undef PIC1DP_DECLARE_DIST
 
-inline PushKernel pick_push(int dist, int dep, bool irk2, bool fused, int cfg) {
+inline PushKernel pick_push(int dist, int dep, bool irk2, bool fused, int cfg, bool rc) {
   switch (dist) {
-    case 1: return pick_push_dist1(dep, irk2, fused, cfg);
-    case 2: return pick_push_dist2(dep, irk2, fused, cfg);
-    case 3: return pick_push_dist3(dep, irk2, fused, cfg);
-    default: return pick_push_dist0(dep, irk2, fused, cfg);
+    case 1: return pick_push_dist1(dep, irk2, fused, cfg, rc);
+    case 2: return pick_push_dist2(dep, irk2, fused, cfg, rc);
+    case 3: return pick_push_dist3(dep, irk2, fused, cfg, rc);
+    default: return pick_push_dist0(dep, irk2, fused, cfg, rc);
   }
 }
 // TMA-pipelined kernels (delta-f nonlinear, fused): cfg in {1, 9, 25}

@@ -1,4 +1,8 @@
 #include "../../pic1dp_b200/csrc/particle_kernels.cuh"
 using namespace pic1dp;
-template __global__ void pic1dp::k_push<3, false, DEP_SMEM_ATOMIC, true, 25>(const ParticleArgs);
-template __global__ void pic1dp::k_push<3, true, DEP_SMEM_ATOMIC, true, 25>(const ParticleArgs);
+// the flagship instantiations (bump-on-tail, default fixed-point deposit, unit constants): the stored-midpoint pair of
+// the per-substep entry points, then the recomputed-midpoint pair of step()
+template __global__ void pic1dp::k_push<3, false, DEP_FIXED, true, 25>(const ParticleArgs);
+template __global__ void pic1dp::k_push<3, true, DEP_FIXED, true, 25>(const ParticleArgs);
+template __global__ void pic1dp::k_push<3, false, DEP_FIXED, true, 25, true>(const ParticleArgs);
+template __global__ void pic1dp::k_push<3, true, DEP_FIXED, true, 25, true>(const ParticleArgs);

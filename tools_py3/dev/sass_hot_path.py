@@ -26,4 +26,4 @@ for cub in sys.argv[1:]:
                 hot=[(x,y) for x,y in hot if not (t<=x<=a)]
         c=collections.Counter((s.split()[1] if s.startswith('@') else s.split()[0]).split('.')[0] for a,s in hot)
         dp=sum(v for k,v in c.items() if k in('DFMA','DMUL','DADD','DSETP'))
-        print(name[17:40],'hot',len(hot),'dp',dp,dict(c.most_common(10)))
+        print(name[17:44],'hot',len(hot),'dp',dp,'LDL/STL',c['LDL']+c['STL'],dict(c.most_common(10)))
