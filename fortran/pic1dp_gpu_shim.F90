@@ -117,6 +117,18 @@ interface
     integer(c_int64_t), intent(inout) :: seeds(4)
     integer(c_int64_t), value :: n
   end function
+  integer(c_int) function pic1dp_gpu_load_markers_superkiss64(handle, isp, np, nlocal, nparticle_init, seeds, iseed, &
+      v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin) bind(c, name = 'pic1dp_gpu_load_markers_superkiss64')
+    import :: c_ptr, c_int, c_int32_t, c_int64_t, c_double
+    type(c_ptr), value :: handle
+    integer(c_int32_t), value :: isp, init_nmode
+    integer(c_int64_t), value :: np, nlocal, nparticle_init
+    integer(c_int64_t), intent(inout) :: seeds(20635)   ! multirand_seeds(0:20634), same bits as the C uint64_t
+    integer(c_int32_t), intent(inout) :: iseed
+    real(c_double), value :: v_max
+    real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
+    integer(c_int32_t), intent(in) :: init_mode(*)
+  end function
   integer(c_int) function pic1dp_gpu_output_all(handle, nx_opd, nv_opd, v_max, scalars, dist) &
       bind(c, name = 'pic1dp_gpu_output_all')
     import :: c_ptr, c_int, c_int32_t, c_double
@@ -236,6 +248,7 @@ public :: pic1dp_gpu_p2p_export, pic1dp_gpu_p2p_import, pic1dp_gpu_output_field,
 public :: pic1dp_gpu_compute_dist_pertb_abs_v, pic1dp_gpu_particle_merge, pic1dp_gpu_particle_remove
 public :: pic1dp_gpu_particle_split
 public :: pic1dp_gpu_load_markers_kiss64, pic1dp_host_kiss64_jump, pic1dp_gpu_output_all
+public :: pic1dp_gpu_load_markers_superkiss64
 
 end module pic1dp_gpu
 
@@ -378,6 +391,29 @@ global_ierr = pic1dp_host_kiss64_jump(seeds, 2_c_int64_t * int(nlocal, c_int64_t
 CHKERRQ(global_ierr)
 multirand_seeds(0 : 3) = seeds(1 : 4)
 end subroutine gpu_particle_load_kiss64
+
+! particle_load with input_multirand_al_int = 3 (SuperKISS64, the default input): no marker-sized host-to-device copy.
+! Call in place of the two multirand_real_array calls (src/pic1dp_particle.F90:180, :222) AFTER multirand_init
+! (:159-160).  The device generates exactly the 2 * nlocal numbers those calls would have drawn and returns the advanced
+! state (table, carry, LCG, xorshift and table position), which is copied back into the multirand module so that later
+! draws (particle_remove, particle_split) continue the same stream.  nlocal = particle_ip_high - particle_ip_low.
+subroutine gpu_particle_load_superkiss64(ispecies, np, nlocal)
+use multirand, only : multirand_seeds, multirand_iseed
+implicit none
+#include "finclude/petsc.h90"
+PetscInt, intent(in) :: ispecies, np, nlocal
+integer(c_int64_t) :: seeds(20635)
+integer(c_int32_t) :: iseed
+seeds(1 : 20635) = multirand_seeds(0 : 20634)
+iseed = int(multirand_iseed, c_int32_t)
+global_ierr = pic1dp_gpu_load_markers_superkiss64(gpu_handle, int(ispecies - 1, c_int32_t), int(np, c_int64_t), &
+  int(nlocal, c_int64_t), int(input_species_nparticle_init(ispecies), c_int64_t), seeds, iseed, &
+  real(input_v_max, c_double), int(input_init_nmode, c_int32_t), int(input_init_mode, c_int32_t), &
+  real(input_init_mode_cos, c_double), real(input_init_mode_sin, c_double))
+CHKERRQ(global_ierr)
+multirand_seeds(0 : 20634) = seeds(1 : 20635)
+multirand_iseed = iseed
+end subroutine gpu_particle_load_superkiss64
 
 ! before output_all / particle_optimize (src/pic1dp_output.F90:128-150, :228-237): device -> host Vecs
 subroutine gpu_particle_refresh_host(ispecies, vx, vv, vp, vw)

@@ -80,6 +80,7 @@ struct Input {
   double input_output_interval = 0.5;
   // placement / implementation (not in the reference)
   int ngpus = 1, deposit_mode = 0, field_mode = 0, fuse = 1;
+  int device_rng = 1;  // 1: SuperKISS64 uniform-v markers are generated on the device (same bits); 0: host stream
   std::string out = "pic1dp_energy.txt";
   std::string petsc_out;          // when set: also write the reference's binary output file (pic1dp.out layout)
   int input_nv = 128, input_nx_opd = 64, input_nv_opd = 64;  // src/pic1dp_input.F90:131, :253-256
@@ -150,6 +151,7 @@ static bool parse(Input &in, int argc, char **argv) {
     else if (k == "split_dv_sig_frac") in.input_split_dv_sig_frac = d;
     else if (k == "markers_out") in.markers_out = v;
     else if (k == "imarker") in.input_imarker = (int)d;
+    else if (k == "device_rng") in.device_rng = (int)d;
     else return false;
   }
   return true;
@@ -426,10 +428,12 @@ static void particle_init(Rank &r, const uint8_t *uid) {
   r.field_mode_im.resize(in.input_nmode);
 }
 
-// particle_load (src/pic1dp_particle.F90:145-269), uniform-v markers (input_imarker = 2): the RNG (multirand, a
-// sequential generator) runs on the host exactly as in the reference -- rand_v is drawn first (:180), then rand_x
-// (:222) -- and the loader arithmetic (:181-237, :260-263) runs on the device (pic1dp_gpu_load_markers), so only the
-// two uniform streams cross PCIe.
+// particle_load (src/pic1dp_particle.F90:145-269): the RNG (multirand, a sequential generator) keeps the reference's
+// draw order -- the whole local array for v first (:174 / :180), then for x (:222) -- and the loader arithmetic
+// (:172-237, :260-263) runs on the device.  With SuperKISS64 (al_int = 3, the default) and uniform-v markers
+// (input_imarker = 2) the device also generates both streams from the generator's state and hands the advanced state
+// back (pic1dp_gpu_load_markers_superkiss64), so nothing marker-sized crosses PCIe; otherwise (or with device_rng=0)
+// the host draws them and only the two uniform streams cross PCIe (pic1dp_gpu_load_markers).  Same markers either way.
 static void particle_load(Rank &r) {
   const pic1dp_input::Input &in = *r.in;
   multirand::Generator &rng = r.rng;
@@ -437,6 +441,20 @@ static void particle_load(Rank &r) {
     fprintf(stderr, "[%d][multirand_selftest] Warning: unexpected head sequence.\n", r.g.global_mype);
   rng.init(in.input_multirand_al_int, in.input_multirand_seed_type, r.g.global_mype, in.input_multirand_warmup);
   const int64_t n = r.particle_ip_high - r.particle_ip_low;
+  // unload not used particles (:240-248): the tail of the local array stays free for particle_split
+  const int64_t ninit = in.input_species_nparticle_init > 0 ? in.input_species_nparticle_init : in.input_nparticle_max;
+  int64_t nparticle_unload = (in.input_nparticle_max - ninit) / r.g.global_npe;
+  if (r.g.global_mype == 0) nparticle_unload += (in.input_nparticle_max - ninit) % r.g.global_npe;
+  r.particle_np = n - nparticle_unload;
+  if (in.input_imarker == 2 && in.input_multirand_al_int == 3 && in.device_rng) {
+    int32_t iseed = rng.iseed;
+    r.g.global_ierr = pic1dp_gpu_load_markers_superkiss64(r.h, 0, r.particle_np, n, ninit, rng.s.data(), &iseed,
+                                                          in.input_v_max, in.input_init_nmode, in.input_init_mode,
+                                                          in.input_init_mode_cos, in.input_init_mode_sin);
+    CHKERRQ(r.g, r.h);
+    rng.iseed = iseed;
+    return;
+  }
   r.v.resize(n);
   r.x.resize(n);
   if (in.input_imarker == 1)
@@ -444,11 +462,6 @@ static void particle_load(Rank &r) {
   else
     rng.real_array(r.v.data(), n);  // :180  (the whole local array is drawn, used or not)
   rng.real_array(r.x.data(), n);  // :222
-  // unload not used particles (:240-248): the tail of the local array stays free for particle_split
-  const int64_t ninit = in.input_species_nparticle_init > 0 ? in.input_species_nparticle_init : in.input_nparticle_max;
-  int64_t nparticle_unload = (in.input_nparticle_max - ninit) / r.g.global_npe;
-  if (r.g.global_mype == 0) nparticle_unload += (in.input_nparticle_max - ninit) % r.g.global_npe;
-  r.particle_np = n - nparticle_unload;
   if (in.input_imarker == 1)
     r.g.global_ierr = pic1dp_gpu_load_markers_maxwellian(r.h, 0, r.particle_np, ninit, r.v.data(), r.x.data(),
                                                          in.input_init_nmode, in.input_init_mode,

@@ -235,8 +235,8 @@ int pic1dp_gpu_load_markers_maxwellian(pic1dp_gpu_t *h, int32_t isp, int64_t np,
  * (LCG, xorshift, multiply-with-carry) to its chunk in O(log offset) and then runs the sequential generator; the
  * uniforms are INT2REAL64 of its outputs (:49).  Afterwards the host advances its own state with
  * pic1dp_host_kiss64_jump(seeds, 2 * nlocal * nspecies) so that later draws (particle_remove, particle_split)
- * continue the same stream.  SuperKISS64 (al_int = 3: lag-20632 carry chain, no practical jump) and MT19937-64
- * streams keep coming from the host through load_markers.
+ * continue the same stream.  SuperKISS64 (al_int = 3) has its own loader below; MT19937-64 streams keep coming from
+ * the host through load_markers.
  */
 int pic1dp_gpu_load_markers_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nparticle_init,
                                    const uint64_t seeds[4], int64_t offset_v, int64_t offset_x, double v_max,
@@ -252,6 +252,24 @@ int pic1dp_gpu_load_markers_counter(pic1dp_gpu_t *h, int32_t isp, int64_t np, in
                                     int64_t first_index, double v_max, int32_t init_nmode, const int32_t *init_mode,
                                     const double *init_mode_cos, const double *init_mode_sin);
 
+/*
+ * load_markers_superkiss64: load_markers with the two uniform streams generated ON THE DEVICE by Marsaglia's 64-bit
+ * SuperKISS, the generator multirand_al_int = 3 selects (the reference's default input, src/multirand.F90:1004-1039),
+ * bit for bit.  seeds = multirand_seeds(0:20634) and *iseed = the table position (0 .. 20632), both as multirand_init
+ * (or earlier draws) left them.  The device draws in particle_load's order: nlocal numbers for pv (:180), then nlocal
+ * for px (:222), nlocal = particle_ip_high - particle_ip_low >= np; the unloaded tail of each array (nlocal > np) is
+ * generated and discarded.  Its lag-20632 multiply-with-carry table has no practical jump: one CTA advances it
+ * sequentially in shared memory, each refill a parallel scan over the carry chain; a grid-wide kernel adds the LCG
+ * and xorshift parts, jumped per chunk.  Before returning, seeds and *iseed are overwritten with the state after the
+ * 2 * nlocal draws (a synchronous 165 KB device-to-host copy), so later host draws (particle_remove, particle_split)
+ * continue the same stream.  PIC1DP_EINVAL for *iseed outside [0, 20632], nlocal < np or NULL pointers.
+ */
+#define PIC1DP_SUPERKISS64_NSEED 20635 /* multirand_nseed: 20632 table words, carry, LCG, xorshift */
+int pic1dp_gpu_load_markers_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                        int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED],
+                                        int32_t *iseed, double v_max, int32_t init_nmode, const int32_t *init_mode,
+                                        const double *init_mode_cos, const double *init_mode_sin);
+
 /* debug / parity: n uniforms of the device KISS64 stream starting at `offset`, copied to the host */
 int pic1dp_gpu_kiss64_uniforms(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t offset, int64_t n, double *out);
 
@@ -260,6 +278,16 @@ int pic1dp_gpu_kiss64_uniforms(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t
  * of load_markers_counter */
 int pic1dp_host_kiss64_jump(uint64_t seeds[4], int64_t n);
 int pic1dp_host_kiss64_fill(uint64_t seeds[4], int64_t n, double *out);
+
+/* parity: n uniforms of the device SuperKISS64 stream from (seeds, *iseed), copied to the host; the state is advanced
+ * past them like load_markers_superkiss64 does */
+int pic1dp_gpu_superkiss64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed,
+                                    int64_t n, double *out);
+/* no handle, no GPU: fill = the sequential SuperKISS64 generator (n uniforms of multirand_real_array, state advanced);
+ * refill = one table refill done the way the device does it, as a scan over the carry maps of nchunks chunks
+ * (1024 = the kernel's chunking), for checking the device algorithm against the sequential recurrence */
+int pic1dp_host_superkiss64_fill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed, int64_t n, double *out);
+int pic1dp_host_superkiss64_refill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t nchunks);
 void pic1dp_host_counter_uniforms(uint64_t seed, int32_t stream, int64_t first_index, int64_t n, double *u_v,
                                   double *u_x);
 

@@ -12,6 +12,7 @@ MAX_SPECIES = 4
 MAX_MODES = 64
 UNIQUE_ID_BYTES = 128
 IPC_HANDLE_BYTES = 64
+SUPERKISS64_NSEED = 20635
 
 OK, EINVAL, ECUDA, ENCCL, ENOMEM, ESTATE, ECAPACITY, ENODEVICE, EUNSUPPORTED = range(9)
 DEPOSIT_AUTO, DEPOSIT_SMEM_ATOMIC, DEPOSIT_GLOBAL_RED, DEPOSIT_WARP_PRIVATE, DEPOSIT_FIXED = range(5)
@@ -92,6 +93,8 @@ EXPORTS = [
     "pic1dp_gpu_launch_timing_start", "pic1dp_gpu_launch_timing_stop",
     "pic1dp_gpu_load_markers_kiss64", "pic1dp_gpu_load_markers_counter", "pic1dp_gpu_kiss64_uniforms",
     "pic1dp_host_kiss64_jump", "pic1dp_host_kiss64_fill", "pic1dp_host_counter_uniforms",
+    "pic1dp_gpu_load_markers_superkiss64", "pic1dp_gpu_superkiss64_uniforms", "pic1dp_host_superkiss64_fill",
+    "pic1dp_host_superkiss64_refill",
     "pic1dp_gpu_p2p_trace", "pic1dp_gpu_p2p_trace_read", "pic1dp_gpu_output_all",
 ]
 
@@ -174,6 +177,11 @@ def load() -> C.CDLL:
     L.pic1dp_host_kiss64_fill.argtypes = [u64p, i64, dp]
     L.pic1dp_host_counter_uniforms.argtypes = [C.c_uint64, i32, i64, i64, dp, dp]
     L.pic1dp_host_counter_uniforms.restype = None
+    i32p = C.POINTER(i32)
+    L.pic1dp_gpu_load_markers_superkiss64.argtypes = [vp, i32, i64, i64, i64, u64p, i32p, dbl, i32, C.POINTER(i32), dp, dp]
+    L.pic1dp_gpu_superkiss64_uniforms.argtypes = [vp, u64p, i32p, i64, dp]
+    L.pic1dp_host_superkiss64_fill.argtypes = [u64p, i32p, i64, dp]
+    L.pic1dp_host_superkiss64_refill.argtypes = [u64p, i32]
     L.pic1dp_gpu_output_all.argtypes = [vp, i32, i32, dbl, dp, dp]
     L.pic1dp_gpu_p2p_trace.argtypes = [vp, i32]
     L.pic1dp_gpu_p2p_trace_read.argtypes = [vp, u64p, i64p]

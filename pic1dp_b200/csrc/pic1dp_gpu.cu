@@ -18,6 +18,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -120,6 +121,7 @@ struct pic1dp_gpu {
   double *d_Fre = nullptr, *d_Fim = nullptr, *d_ginv = nullptr;
   double *d_partial = nullptr, *d_red = nullptr, *d_energy = nullptr;
   void *d_kiss_tab = nullptr;   // KissTables: jump-ahead tables of the device KISS64 (allocated on first use)
+  uint64_t *d_sk_state = nullptr;   // SuperKISS64 table + carry advanced by k_superkiss64_table (allocated on first use)
   unsigned long long *d_noob = nullptr;
   unsigned *d_wmax_hi = nullptr;              // [species] running max |deposit source| (high words), DEP_FIXED
   unsigned long long *d_dep_overflow = nullptr, *h_dep_overflow = nullptr;  // conversion overflows (+ pinned mirror)
@@ -372,6 +374,7 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
     }
   if (h->d_noob) cudaFree(h->d_noob);
   if (h->d_kiss_tab) cudaFree(h->d_kiss_tab);
+  if (h->d_sk_state) cudaFree(h->d_sk_state);
   if (h->d_wmax_hi) cudaFree(h->d_wmax_hi);
   if (h->d_dep_overflow) cudaFree(h->d_dep_overflow);
   if (h->d_hist_tab) cudaFree(h->d_hist_tab);
@@ -942,6 +945,140 @@ int pic1dp_host_kiss64_fill(uint64_t seeds[4], int64_t n, double *out) {
   Kiss64 s = {seeds[0], seeds[1], seeds[2], seeds[3]};
   for (int64_t i = 0; i < n; i++) out[i] = int2real64(kiss64_next(s));
   seeds[0] = s.x; seeds[1] = s.xs; seeds[2] = s.z; seeds[3] = s.c;
+  return PIC1DP_OK;
+}
+
+// ---- SuperKISS64 on the device (rng_kernels.cuh) ----
+static bool sk_bad_state(const uint64_t *seeds, const int32_t *iseed) {
+  return !seeds || !iseed || *iseed < 0 || *iseed > PIC1DP_SK_N;
+}
+
+// table position after ntot draws from position i0 (a refill happens lazily, at the draw that finds iseed = N)
+static int32_t sk_iseed_after(int32_t i0, int64_t ntot) {
+  const int64_t rest = PIC1DP_SK_N - i0;
+  if (ntot <= rest) return (int32_t)(i0 + ntot);
+  return (int32_t)((ntot - rest - 1) % PIC1DP_SK_N + 1);
+}
+
+// draws [0, ntot) of the stream at (seeds, *iseed): draw p becomes the uniform d_a[p] (p < na) or d_b[p - pb]
+// (0 <= p - pb < nb), the others are discarded.  seeds / *iseed are advanced past all ntot draws (synchronous D2H of
+// the table), so the host generator continues the same stream.
+static int superkiss64_fill_device(pic1dp_gpu_t *h, uint64_t *seeds, int32_t *iseed, int64_t ntot, double *d_a,
+                                   int64_t na, double *d_b, int64_t pb, int64_t nb) {
+  int rc = kiss_tables(h);
+  if (rc) return rc;
+  if (ntot == 0) return PIC1DP_OK;
+  const size_t state_bytes = (PIC1DP_SK_N + 1) * sizeof(uint64_t);
+  if (!h->d_sk_state) CK(cudaMalloc(&h->d_sk_state, state_bytes));
+  const uint64_t lcg0 = seeds[PIC1DP_SK_N + 1], xs0 = seeds[PIC1DP_SK_N + 2];
+  CK(cudaMemcpyAsync(h->d_sk_state, seeds, state_bytes, cudaMemcpyHostToDevice, h->stream));
+  h->h2d += state_bytes;
+  const int smem = PIC1DP_SK_N * sizeof(uint64_t);
+  CK(cudaFuncSetAttribute(k_superkiss64_table, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  k_superkiss64_table<<<1, PIC1DP_SK_THREADS, smem, h->stream>>>(h->d_sk_state, *iseed, ntot, d_a, na, d_b, pb, nb);
+  CKL(h);
+  const int chunk = 512;   // a multiple of 32 (the tile protocol of k_superkiss64_finish)
+  const struct { double *d; int64_t off, n; } win[2] = {{d_a, 0, na}, {d_b, pb, nb}};
+  for (const auto &w : win) {
+    if (w.n == 0) continue;
+    const int64_t nchunks = (w.n + chunk - 1) / chunk;
+    int blocks = (int)((nchunks + 127) / 128);
+    if (blocks > h->nsm * 16) blocks = h->nsm * 16;
+    k_superkiss64_finish<<<blocks, 128, 0, h->stream>>>(lcg0, xs0, (uint64_t)w.off, w.n, chunk,
+                                                        (const KissTables *)h->d_kiss_tab, w.d);
+    CKL(h);
+  }
+  CK(cudaMemcpyAsync(seeds, h->d_sk_state, state_bytes, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->d2h += state_bytes;
+  seeds[PIC1DP_SK_N + 1] = sk_lcg_jump(lcg0, (uint64_t)ntot);
+  seeds[PIC1DP_SK_N + 2] = sk_xs_jump(xs0, (uint64_t)ntot, kiss_xs_jump);
+  *iseed = sk_iseed_after(*iseed, ntot);
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_load_markers_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                        int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed,
+                                        double v_max, int32_t init_nmode, const int32_t *init_mode,
+                                        const double *init_mode_cos, const double *init_mode_sin) {
+  int rc = load_check_args(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if (sk_bad_state(seeds, iseed) || nlocal < np) {
+    h->err = "load_markers_superkiss64: bad stream argument (iseed in [0, 20632], nlocal >= np)";
+    return PIC1DP_EINVAL;
+  }
+  CK(cudaSetDevice(h->p.device));
+  Species &S = h->sp[isp];
+  // multirand_real_array(pv) over the whole local array (:180), then multirand_real_array(px) (:222)
+  if ((rc = superkiss64_fill_device(h, seeds, iseed, 2 * nlocal, S.v[0], np, S.x[0], nlocal, np))) return rc;
+  return load_markers_finish(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin, 2);
+}
+
+int pic1dp_gpu_superkiss64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed, int64_t n,
+                                    double *out) {
+  if (!h || sk_bad_state(seeds, iseed) || n < 0 || (n > 0 && !out)) {
+    if (h) h->err = "superkiss64_uniforms: bad argument";
+    return PIC1DP_EINVAL;
+  }
+  if (n == 0) return PIC1DP_OK;
+  CK(cudaSetDevice(h->p.device));
+  double *d = nullptr;
+  CK(cudaMalloc(&d, (size_t)n * 8));
+  int rc = superkiss64_fill_device(h, seeds, iseed, n, d, n, nullptr, 0, 0);
+  cudaError_t e = cudaSuccess;
+  if (!rc) {
+    e = cudaMemcpyAsync(out, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    h->d2h += n * 8;
+  }
+  cudaFree(d);
+  if (rc) return rc;
+  if (e != cudaSuccess) { h->err = std::string("superkiss64_uniforms: ") + cudaGetErrorString(e); return PIC1DP_ECUDA; }
+  return PIC1DP_OK;
+}
+
+int pic1dp_host_superkiss64_fill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed, int64_t n, double *out) {
+  if (sk_bad_state(seeds, iseed) || n < 0 || (n > 0 && !out)) return PIC1DP_EINVAL;
+  const int N = PIC1DP_SK_N;
+  int32_t i = *iseed;
+  uint64_t z = seeds[N + 1], xs = seeds[N + 2];
+  for (int64_t k = 0; k < n; k++) {
+    if (i >= N) {
+      seeds[N] = sk_chunk_rewrite(seeds, 0, N, seeds[N]);
+      i = 0;
+    }
+    z = sk_lcg_next(z);
+    xs = sk_xs_next(xs);
+    out[k] = int2real64(seeds[i++] + z + xs);
+  }
+  seeds[N + 1] = z;
+  seeds[N + 2] = xs;
+  *iseed = i;
+  return PIC1DP_OK;
+}
+
+int pic1dp_host_superkiss64_refill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t nchunks) {
+  const int N = PIC1DP_SK_N;
+  if (!seeds || nchunks < 1 || nchunks > N) return PIC1DP_EINVAL;
+  const int K = (N + nchunks - 1) / nchunks;
+  std::vector<unsigned> m(nchunks), prev;
+  std::vector<uint64_t> left(nchunks, 0);
+  const uint64_t c0 = seeds[N];
+  for (int k = 0; k < nchunks; k++) {
+    const int s = std::min(k * K, N), e = std::min(s + K, N);
+    m[k] = sk_chunk_map(seeds, s, e, c0);
+    if (s > 0 && s < e) left[k] = seeds[s - 1];
+  }
+  for (int d = 1; d < nchunks; d <<= 1) {   // inclusive scan of the chunk maps (Hillis-Steele, as across warp lanes)
+    prev = m;
+    for (int k = d; k < nchunks; k++) m[k] = sk_compose(prev[k], prev[k - d]);
+  }
+  for (int k = 0; k < nchunks; k++) {
+    const int s = std::min(k * K, N), e = std::min(s + K, N);
+    if (s >= e) continue;
+    const uint64_t cout = sk_chunk_rewrite(seeds, s, e, s == 0 ? c0 : sk_hi(left[k]) + sk_apply(m[k - 1], 0));
+    if (e == N) seeds[N] = cout;
+  }
   return PIC1DP_OK;
 }
 

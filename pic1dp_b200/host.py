@@ -48,6 +48,13 @@ def _dp(a: Optional[np.ndarray]):
     return a.ctypes.data_as(C.POINTER(C.c_double))
 
 
+def _u64p(seeds: np.ndarray):
+    """The SuperKISS64 state multirand_seeds(0:20634), passed for in-place update."""
+    assert seeds.dtype == np.uint64 and seeds.size == _capi.SUPERKISS64_NSEED and seeds.flags["C_CONTIGUOUS"], \
+        "SuperKISS64 state: C-contiguous uint64 array of 20635 words"
+    return seeds.ctypes.data_as(C.POINTER(C.c_uint64))
+
+
 def _ptr(addr: int):
     return C.cast(C.c_void_p(addr), C.POINTER(C.c_double))
 
@@ -143,6 +150,29 @@ class Pic1dGpu:
         sd = (C.c_uint64 * 4)(*[int(v) & 0xFFFFFFFFFFFFFFFF for v in seeds])
         self._ck(self.L.pic1dp_gpu_load_markers_kiss64(self._h, isp, int(n), int(nparticle_init), sd, int(offset_v),
                                                        int(offset_x), float(v_max), nm, im, ic, isn), "load_markers_kiss64")
+
+    def load_markers_superkiss64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, nparticle_init: int,
+                                 v_max: float = 8.0, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)) -> int:
+        """Device-side particle_load with the device SuperKISS64 stream (multirand_al_int = 3), bit-exact to multirand.
+        seeds: multirand_seeds(0:20634) as a uint64 array, advanced IN PLACE past the 2 * nlocal draws; iseed: the
+        table position before them.  Returns the table position after them."""
+        nm = len(init_mode)
+        im = (C.c_int32 * nm)(*init_mode)
+        ic = (C.c_double * nm)(*init_cos)
+        isn = (C.c_double * nm)(*init_sin)
+        pos = C.c_int32(int(iseed))
+        self._ck(self.L.pic1dp_gpu_load_markers_superkiss64(self._h, isp, int(n), int(nlocal), int(nparticle_init),
+                                                            _u64p(seeds), C.byref(pos), float(v_max), nm, im, ic, isn),
+                 "load_markers_superkiss64")
+        return pos.value
+
+    def superkiss64_uniforms(self, seeds, iseed: int, n: int):
+        """(n uniforms of the device SuperKISS64 stream, table position after them); seeds advanced in place."""
+        out = np.empty(n)
+        pos = C.c_int32(int(iseed))
+        self._ck(self.L.pic1dp_gpu_superkiss64_uniforms(self._h, _u64p(seeds), C.byref(pos), int(n), _dp(out)),
+                 "superkiss64_uniforms")
+        return out, pos.value
 
     def load_markers_counter(self, isp: int, n: int, seed: int, first_index: int, nparticle_init: int,
                              v_max: float = 8.0, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)):
@@ -567,3 +597,21 @@ def host_counter_uniforms(seed: int, stream: int, first_index: int, n: int):
     u_v, u_x = np.empty(n), np.empty(n)
     _capi.load().pic1dp_host_counter_uniforms(int(seed), int(stream), int(first_index), int(n), _dp(u_v), _dp(u_x))
     return u_v, u_x
+
+
+def host_superkiss64_fill(seeds, iseed: int, n: int):
+    """(n uniforms of multirand_real_array with SuperKISS64, table position after them); seeds (uint64 array of
+    20635 words) advanced in place."""
+    out = np.empty(n)
+    pos = C.c_int32(int(iseed))
+    rc = _capi.load().pic1dp_host_superkiss64_fill(_u64p(seeds), C.byref(pos), int(n), _dp(out))
+    if rc:
+        raise Pic1dpError(rc, "pic1dp_host_superkiss64_fill", "bad argument")
+    return out, pos.value
+
+
+def host_superkiss64_refill(seeds, nchunks: int):
+    """One table refill of seeds (in place) by the device's chunked carry-map scan, run on the host."""
+    rc = _capi.load().pic1dp_host_superkiss64_refill(_u64p(seeds), int(nchunks))
+    if rc:
+        raise Pic1dpError(rc, "pic1dp_host_superkiss64_refill", "bad argument")
