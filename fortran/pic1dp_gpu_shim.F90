@@ -129,6 +129,32 @@ interface
     real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
     integer(c_int32_t), intent(in) :: init_mode(*)
   end function
+  integer(c_int) function pic1dp_gpu_load_markers_maxwellian_kiss64(handle, isp, np, nlocal, nparticle_init, seeds, &
+      gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin) &
+      bind(c, name = 'pic1dp_gpu_load_markers_maxwellian_kiss64')
+    import :: c_ptr, c_int, c_int32_t, c_int64_t, c_double
+    type(c_ptr), value :: handle
+    integer(c_int32_t), value :: isp, init_nmode
+    integer(c_int64_t), value :: np, nlocal, nparticle_init
+    integer(c_int64_t), intent(inout) :: seeds(4)   ! multirand_seeds(0:3), same bits as the C uint64_t
+    integer(c_int32_t), intent(inout) :: gauss_filled
+    real(c_double), intent(inout) :: gauss_buf
+    real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
+    integer(c_int32_t), intent(in) :: init_mode(*)
+  end function
+  integer(c_int) function pic1dp_gpu_load_markers_maxwellian_superkiss64(handle, isp, np, nlocal, nparticle_init, &
+      seeds, iseed, gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin) &
+      bind(c, name = 'pic1dp_gpu_load_markers_maxwellian_superkiss64')
+    import :: c_ptr, c_int, c_int32_t, c_int64_t, c_double
+    type(c_ptr), value :: handle
+    integer(c_int32_t), value :: isp, init_nmode
+    integer(c_int64_t), value :: np, nlocal, nparticle_init
+    integer(c_int64_t), intent(inout) :: seeds(20635)   ! multirand_seeds(0:20634), same bits as the C uint64_t
+    integer(c_int32_t), intent(inout) :: iseed, gauss_filled
+    real(c_double), intent(inout) :: gauss_buf
+    real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
+    integer(c_int32_t), intent(in) :: init_mode(*)
+  end function
   integer(c_int) function pic1dp_gpu_output_all(handle, nx_opd, nv_opd, v_max, scalars, dist) &
       bind(c, name = 'pic1dp_gpu_output_all')
     import :: c_ptr, c_int, c_int32_t, c_double
@@ -249,6 +275,7 @@ public :: pic1dp_gpu_compute_dist_pertb_abs_v, pic1dp_gpu_particle_merge, pic1dp
 public :: pic1dp_gpu_particle_split
 public :: pic1dp_gpu_load_markers_kiss64, pic1dp_host_kiss64_jump, pic1dp_gpu_output_all
 public :: pic1dp_gpu_load_markers_superkiss64
+public :: pic1dp_gpu_load_markers_maxwellian_kiss64, pic1dp_gpu_load_markers_maxwellian_superkiss64
 
 end module pic1dp_gpu
 
@@ -414,6 +441,49 @@ CHKERRQ(global_ierr)
 multirand_seeds(0 : 20634) = seeds(1 : 20635)
 multirand_iseed = iseed
 end subroutine gpu_particle_load_superkiss64
+
+! particle_load with input_imarker = 1 (Maxwellian markers, iptcldist = 0): no marker-sized host-to-device copy.  Call in
+! place of multirand_gaussian_array(pv) and multirand_real_array(px) (src/pic1dp_particle.F90:172-178, :222) AFTER
+! multirand_init.  The device draws exactly what those two calls would have drawn (src/multirand.F90:838-872, then :664)
+! and returns the advanced state, which is copied back into the multirand module.  gauss_filled / gauss_buf are the
+! one-slot buffer of multirand_gaussian_array (a value left over by an odd-length call): pass the module's buffer and
+! store the returned one back, so that the next Gaussian draws (the next species, particle_split) continue the stream.
+subroutine gpu_particle_load_maxwellian_kiss64(ispecies, np, nlocal, gauss_filled, gauss_buf)
+use multirand, only : multirand_seeds
+implicit none
+#include "finclude/petsc.h90"
+PetscInt, intent(in) :: ispecies, np, nlocal
+integer(c_int32_t), intent(inout) :: gauss_filled
+real(c_double), intent(inout) :: gauss_buf
+integer(c_int64_t) :: seeds(4)
+seeds(1 : 4) = multirand_seeds(0 : 3)
+global_ierr = pic1dp_gpu_load_markers_maxwellian_kiss64(gpu_handle, int(ispecies - 1, c_int32_t), int(np, c_int64_t), &
+  int(nlocal, c_int64_t), int(input_species_nparticle_init(ispecies), c_int64_t), seeds, gauss_filled, gauss_buf, &
+  int(input_init_nmode, c_int32_t), int(input_init_mode, c_int32_t), &
+  real(input_init_mode_cos, c_double), real(input_init_mode_sin, c_double))
+CHKERRQ(global_ierr)
+multirand_seeds(0 : 3) = seeds(1 : 4)
+end subroutine gpu_particle_load_maxwellian_kiss64
+
+subroutine gpu_particle_load_maxwellian_superkiss64(ispecies, np, nlocal, gauss_filled, gauss_buf)
+use multirand, only : multirand_seeds, multirand_iseed
+implicit none
+#include "finclude/petsc.h90"
+PetscInt, intent(in) :: ispecies, np, nlocal
+integer(c_int32_t), intent(inout) :: gauss_filled
+real(c_double), intent(inout) :: gauss_buf
+integer(c_int64_t) :: seeds(20635)
+integer(c_int32_t) :: iseed
+seeds(1 : 20635) = multirand_seeds(0 : 20634)
+iseed = int(multirand_iseed, c_int32_t)
+global_ierr = pic1dp_gpu_load_markers_maxwellian_superkiss64(gpu_handle, int(ispecies - 1, c_int32_t), &
+  int(np, c_int64_t), int(nlocal, c_int64_t), int(input_species_nparticle_init(ispecies), c_int64_t), seeds, iseed, &
+  gauss_filled, gauss_buf, int(input_init_nmode, c_int32_t), int(input_init_mode, c_int32_t), &
+  real(input_init_mode_cos, c_double), real(input_init_mode_sin, c_double))
+CHKERRQ(global_ierr)
+multirand_seeds(0 : 20634) = seeds(1 : 20635)
+multirand_iseed = iseed
+end subroutine gpu_particle_load_maxwellian_superkiss64
 
 ! before output_all / particle_optimize (src/pic1dp_output.F90:128-150, :228-237): device -> host Vecs
 subroutine gpu_particle_refresh_host(ispecies, vx, vv, vp, vw)

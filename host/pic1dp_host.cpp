@@ -80,7 +80,7 @@ struct Input {
   double input_output_interval = 0.5;
   // placement / implementation (not in the reference)
   int ngpus = 1, deposit_mode = 0, field_mode = 0, fuse = 1;
-  int device_rng = 1;  // 1: SuperKISS64 uniform-v markers are generated on the device (same bits); 0: host stream
+  int device_rng = 1;  // 1: KISS64 / SuperKISS64 marker streams are generated on the device; 0: host streams
   std::string out = "pic1dp_energy.txt";
   std::string petsc_out;          // when set: also write the reference's binary output file (pic1dp.out layout)
   int input_nv = 128, input_nx_opd = 64, input_nv_opd = 64;  // src/pic1dp_input.F90:131, :253-256
@@ -430,10 +430,12 @@ static void particle_init(Rank &r, const uint8_t *uid) {
 
 // particle_load (src/pic1dp_particle.F90:145-269): the RNG (multirand, a sequential generator) keeps the reference's
 // draw order -- the whole local array for v first (:174 / :180), then for x (:222) -- and the loader arithmetic
-// (:172-237, :260-263) runs on the device.  With SuperKISS64 (al_int = 3, the default) and uniform-v markers
-// (input_imarker = 2) the device also generates both streams from the generator's state and hands the advanced state
-// back (pic1dp_gpu_load_markers_superkiss64), so nothing marker-sized crosses PCIe; otherwise (or with device_rng=0)
-// the host draws them and only the two uniform streams cross PCIe (pic1dp_gpu_load_markers).  Same markers either way.
+// (:172-237, :260-263) runs on the device.  With KISS64 (al_int = 1) or SuperKISS64 (al_int = 3, the default) the device
+// also generates both streams from the generator's state -- uniform v (input_imarker = 2) or the Gaussian v of
+// Maxwellian markers (input_imarker = 1) -- and the generator (with the Gaussian one-slot buffer) continues after them,
+// so nothing marker-sized crosses PCIe.  With MT19937-64, or device_rng=0, the host draws the streams and they cross
+// PCIe (pic1dp_gpu_load_markers / _maxwellian).  The same markers either way: bit for bit for uniform v, and for
+// Gaussian v to a few ulp (the device log is not glibc's; every accept decision and every other stream is exact).
 static void particle_load(Rank &r) {
   const pic1dp_input::Input &in = *r.in;
   multirand::Generator &rng = r.rng;
@@ -446,13 +448,31 @@ static void particle_load(Rank &r) {
   int64_t nparticle_unload = (in.input_nparticle_max - ninit) / r.g.global_npe;
   if (r.g.global_mype == 0) nparticle_unload += (in.input_nparticle_max - ninit) % r.g.global_npe;
   r.particle_np = n - nparticle_unload;
-  if (in.input_imarker == 2 && in.input_multirand_al_int == 3 && in.device_rng) {
-    int32_t iseed = rng.iseed;
-    r.g.global_ierr = pic1dp_gpu_load_markers_superkiss64(r.h, 0, r.particle_np, n, ninit, rng.s.data(), &iseed,
-                                                          in.input_v_max, in.input_init_nmode, in.input_init_mode,
-                                                          in.input_init_mode_cos, in.input_init_mode_sin);
+  const int al = in.input_multirand_al_int;
+  if (in.device_rng && (al == 1 || al == 3)) {
+    int32_t iseed = rng.iseed, filled = rng.has_spare ? 1 : 0;
+    double spare = rng.spare;
+    if (in.input_imarker == 1 && al == 3)
+      r.g.global_ierr = pic1dp_gpu_load_markers_maxwellian_superkiss64(
+          r.h, 0, r.particle_np, n, ninit, rng.s.data(), &iseed, &filled, &spare, in.input_init_nmode, in.input_init_mode,
+          in.input_init_mode_cos, in.input_init_mode_sin);
+    else if (in.input_imarker == 1)
+      r.g.global_ierr = pic1dp_gpu_load_markers_maxwellian_kiss64(r.h, 0, r.particle_np, n, ninit, rng.s.data(), &filled,
+                                                                  &spare, in.input_init_nmode, in.input_init_mode,
+                                                                  in.input_init_mode_cos, in.input_init_mode_sin);
+    else if (al == 3)
+      r.g.global_ierr = pic1dp_gpu_load_markers_superkiss64(r.h, 0, r.particle_np, n, ninit, rng.s.data(), &iseed,
+                                                            in.input_v_max, in.input_init_nmode, in.input_init_mode,
+                                                            in.input_init_mode_cos, in.input_init_mode_sin);
+    else   // KISS64 jumps: pv is draws [0, n), px draws [n, 2n); the host generator then skips both
+      r.g.global_ierr = pic1dp_gpu_load_markers_kiss64(r.h, 0, r.particle_np, ninit, rng.s.data(), 0, n, in.input_v_max,
+                                                       in.input_init_nmode, in.input_init_mode, in.input_init_mode_cos,
+                                                       in.input_init_mode_sin);
     CHKERRQ(r.g, r.h);
+    if (in.input_imarker != 1 && al == 1) pic1dp_host_kiss64_jump(rng.s.data(), 2 * n);
     rng.iseed = iseed;
+    rng.has_spare = filled != 0;
+    rng.spare = spare;
     return;
   }
   r.v.resize(n);

@@ -235,8 +235,9 @@ int pic1dp_gpu_load_markers_maxwellian(pic1dp_gpu_t *h, int32_t isp, int64_t np,
  * (LCG, xorshift, multiply-with-carry) to its chunk in O(log offset) and then runs the sequential generator; the
  * uniforms are INT2REAL64 of its outputs (:49).  Afterwards the host advances its own state with
  * pic1dp_host_kiss64_jump(seeds, 2 * nlocal * nspecies) so that later draws (particle_remove, particle_split)
- * continue the same stream.  SuperKISS64 (al_int = 3) has its own loader below; MT19937-64 streams keep coming from
- * the host through load_markers.
+ * continue the same stream.  SuperKISS64 (al_int = 3) has its own loader below, and both generators have a
+ * Maxwellian loader (input_imarker = 1) below; MT19937-64 (al_int = 2) streams keep coming from the host through
+ * load_markers / load_markers_maxwellian.
  */
 int pic1dp_gpu_load_markers_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nparticle_init,
                                    const uint64_t seeds[4], int64_t offset_v, int64_t offset_x, double v_max,
@@ -269,6 +270,38 @@ int pic1dp_gpu_load_markers_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np
                                         int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED],
                                         int32_t *iseed, double v_max, int32_t init_nmode, const int32_t *init_mode,
                                         const double *init_mode_cos, const double *init_mode_sin);
+
+/*
+ * load_markers_maxwellian_kiss64 / _superkiss64: load_markers_maxwellian (input_imarker = 1, iptcldist = 0,
+ * src/pic1dp_particle.F90:172-178) with BOTH of particle_load's streams generated ON THE DEVICE from the generator's
+ * state: multirand_gaussian_array(pv, nlocal) (:174; Marsaglia's polar method, src/multirand.F90:838-872), then
+ * multirand_real_array(px, nlocal) (:222), nlocal = particle_ip_high - particle_ip_low >= np; elements past np are drawn
+ * and discarded.  The Gaussian call's one-slot buffer is part of the state: *gauss_filled / *gauss_buf = the value
+ * a previous gaussian_array left buffered (it becomes element 0 without a draw), and on return the value the call leaves
+ * buffered when it needs an odd number of values after that (element nlocal).  Attempts are pairs of draws; whether one
+ * is accepted depends on its own two words and is decided with the reference's IEEE operations, so the draws consumed,
+ * the x stream and the returned state are exact; the Gaussian values x * sqrt(-2 log(w) / w) go through the device log
+ * and match the host's to a few ulp.  The device works in rounds of PIC1DP_GAUSS_ROUND_DRAWS draws (32 MB of scratch)
+ * and reads one count per round.  State in / out: KISS64 seeds = multirand_seeds(0:3); SuperKISS64 seeds =
+ * multirand_seeds(0:20634) and *iseed = the table position (its x stream is regenerated from a copy of the table taken
+ * at the start of the round that holds the last attempt, at most one round of draws).  On success the state is the one
+ * after all draws of both calls, so later host draws (particle_remove, particle_split's gaussian_array) continue the
+ * same stream.  PIC1DP_EINVAL for iptcldist != 0, nlocal < np, *iseed outside [0, 20632] or NULL pointers,
+ * PIC1DP_ECAPACITY for np > capacity; a refused call leaves the state untouched.
+ */
+#define PIC1DP_GAUSS_ROUND_DRAWS 4194304
+int pic1dp_gpu_load_markers_maxwellian_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                              int64_t nparticle_init, uint64_t seeds[4], int32_t *gauss_filled,
+                                              double *gauss_buf, int32_t init_nmode, const int32_t *init_mode,
+                                              const double *init_mode_cos, const double *init_mode_sin);
+int pic1dp_gpu_load_markers_maxwellian_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                                   int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED],
+                                                   int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
+                                                   int32_t init_nmode, const int32_t *init_mode,
+                                                   const double *init_mode_cos, const double *init_mode_sin);
+/* the last Maxwellian load of this handle: draws its Gaussian call consumed, rounds it ran, and the SuperKISS64 draws
+ * it generated a second time for the x stream (0 for KISS64) */
+int pic1dp_gpu_last_gaussian_load(pic1dp_gpu_t *h, int64_t *draws, int64_t *rounds, int64_t *regenerated);
 
 /* debug / parity: n uniforms of the device KISS64 stream starting at `offset`, copied to the host */
 int pic1dp_gpu_kiss64_uniforms(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t offset, int64_t n, double *out);

@@ -13,6 +13,7 @@ MAX_MODES = 64
 UNIQUE_ID_BYTES = 128
 IPC_HANDLE_BYTES = 64
 SUPERKISS64_NSEED = 20635
+GAUSS_ROUND_DRAWS = 4194304   # PIC1DP_GAUSS_ROUND_DRAWS: draws per round of the device Gaussian stream
 
 OK, EINVAL, ECUDA, ENCCL, ENOMEM, ESTATE, ECAPACITY, ENODEVICE, EUNSUPPORTED = range(9)
 DEPOSIT_AUTO, DEPOSIT_SMEM_ATOMIC, DEPOSIT_GLOBAL_RED, DEPOSIT_WARP_PRIVATE, DEPOSIT_FIXED = range(5)
@@ -94,7 +95,8 @@ EXPORTS = [
     "pic1dp_gpu_load_markers_kiss64", "pic1dp_gpu_load_markers_counter", "pic1dp_gpu_kiss64_uniforms",
     "pic1dp_host_kiss64_jump", "pic1dp_host_kiss64_fill", "pic1dp_host_counter_uniforms",
     "pic1dp_gpu_load_markers_superkiss64", "pic1dp_gpu_superkiss64_uniforms", "pic1dp_host_superkiss64_fill",
-    "pic1dp_host_superkiss64_refill",
+    "pic1dp_host_superkiss64_refill", "pic1dp_gpu_load_markers_maxwellian_kiss64",
+    "pic1dp_gpu_load_markers_maxwellian_superkiss64", "pic1dp_gpu_last_gaussian_load",
     "pic1dp_gpu_p2p_trace", "pic1dp_gpu_p2p_trace_read", "pic1dp_gpu_output_all",
 ]
 
@@ -182,6 +184,10 @@ def load() -> C.CDLL:
     L.pic1dp_gpu_superkiss64_uniforms.argtypes = [vp, u64p, i32p, i64, dp]
     L.pic1dp_host_superkiss64_fill.argtypes = [u64p, i32p, i64, dp]
     L.pic1dp_host_superkiss64_refill.argtypes = [u64p, i32]
+    L.pic1dp_gpu_load_markers_maxwellian_kiss64.argtypes = [vp, i32, i64, i64, i64, u64p, i32p, dp, i32, i32p, dp, dp]
+    L.pic1dp_gpu_load_markers_maxwellian_superkiss64.argtypes = [vp, i32, i64, i64, i64, u64p, i32p, i32p, dp, i32, i32p,
+                                                                 dp, dp]
+    L.pic1dp_gpu_last_gaussian_load.argtypes = [vp, i64p, i64p, i64p]
     L.pic1dp_gpu_output_all.argtypes = [vp, i32, i32, dbl, dp, dp]
     L.pic1dp_gpu_p2p_trace.argtypes = [vp, i32]
     L.pic1dp_gpu_p2p_trace_read.argtypes = [vp, u64p, i64p]

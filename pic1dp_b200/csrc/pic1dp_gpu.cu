@@ -19,6 +19,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -122,6 +123,12 @@ struct pic1dp_gpu {
   double *d_partial = nullptr, *d_red = nullptr, *d_energy = nullptr;
   void *d_kiss_tab = nullptr;   // KissTables: jump-ahead tables of the device KISS64 (allocated on first use)
   uint64_t *d_sk_state = nullptr;   // SuperKISS64 table + carry advanced by k_superkiss64_table (allocated on first use)
+  uint64_t *d_sk_round = nullptr;   // copy of d_sk_state at the start of the current Gaussian round
+  // Gaussian marker stream (allocated on first use): one round of raw words, per-CTA accept counts, GaussCtl
+  double *d_gauss_words = nullptr;
+  unsigned *d_gauss_bcount = nullptr;
+  void *d_gauss_ctl = nullptr;
+  int64_t gauss_draws = 0, gauss_rounds = 0, gauss_regenerated = 0;   // of the last Gaussian load
   unsigned long long *d_noob = nullptr;
   unsigned *d_wmax_hi = nullptr;              // [species] running max |deposit source| (high words), DEP_FIXED
   unsigned long long *d_dep_overflow = nullptr, *h_dep_overflow = nullptr;  // conversion overflows (+ pinned mirror)
@@ -375,6 +382,10 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
   if (h->d_noob) cudaFree(h->d_noob);
   if (h->d_kiss_tab) cudaFree(h->d_kiss_tab);
   if (h->d_sk_state) cudaFree(h->d_sk_state);
+  if (h->d_sk_round) cudaFree(h->d_sk_round);
+  if (h->d_gauss_words) cudaFree(h->d_gauss_words);
+  if (h->d_gauss_bcount) cudaFree(h->d_gauss_bcount);
+  if (h->d_gauss_ctl) cudaFree(h->d_gauss_ctl);
   if (h->d_wmax_hi) cudaFree(h->d_wmax_hi);
   if (h->d_dep_overflow) cudaFree(h->d_dep_overflow);
   if (h->d_hist_tab) cudaFree(h->d_hist_tab);
@@ -868,7 +879,9 @@ static int kiss_tables(pic1dp_gpu_t *h) {
   return PIC1DP_OK;
 }
 
-static int kiss64_fill_device(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t offset, int64_t n, double *d_out) {
+// raw: the 64-bit outputs themselves (bits in the double slots) instead of the uniforms
+static int kiss64_fill_device(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t offset, int64_t n, double *d_out,
+                              bool raw = false) {
   int rc = kiss_tables(h);
   if (rc) return rc;
   if (n == 0) return PIC1DP_OK;
@@ -877,7 +890,11 @@ static int kiss64_fill_device(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t 
   const int64_t nchunks = (n + chunk - 1) / chunk;
   int blocks = (int)((nchunks + 127) / 128);
   if (blocks > h->nsm * 16) blocks = h->nsm * 16;
-  k_kiss64_fill<<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, (const KissTables *)h->d_kiss_tab, d_out);
+  if (raw)
+    k_kiss64_fill<true><<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, (const KissTables *)h->d_kiss_tab,
+                                                       d_out);
+  else
+    k_kiss64_fill<<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, (const KissTables *)h->d_kiss_tab, d_out);
   CKL(h);
   return PIC1DP_OK;
 }
@@ -960,6 +977,33 @@ static int32_t sk_iseed_after(int32_t i0, int64_t ntot) {
   return (int32_t)((ntot - rest - 1) % PIC1DP_SK_N + 1);
 }
 
+// io[i] = the finished draw offset + i, i < n, from its raw table word (k_superkiss64_finish); (lcg0, xs0) = the LCG and
+// xorshift before draw 0; raw: the 64-bit outputs instead of the uniforms
+static int superkiss64_finish_device(pic1dp_gpu_t *h, uint64_t lcg0, uint64_t xs0, int64_t offset, int64_t n, double *io,
+                                     bool raw = false) {
+  if (n == 0) return PIC1DP_OK;
+  const int chunk = 512;   // a multiple of 32 (the tile protocol of k_superkiss64_finish)
+  const int64_t nchunks = (n + chunk - 1) / chunk;
+  int blocks = (int)((nchunks + 127) / 128);
+  if (blocks > h->nsm * 16) blocks = h->nsm * 16;
+  const KissTables *tab = (const KissTables *)h->d_kiss_tab;
+  if (raw)
+    k_superkiss64_finish<true><<<blocks, 128, 0, h->stream>>>(lcg0, xs0, (uint64_t)offset, n, chunk, tab, io);
+  else
+    k_superkiss64_finish<<<blocks, 128, 0, h->stream>>>(lcg0, xs0, (uint64_t)offset, n, chunk, tab, io);
+  CKL(h);
+  return PIC1DP_OK;
+}
+
+static int superkiss64_table_device(pic1dp_gpu_t *h, int32_t i0, int64_t ntot, double *d_a, int64_t na, double *d_b,
+                                    int64_t pb, int64_t nb) {
+  const int smem = PIC1DP_SK_N * sizeof(uint64_t);
+  CK(cudaFuncSetAttribute(k_superkiss64_table, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  k_superkiss64_table<<<1, PIC1DP_SK_THREADS, smem, h->stream>>>(h->d_sk_state, i0, ntot, d_a, na, d_b, pb, nb);
+  CKL(h);
+  return PIC1DP_OK;
+}
+
 // draws [0, ntot) of the stream at (seeds, *iseed): draw p becomes the uniform d_a[p] (p < na) or d_b[p - pb]
 // (0 <= p - pb < nb), the others are discarded.  seeds / *iseed are advanced past all ntot draws (synchronous D2H of
 // the table), so the host generator continues the same stream.
@@ -973,21 +1017,9 @@ static int superkiss64_fill_device(pic1dp_gpu_t *h, uint64_t *seeds, int32_t *is
   const uint64_t lcg0 = seeds[PIC1DP_SK_N + 1], xs0 = seeds[PIC1DP_SK_N + 2];
   CK(cudaMemcpyAsync(h->d_sk_state, seeds, state_bytes, cudaMemcpyHostToDevice, h->stream));
   h->h2d += state_bytes;
-  const int smem = PIC1DP_SK_N * sizeof(uint64_t);
-  CK(cudaFuncSetAttribute(k_superkiss64_table, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  k_superkiss64_table<<<1, PIC1DP_SK_THREADS, smem, h->stream>>>(h->d_sk_state, *iseed, ntot, d_a, na, d_b, pb, nb);
-  CKL(h);
-  const int chunk = 512;   // a multiple of 32 (the tile protocol of k_superkiss64_finish)
-  const struct { double *d; int64_t off, n; } win[2] = {{d_a, 0, na}, {d_b, pb, nb}};
-  for (const auto &w : win) {
-    if (w.n == 0) continue;
-    const int64_t nchunks = (w.n + chunk - 1) / chunk;
-    int blocks = (int)((nchunks + 127) / 128);
-    if (blocks > h->nsm * 16) blocks = h->nsm * 16;
-    k_superkiss64_finish<<<blocks, 128, 0, h->stream>>>(lcg0, xs0, (uint64_t)w.off, w.n, chunk,
-                                                        (const KissTables *)h->d_kiss_tab, w.d);
-    CKL(h);
-  }
+  if ((rc = superkiss64_table_device(h, *iseed, ntot, d_a, na, d_b, pb, nb))) return rc;
+  if ((rc = superkiss64_finish_device(h, lcg0, xs0, 0, na, d_a))) return rc;
+  if ((rc = superkiss64_finish_device(h, lcg0, xs0, pb, nb, d_b))) return rc;
   CK(cudaMemcpyAsync(seeds, h->d_sk_state, state_bytes, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   h->d2h += state_bytes;
@@ -1079,6 +1111,177 @@ int pic1dp_host_superkiss64_refill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int
     const uint64_t cout = sk_chunk_rewrite(seeds, s, e, s == 0 ? c0 : sk_hi(left[k]) + sk_apply(m[k - 1], 0));
     if (e == N) seeds[N] = cout;
   }
+  return PIC1DP_OK;
+}
+
+// ---- Maxwellian markers: multirand_gaussian_array(pv) on the device (rng_kernels.cuh) ----
+static_assert(PIC1DP_GAUSS_ROUND == PIC1DP_GAUSS_ROUND_DRAWS && PIC1DP_GAUSS_ROUND % 2 == 0, "Gaussian round size");
+struct GaussResult {
+  int64_t cut = 0;       // draws the Gaussian call consumed: the x stream starts here
+  int32_t filled = 0;    // the one-slot buffer after the call
+  double buf = 0.0;
+};
+
+// gaussian_array(pv, nlocal) from the raw-word stream that produce(a, d) writes (words [a, a + PIC1DP_GAUSS_ROUND) from
+// the call's first draw, into d), in rounds: words, accept counts, compaction into d_v (elements < np kept), then one
+// read of the running count.  The first round whose count reaches the attempts needed holds the cut.  (filled, buf) is
+// the caller's buffer on entry; the result carries it out, the caller's copy is left alone.
+static int gauss_stream_device(pic1dp_gpu_t *h, int64_t np, int64_t nlocal, int32_t filled, double buf, double *d_v,
+                               GaussResult &out, const std::function<int(int64_t, double *)> &produce) {
+  out = GaussResult();
+  out.filled = filled;
+  out.buf = buf;
+  h->gauss_rounds = 0;
+  if (nlocal == 0) return PIC1DP_OK;
+  int64_t lo = 0;
+  if (filled) {   // the buffered value is element 0; no draw for it
+    if (np > 0) {
+      CK(cudaMemcpyAsync(d_v, &buf, 8, cudaMemcpyHostToDevice, h->stream));
+      CK(cudaStreamSynchronize(h->stream));
+      h->h2d += 8;
+    }
+    lo = 1;
+  }
+  const int64_t need = (nlocal - lo + 1) / 2;   // accepted attempts
+  out.filled = (int32_t)((nlocal - lo) & 1);
+  if (need == 0) return PIC1DP_OK;
+  const int64_t R = PIC1DP_GAUSS_ROUND, npairs = R / 2, nblk = (npairs + PIC1DP_GAUSS_TILE - 1) / PIC1DP_GAUSS_TILE;
+  if (!h->d_gauss_words) CK(cudaMalloc(&h->d_gauss_words, (size_t)R * 8));
+  if (!h->d_gauss_bcount) CK(cudaMalloc(&h->d_gauss_bcount, (size_t)nblk * sizeof(unsigned)));
+  if (!h->d_gauss_ctl) CK(cudaMalloc(&h->d_gauss_ctl, sizeof(GaussCtl)));
+  GaussCtl *ctl = (GaussCtl *)h->d_gauss_ctl;
+  GaussCtl c = {0ULL, -1LL, 0.0};
+  CK(cudaMemcpyAsync(ctl, &c, sizeof(c), cudaMemcpyHostToDevice, h->stream));
+  h->h2d += sizeof(c);
+  const double2 *words = (const double2 *)h->d_gauss_words;
+  for (int64_t a = 0;; a += R) {
+    int rc = produce(a, h->d_gauss_words);
+    if (rc) return rc;
+    const int64_t base = (int64_t)c.total;
+    k_gauss_count<<<(unsigned)nblk, PIC1DP_GAUSS_THREADS, 0, h->stream>>>(words, npairs, h->d_gauss_bcount, ctl);
+    CKL(h);
+    k_gauss_scatter<<<(unsigned)nblk, PIC1DP_GAUSS_THREADS, 0, h->stream>>>(words, npairs, h->d_gauss_bcount, base, a, lo,
+                                                                          need, np, nlocal, d_v, ctl);
+    CKL(h);
+    CK(cudaMemcpyAsync(&c, ctl, sizeof(c), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    h->d2h += sizeof(c);
+    h->gauss_rounds++;
+    if ((int64_t)c.total >= need) break;
+  }
+  out.cut = c.cut;
+  if (out.filled) out.buf = c.spare;
+  return PIC1DP_OK;
+}
+
+static int maxwellian_check_args(pic1dp_gpu_t *h, const char *who, int32_t isp, int64_t np, int64_t nlocal,
+                                 int64_t nparticle_init, const void *seeds, const int32_t *gauss_filled,
+                                 const double *gauss_buf, int32_t init_nmode, const int32_t *init_mode,
+                                 const double *init_mode_cos, const double *init_mode_sin) {
+  int rc = load_check_args(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if (h->p.iptcldist != 0) {  // input_init: "case of input_iptcldist >= 1 and input_imarker = 1 not implemented yet"
+    h->err = std::string(who) + ": input_imarker = 1 supports only iptcldist = 0 (src/pic1dp_input.F90:291-299)";
+    return PIC1DP_EINVAL;
+  }
+  if (!seeds || !gauss_filled || !gauss_buf || nlocal < np) {
+    h->err = std::string(who) + ": bad stream argument (NULL state or nlocal < np)";
+    return PIC1DP_EINVAL;
+  }
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_load_markers_maxwellian_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                              int64_t nparticle_init, uint64_t seeds[4], int32_t *gauss_filled,
+                                              double *gauss_buf, int32_t init_nmode, const int32_t *init_mode,
+                                              const double *init_mode_cos, const double *init_mode_sin) {
+  int rc = maxwellian_check_args(h, "load_markers_maxwellian_kiss64", isp, np, nlocal, nparticle_init, seeds,
+                                 gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  CK(cudaSetDevice(h->p.device));
+  Species &S = h->sp[isp];
+  GaussResult g;
+  rc = gauss_stream_device(h, np, nlocal, *gauss_filled, *gauss_buf, S.v[0], g, [&](int64_t a, double *d) -> int {
+    return kiss64_fill_device(h, seeds, a, PIC1DP_GAUSS_ROUND, d, true);
+  });
+  if (rc) return rc;
+  // multirand_real_array(px) (:222): from the first draw after the last attempt; its unloaded tail is not generated
+  if ((rc = kiss64_fill_device(h, seeds, g.cut, np, S.x[0]))) return rc;
+  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
+    return rc;
+  Kiss64 s = {seeds[0], seeds[1], seeds[2], seeds[3]};
+  kiss64_jump_host(s, (uint64_t)(g.cut + nlocal));
+  seeds[0] = s.x; seeds[1] = s.xs; seeds[2] = s.z; seeds[3] = s.c;
+  *gauss_filled = g.filled;
+  *gauss_buf = g.buf;
+  h->gauss_draws = g.cut;
+  h->gauss_regenerated = 0;
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_load_markers_maxwellian_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                                   int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED],
+                                                   int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
+                                                   int32_t init_nmode, const int32_t *init_mode,
+                                                   const double *init_mode_cos, const double *init_mode_sin) {
+  int rc = maxwellian_check_args(h, "load_markers_maxwellian_superkiss64", isp, np, nlocal, nparticle_init, seeds,
+                                 gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if (sk_bad_state(seeds, iseed)) {
+    h->err = "load_markers_maxwellian_superkiss64: table position outside [0, 20632]";
+    return PIC1DP_EINVAL;
+  }
+  CK(cudaSetDevice(h->p.device));
+  if ((rc = kiss_tables(h))) return rc;
+  Species &S = h->sp[isp];
+  const size_t state_bytes = (PIC1DP_SK_N + 1) * sizeof(uint64_t);
+  if (!h->d_sk_state) CK(cudaMalloc(&h->d_sk_state, state_bytes));
+  if (!h->d_sk_round) CK(cudaMalloc(&h->d_sk_round, state_bytes));
+  const uint64_t lcg0 = seeds[PIC1DP_SK_N + 1], xs0 = seeds[PIC1DP_SK_N + 2];
+  CK(cudaMemcpyAsync(h->d_sk_state, seeds, state_bytes, cudaMemcpyHostToDevice, h->stream));
+  h->h2d += state_bytes;
+  // the table cannot be jumped back: each round starts from a copy of it, from which the x stream is regenerated
+  int64_t round_start = 0;
+  int32_t round_pos = *iseed;
+  bool saved = false;
+  GaussResult g;
+  rc = gauss_stream_device(h, np, nlocal, *gauss_filled, *gauss_buf, S.v[0], g, [&](int64_t a, double *d) -> int {
+    CK(cudaMemcpyAsync(h->d_sk_round, h->d_sk_state, state_bytes, cudaMemcpyDeviceToDevice, h->stream));
+    saved = true;
+    round_start = a;
+    round_pos = sk_iseed_after(*iseed, a);
+    int rc2 = superkiss64_table_device(h, round_pos, PIC1DP_GAUSS_ROUND, d, PIC1DP_GAUSS_ROUND, nullptr, 0, 0);
+    return rc2 ? rc2 : superkiss64_finish_device(h, lcg0, xs0, a, PIC1DP_GAUSS_ROUND, d, true);
+  });
+  if (rc) return rc;
+  // multirand_real_array(px) (:222): rerun the table from the start of the cut's round over the rest of that round's
+  // attempts and the nlocal draws of px, keeping the first np of them
+  if (saved) CK(cudaMemcpyAsync(h->d_sk_state, h->d_sk_round, state_bytes, cudaMemcpyDeviceToDevice, h->stream));
+  const int64_t skip = g.cut - round_start;
+  if (skip + nlocal > 0 && (rc = superkiss64_table_device(h, round_pos, skip + nlocal, nullptr, 0, S.x[0], skip, np)))
+    return rc;
+  if ((rc = superkiss64_finish_device(h, lcg0, xs0, g.cut, np, S.x[0]))) return rc;
+  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
+    return rc;
+  CK(cudaMemcpyAsync(seeds, h->d_sk_state, state_bytes, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->d2h += state_bytes;
+  const int64_t ntot = g.cut + nlocal;
+  seeds[PIC1DP_SK_N + 1] = sk_lcg_jump(lcg0, (uint64_t)ntot);
+  seeds[PIC1DP_SK_N + 2] = sk_xs_jump(xs0, (uint64_t)ntot, kiss_xs_jump);
+  *iseed = sk_iseed_after(*iseed, ntot);
+  *gauss_filled = g.filled;
+  *gauss_buf = g.buf;
+  h->gauss_draws = g.cut;
+  h->gauss_regenerated = skip;
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_last_gaussian_load(pic1dp_gpu_t *h, int64_t *draws, int64_t *rounds, int64_t *regenerated) {
+  if (!h || !draws || !rounds || !regenerated) return PIC1DP_EINVAL;
+  *draws = h->gauss_draws;
+  *rounds = h->gauss_rounds;
+  *regenerated = h->gauss_regenerated;
   return PIC1DP_OK;
 }
 

@@ -166,6 +166,45 @@ class Pic1dGpu:
                  "load_markers_superkiss64")
         return pos.value
 
+    def load_markers_maxwellian_kiss64(self, isp: int, n: int, nlocal: int, seeds, gauss_filled: int, gauss_buf: float,
+                                       nparticle_init: int, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)):
+        """Device-side particle_load for input_imarker = 1 with both streams (gaussian_array(pv, nlocal), then
+        real_array(px, nlocal)) generated on the device by KISS64.  seeds: multirand_seeds(0:3) as a C-contiguous uint64
+        array, advanced IN PLACE past every draw; (gauss_filled, gauss_buf): the Gaussian one-slot buffer before the
+        call.  Returns the buffer after it."""
+        assert seeds.dtype == np.uint64 and seeds.size == 4 and seeds.flags["C_CONTIGUOUS"], \
+            "KISS64 state: C-contiguous uint64 array of 4 words"
+        nm = len(init_mode)
+        im = (C.c_int32 * nm)(*init_mode)
+        ic = (C.c_double * nm)(*init_cos)
+        isn = (C.c_double * nm)(*init_sin)
+        filled, buf = C.c_int32(int(gauss_filled)), C.c_double(float(gauss_buf))
+        self._ck(self.L.pic1dp_gpu_load_markers_maxwellian_kiss64(
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), seeds.ctypes.data_as(C.POINTER(C.c_uint64)),
+            C.byref(filled), C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_kiss64")
+        return filled.value, buf.value
+
+    def load_markers_maxwellian_superkiss64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, gauss_filled: int,
+                                            gauss_buf: float, nparticle_init: int, init_mode=(1,), init_cos=(0.0,),
+                                            init_sin=(1e-5,)):
+        """The same with SuperKISS64: seeds = multirand_seeds(0:20634) (advanced in place), iseed = the table position.
+        Returns (iseed, gauss_filled, gauss_buf) after the call."""
+        nm = len(init_mode)
+        im = (C.c_int32 * nm)(*init_mode)
+        ic = (C.c_double * nm)(*init_cos)
+        isn = (C.c_double * nm)(*init_sin)
+        pos, filled, buf = C.c_int32(int(iseed)), C.c_int32(int(gauss_filled)), C.c_double(float(gauss_buf))
+        self._ck(self.L.pic1dp_gpu_load_markers_maxwellian_superkiss64(
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _u64p(seeds), C.byref(pos), C.byref(filled),
+            C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_superkiss64")
+        return pos.value, filled.value, buf.value
+
+    def last_gaussian_load(self):
+        """(draws the Gaussian call consumed, rounds, SuperKISS64 draws regenerated) of the last Maxwellian load."""
+        d, r, g = C.c_int64(), C.c_int64(), C.c_int64()
+        self._ck(self.L.pic1dp_gpu_last_gaussian_load(self._h, C.byref(d), C.byref(r), C.byref(g)), "last_gaussian_load")
+        return d.value, r.value, g.value
+
     def superkiss64_uniforms(self, seeds, iseed: int, n: int):
         """(n uniforms of the device SuperKISS64 stream, table position after them); seeds advanced in place."""
         out = np.empty(n)
