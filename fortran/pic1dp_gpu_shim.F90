@@ -155,6 +155,31 @@ interface
     real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
     integer(c_int32_t), intent(in) :: init_mode(*)
   end function
+  integer(c_int) function pic1dp_gpu_load_markers_mt19937_64(handle, isp, np, nlocal, nparticle_init, seeds, iseed, &
+      v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin) bind(c, name = 'pic1dp_gpu_load_markers_mt19937_64')
+    import :: c_ptr, c_int, c_int32_t, c_int64_t, c_double
+    type(c_ptr), value :: handle
+    integer(c_int32_t), value :: isp, init_nmode
+    integer(c_int64_t), value :: np, nlocal, nparticle_init
+    integer(c_int64_t), intent(inout) :: seeds(312)   ! multirand_seeds(0:311), same bits as the C uint64_t
+    integer(c_int32_t), intent(inout) :: iseed
+    real(c_double), value :: v_max
+    real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
+    integer(c_int32_t), intent(in) :: init_mode(*)
+  end function
+  integer(c_int) function pic1dp_gpu_load_markers_maxwellian_mt19937_64(handle, isp, np, nlocal, nparticle_init, &
+      seeds, iseed, gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin) &
+      bind(c, name = 'pic1dp_gpu_load_markers_maxwellian_mt19937_64')
+    import :: c_ptr, c_int, c_int32_t, c_int64_t, c_double
+    type(c_ptr), value :: handle
+    integer(c_int32_t), value :: isp, init_nmode
+    integer(c_int64_t), value :: np, nlocal, nparticle_init
+    integer(c_int64_t), intent(inout) :: seeds(312)   ! multirand_seeds(0:311), same bits as the C uint64_t
+    integer(c_int32_t), intent(inout) :: iseed, gauss_filled
+    real(c_double), intent(inout) :: gauss_buf
+    real(c_double), intent(in) :: init_mode_cos(*), init_mode_sin(*)
+    integer(c_int32_t), intent(in) :: init_mode(*)
+  end function
   integer(c_int) function pic1dp_gpu_output_all(handle, nx_opd, nv_opd, v_max, scalars, dist) &
       bind(c, name = 'pic1dp_gpu_output_all')
     import :: c_ptr, c_int, c_int32_t, c_double
@@ -276,6 +301,7 @@ public :: pic1dp_gpu_particle_split
 public :: pic1dp_gpu_load_markers_kiss64, pic1dp_host_kiss64_jump, pic1dp_gpu_output_all
 public :: pic1dp_gpu_load_markers_superkiss64
 public :: pic1dp_gpu_load_markers_maxwellian_kiss64, pic1dp_gpu_load_markers_maxwellian_superkiss64
+public :: pic1dp_gpu_load_markers_mt19937_64, pic1dp_gpu_load_markers_maxwellian_mt19937_64
 
 end module pic1dp_gpu
 
@@ -484,6 +510,50 @@ CHKERRQ(global_ierr)
 multirand_seeds(0 : 20634) = seeds(1 : 20635)
 multirand_iseed = iseed
 end subroutine gpu_particle_load_maxwellian_superkiss64
+
+! particle_load with input_multirand_al_int = 2 (MT19937-64): no marker-sized host-to-device copy.  Call in place of the
+! two multirand_real_array calls (src/pic1dp_particle.F90:180, :222) AFTER multirand_init (:159-160).  The device
+! generates exactly the 2 * nlocal numbers those calls would have drawn and returns the advanced state (the block that
+! holds the last draw and the position after it), which is copied back into the multirand module so that later draws
+! (particle_remove, particle_split) continue the same stream.  nlocal = particle_ip_high - particle_ip_low.
+subroutine gpu_particle_load_mt19937_64(ispecies, np, nlocal)
+use multirand, only : multirand_seeds, multirand_iseed
+implicit none
+#include "finclude/petsc.h90"
+PetscInt, intent(in) :: ispecies, np, nlocal
+integer(c_int64_t) :: seeds(312)
+integer(c_int32_t) :: iseed
+seeds(1 : 312) = multirand_seeds(0 : 311)
+iseed = int(multirand_iseed, c_int32_t)
+global_ierr = pic1dp_gpu_load_markers_mt19937_64(gpu_handle, int(ispecies - 1, c_int32_t), int(np, c_int64_t), &
+  int(nlocal, c_int64_t), int(input_species_nparticle_init(ispecies), c_int64_t), seeds, iseed, &
+  real(input_v_max, c_double), int(input_init_nmode, c_int32_t), int(input_init_mode, c_int32_t), &
+  real(input_init_mode_cos, c_double), real(input_init_mode_sin, c_double))
+CHKERRQ(global_ierr)
+multirand_seeds(0 : 311) = seeds(1 : 312)
+multirand_iseed = iseed
+end subroutine gpu_particle_load_mt19937_64
+
+! the Maxwellian form (input_imarker = 1) with MT19937-64, used like gpu_particle_load_maxwellian_kiss64
+subroutine gpu_particle_load_maxwellian_mt19937_64(ispecies, np, nlocal, gauss_filled, gauss_buf)
+use multirand, only : multirand_seeds, multirand_iseed
+implicit none
+#include "finclude/petsc.h90"
+PetscInt, intent(in) :: ispecies, np, nlocal
+integer(c_int32_t), intent(inout) :: gauss_filled
+real(c_double), intent(inout) :: gauss_buf
+integer(c_int64_t) :: seeds(312)
+integer(c_int32_t) :: iseed
+seeds(1 : 312) = multirand_seeds(0 : 311)
+iseed = int(multirand_iseed, c_int32_t)
+global_ierr = pic1dp_gpu_load_markers_maxwellian_mt19937_64(gpu_handle, int(ispecies - 1, c_int32_t), &
+  int(np, c_int64_t), int(nlocal, c_int64_t), int(input_species_nparticle_init(ispecies), c_int64_t), seeds, iseed, &
+  gauss_filled, gauss_buf, int(input_init_nmode, c_int32_t), int(input_init_mode, c_int32_t), &
+  real(input_init_mode_cos, c_double), real(input_init_mode_sin, c_double))
+CHKERRQ(global_ierr)
+multirand_seeds(0 : 311) = seeds(1 : 312)
+multirand_iseed = iseed
+end subroutine gpu_particle_load_maxwellian_mt19937_64
 
 ! before output_all / particle_optimize (src/pic1dp_output.F90:128-150, :228-237): device -> host Vecs
 subroutine gpu_particle_refresh_host(ispecies, vx, vv, vp, vw)

@@ -235,9 +235,8 @@ int pic1dp_gpu_load_markers_maxwellian(pic1dp_gpu_t *h, int32_t isp, int64_t np,
  * (LCG, xorshift, multiply-with-carry) to its chunk in O(log offset) and then runs the sequential generator; the
  * uniforms are INT2REAL64 of its outputs (:49).  Afterwards the host advances its own state with
  * pic1dp_host_kiss64_jump(seeds, 2 * nlocal * nspecies) so that later draws (particle_remove, particle_split)
- * continue the same stream.  SuperKISS64 (al_int = 3) has its own loader below, and both generators have a
- * Maxwellian loader (input_imarker = 1) below; MT19937-64 (al_int = 2) streams keep coming from the host through
- * load_markers / load_markers_maxwellian.
+ * continue the same stream.  SuperKISS64 (al_int = 3) and MT19937-64 (al_int = 2) have their own loaders below, and
+ * every generator has a Maxwellian loader (input_imarker = 1) below.
  */
 int pic1dp_gpu_load_markers_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nparticle_init,
                                    const uint64_t seeds[4], int64_t offset_v, int64_t offset_x, double v_max,
@@ -300,7 +299,7 @@ int pic1dp_gpu_load_markers_maxwellian_superkiss64(pic1dp_gpu_t *h, int32_t isp,
                                                    int32_t init_nmode, const int32_t *init_mode,
                                                    const double *init_mode_cos, const double *init_mode_sin);
 /* the last Maxwellian load of this handle: draws its Gaussian call consumed, rounds it ran, and the SuperKISS64 draws
- * it generated a second time for the x stream (0 for KISS64) */
+ * it generated a second time for the x stream (0 for KISS64 and MT19937-64) */
 int pic1dp_gpu_last_gaussian_load(pic1dp_gpu_t *h, int64_t *draws, int64_t *rounds, int64_t *regenerated);
 
 /* debug / parity: n uniforms of the device KISS64 stream starting at `offset`, copied to the host */
@@ -323,6 +322,40 @@ int pic1dp_host_superkiss64_fill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32
 int pic1dp_host_superkiss64_refill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t nchunks);
 void pic1dp_host_counter_uniforms(uint64_t seed, int32_t stream, int64_t first_index, int64_t n, double *u_v,
                                   double *u_x);
+
+/*
+ * load_markers_mt19937_64: load_markers with the two uniform streams generated ON THE DEVICE by the 64-bit Mersenne
+ * Twister, the generator multirand_al_int = 2 selects (src/multirand.F90:952-997), bit for bit.  seeds =
+ * multirand_seeds(0:311) and *iseed = the block position (0 .. 312), both as multirand_init (or earlier draws) left them.
+ * The device draws in particle_load's order: nlocal numbers for pv (:180), then nlocal for px (:222), nlocal =
+ * particle_ip_high - particle_ip_low >= np; the unloaded tail of each array is generated and discarded.  The generator
+ * is linear over GF(2): a window of 312 generated words jumps ahead by an XOR of shifted windows over the set bits of a
+ * jump polynomial (t^J mod the characteristic polynomial), which forms the start states of chunks of 2^16 words as a
+ * doubling tree; each chunk is then twisted sequentially by one CTA.  Before returning, seeds and *iseed are overwritten
+ * with the state after the 2 * nlocal draws: seeds = the block that holds the last draw, *iseed = the position after
+ * it (which can be 312), so later host draws (particle_remove, particle_split) continue the same stream.
+ * load_markers_maxwellian_mt19937_64 is the Maxwellian loader (input_imarker = 1) with the same state and the Gaussian
+ * one-slot buffer, as load_markers_maxwellian_superkiss64 (each round ends with the next round's start block on the
+ * device; the x stream starts from a chunk state of the round that holds the cut).  PIC1DP_EINVAL for *iseed outside
+ * [0, 312], nlocal < np, NULL pointers or (Maxwellian) iptcldist != 0, PIC1DP_ECAPACITY for np > capacity; a refused
+ * call leaves the state untouched.
+ */
+#define PIC1DP_MT19937_64_NSEED 312 /* multirand_seeds(0:311) */
+int pic1dp_gpu_load_markers_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal, int64_t nparticle_init,
+                                       uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, double v_max,
+                                       int32_t init_nmode, const int32_t *init_mode, const double *init_mode_cos,
+                                       const double *init_mode_sin);
+int pic1dp_gpu_load_markers_maxwellian_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                                  int64_t nparticle_init, uint64_t seeds[PIC1DP_MT19937_64_NSEED],
+                                                  int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
+                                                  int32_t init_nmode, const int32_t *init_mode,
+                                                  const double *init_mode_cos, const double *init_mode_sin);
+/* parity: n uniforms of the device MT19937-64 stream from (seeds, *iseed), copied to the host; the state is advanced
+ * past them like load_markers_mt19937_64 does */
+int pic1dp_gpu_mt19937_64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, int64_t n,
+                                   double *out);
+/* no handle, no GPU: (seeds, *iseed) advanced by n draws with the device's window-XOR jump, run on the host */
+int pic1dp_host_mt19937_64_jump(uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, int64_t n);
 
 /*
  * get_markers: D2H refresh of the host Vecs before pic1dp_output reads them (src/pic1dp_output.F90:128-150,

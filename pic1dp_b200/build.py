@@ -17,6 +17,9 @@ UNITS = [("pic1dp_gpu", "pic1dp_gpu.cu", [])] + \
 HEADERS = ["particle_kernels.cuh", "field_kernels.cuh", "diag_kernels.cuh", "optimize_kernels.cuh", "optimize_host.hpp",
            "push_tables.hpp", "fp_strict.cuh", "grid_device.cuh", "loader_kernels.cuh", "rng_kernels.cuh", "kiss_jump_tables.h"]
 OBJDIR = os.path.join(HERE, "build")
+# generated, not committed: the MT19937-64 jump polynomials, written into the object directory before compiling
+MT_GEN = os.path.join(HERE, "..", "tools_py3", "gen_mt_jump.py")
+MT_TABLES = "mt_jump_tables.h"
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",
@@ -38,7 +41,7 @@ def _headers():
 def _unit_hash(src, defines) -> str:
     import hashlib
     h = hashlib.sha256()
-    for d in [os.path.join(CSRC, src)] + _headers():
+    for d in [os.path.join(CSRC, src), MT_GEN] + _headers():
         h.update(open(d, "rb").read())
     h.update(" ".join(NVCC_FLAGS + defines + _extra_flags()).encode())
     return h.hexdigest()
@@ -67,7 +70,7 @@ def _compile_unit(args):
         return obj, ""
     nvcc = os.environ.get("NVCC", "nvcc")
     cmd = [nvcc] + NVCC_FLAGS + defines + _extra_flags() + (["-Xptxas", "-v"] if verbose else []) + \
-        ["-c", "-o", obj, os.path.join(CSRC, src)]
+        ["-I", objdir, "-c", "-o", obj, os.path.join(CSRC, src)]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + " ".join(cmd) + "\n" + r.stdout + r.stderr)
@@ -76,12 +79,22 @@ def _compile_unit(args):
     return obj, r.stderr
 
 
+def write_mt_tables(path: str) -> None:
+    """Run tools_py3/gen_mt_jump.py's generator into path (rewritten only when its text changes)."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("gen_mt_jump", MT_GEN)
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    mod.write(path)
+
+
 def build(force: bool = False, verbose: bool = False, lib: str = LIB, objdir: str = OBJDIR) -> str:
     """nvcc -c every unit (in parallel, content-hashed objects), then link the shared library in-tree."""
     if not (force or needs_build(lib)):
         return lib
     from concurrent.futures import ThreadPoolExecutor
     os.makedirs(objdir, exist_ok=True)
+    write_mt_tables(os.path.join(objdir, MT_TABLES))
     with ThreadPoolExecutor(max_workers=len(UNITS)) as ex:
         res = list(ex.map(_compile_unit, [(n, s, d, objdir, verbose, force) for n, s, d in UNITS]))
     if verbose:

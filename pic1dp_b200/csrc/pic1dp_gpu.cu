@@ -124,6 +124,10 @@ struct pic1dp_gpu {
   void *d_kiss_tab = nullptr;   // KissTables: jump-ahead tables of the device KISS64 (allocated on first use)
   uint64_t *d_sk_state = nullptr;   // SuperKISS64 table + carry advanced by k_superkiss64_table (allocated on first use)
   uint64_t *d_sk_round = nullptr;   // copy of d_sk_state at the start of the current Gaussian round
+  uint64_t *d_mt_poly = nullptr;     // MT19937-64 jump polynomials P_k (mt_jump_tables.h; allocated on first use)
+  uint64_t *d_mt_state = nullptr;    // MT19937-64 windows: the caller's block, two round states, the final block
+  uint64_t *d_mt_chunks = nullptr;   // MT19937-64 chunk start windows of the current stream (mt_chunks_cap windows)
+  int64_t mt_chunks_cap = 0;
   // Gaussian marker stream (allocated on first use): one round of raw words, per-CTA accept counts, GaussCtl
   double *d_gauss_words = nullptr;
   unsigned *d_gauss_bcount = nullptr;
@@ -383,6 +387,9 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
   if (h->d_kiss_tab) cudaFree(h->d_kiss_tab);
   if (h->d_sk_state) cudaFree(h->d_sk_state);
   if (h->d_sk_round) cudaFree(h->d_sk_round);
+  if (h->d_mt_poly) cudaFree(h->d_mt_poly);
+  if (h->d_mt_state) cudaFree(h->d_mt_state);
+  if (h->d_mt_chunks) cudaFree(h->d_mt_chunks);
   if (h->d_gauss_words) cudaFree(h->d_gauss_words);
   if (h->d_gauss_bcount) cudaFree(h->d_gauss_bcount);
   if (h->d_gauss_ctl) cudaFree(h->d_gauss_ctl);
@@ -1274,6 +1281,249 @@ int pic1dp_gpu_load_markers_maxwellian_superkiss64(pic1dp_gpu_t *h, int32_t isp,
   *gauss_buf = g.buf;
   h->gauss_draws = g.cut;
   h->gauss_regenerated = skip;
+  return PIC1DP_OK;
+}
+
+// ---- MT19937-64 on the device (rng_kernels.cuh) ----
+// Streams are addressed by "local words": word 0 is the first word of a window the caller holds on the device, and the
+// generated words follow it.  Every window a call starts from or hands back begins a reference block (a multiple of
+// 312 words from the caller's block), so the block that holds any later draw can be formed from it.
+#define PIC1DP_MT_LOG2_CHUNK 16   // words per k_mt64_fill CTA = 2^16
+static_assert(PIC1DP_MT_LOG2_CHUNK + 32 <= PIC1DP_MT_NK, "jump polynomials for the doubling tree");
+
+static bool mt_bad_state(const uint64_t *seeds, const int32_t *iseed) {
+  return !seeds || !iseed || *iseed < 0 || *iseed > PIC1DP_MT_N;
+}
+
+// the caller's block made a window of generated words: a block at iseed = 312 (multirand_init's, or fully used) is
+// twisted once, as the next draw would.  Only for calls that draw.
+static void mt_start_block(const uint64_t *seeds, int32_t iseed, uint64_t B[PIC1DP_MT_N], int64_t &p) {
+  memcpy(B, seeds, PIC1DP_MT_N * sizeof(uint64_t));
+  p = iseed;
+  if (p == PIC1DP_MT_N) {
+    mt64_twist_block(B);
+    p = 0;
+  }
+}
+
+// after the draws at local words [.., last] from the block at word 0: the block holding the last draw starts at word
+// mt_block_of(last), and iseed is the position after that draw (1 .. 312)
+static int64_t mt_block_of(int64_t last) { return last - last % PIC1DP_MT_N; }
+
+static int mt_alloc(pic1dp_gpu_t *h) {
+  if (!h->d_mt_poly) {
+    CK(cudaMalloc(&h->d_mt_poly, sizeof(mt_jump_poly)));
+    CK(cudaMemcpy(h->d_mt_poly, mt_jump_poly, sizeof(mt_jump_poly), cudaMemcpyHostToDevice));
+    h->h2d += sizeof(mt_jump_poly);
+  }
+  if (!h->d_mt_state) CK(cudaMalloc(&h->d_mt_state, 4 * PIC1DP_MT_N * sizeof(uint64_t)));
+  return PIC1DP_OK;
+}
+
+// Words of the stream that starts at the window src (device, local word 0): local word first + q is draw q, written
+// to d_a[q] (q < na) or d_b[q - pb] (0 <= q - pb < nb); save >= 0 also writes the window at local word save to
+// d_save.  Chunk c of 2^PIC1DP_MT_LOG2_CHUNK words starts from the window at word c * chunk: chunk 0 is src, and level
+// j of the doubling tree jumps chunks [0, 2^j) by P_{log2 chunk + j} to [2^j, 2^(j+1)).  The chunk windows stay in
+// h->d_mt_chunks until the next call (src may be one of them).
+static int mt_stream_device(pic1dp_gpu_t *h, const uint64_t *src, int64_t first, double *d_a, int64_t na, double *d_b,
+                            int64_t pb, int64_t nb, int64_t save, uint64_t *d_save, bool raw) {
+  const int64_t chunk = (int64_t)1 << PIC1DP_MT_LOG2_CHUNK;
+  int64_t last = first;   // the last local word the tree has to reach
+  if (na > 0) last = std::max(last, first + na - 1);
+  if (nb > 0) last = std::max(last, first + pb + nb - 1);
+  if (save >= 0) last = std::max(last, save + PIC1DP_MT_N - 1);
+  const int64_t nchunks = last / chunk + 1;
+  if (nchunks > h->mt_chunks_cap) {
+    // a window inside the old buffer (src) is copied out first
+    uint64_t *fresh = nullptr;
+    CK(cudaMalloc(&fresh, (size_t)nchunks * PIC1DP_MT_N * sizeof(uint64_t)));
+    CK(cudaMemcpyAsync(fresh, src, PIC1DP_MT_N * sizeof(uint64_t), cudaMemcpyDeviceToDevice, h->stream));
+    if (h->d_mt_chunks) {
+      CK(cudaStreamSynchronize(h->stream));
+      cudaFree(h->d_mt_chunks);
+    }
+    h->d_mt_chunks = fresh;
+    h->mt_chunks_cap = nchunks;
+  } else if (src != h->d_mt_chunks) {
+    CK(cudaMemcpyAsync(h->d_mt_chunks, src, PIC1DP_MT_N * sizeof(uint64_t), cudaMemcpyDeviceToDevice, h->stream));
+  }
+  const int smem = PIC1DP_MT_JUMP_WORDS * sizeof(uint64_t);
+  CK(cudaFuncSetAttribute(k_mt64_jump, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  for (int j = 0; ((int64_t)1 << j) < nchunks; j++) {
+    const int64_t half = (int64_t)1 << j;
+    const int64_t m = std::min(half, nchunks - half);
+    k_mt64_jump<<<(unsigned)m, PIC1DP_MT_JUMP_THREADS, smem, h->stream>>>(
+        h->d_mt_chunks, h->d_mt_chunks + half * PIC1DP_MT_N,
+        h->d_mt_poly + (size_t)(PIC1DP_MT_LOG2_CHUNK + j) * PIC1DP_MT_POLY_WORDS, 0);
+    CKL(h);
+  }
+  if (raw)
+    k_mt64_fill<true><<<(unsigned)nchunks, PIC1DP_MT_FILL_THREADS, 0, h->stream>>>(h->d_mt_chunks, chunk, first, d_a, na,
+                                                                                   d_b, pb, nb, save, d_save);
+  else
+    k_mt64_fill<<<(unsigned)nchunks, PIC1DP_MT_FILL_THREADS, 0, h->stream>>>(h->d_mt_chunks, chunk, first, d_a, na, d_b,
+                                                                             pb, nb, save, d_save);
+  CKL(h);
+  return PIC1DP_OK;
+}
+
+// draws [0, ntot) of the stream at (seeds, *iseed), placed as in mt_stream_device; on success seeds / *iseed hold the
+// state after them (synchronous copy of the final block)
+static int mt19937_64_fill_device(pic1dp_gpu_t *h, uint64_t *seeds, int32_t *iseed, int64_t ntot, double *d_a,
+                                  int64_t na, double *d_b, int64_t pb, int64_t nb) {
+  if (ntot == 0) return PIC1DP_OK;
+  int rc = mt_alloc(h);
+  if (rc) return rc;
+  uint64_t B[PIC1DP_MT_N];
+  int64_t p;
+  mt_start_block(seeds, *iseed, B, p);
+  const int64_t last = p + ntot - 1, T = mt_block_of(last);
+  uint64_t *d_src = h->d_mt_state, *d_fin = h->d_mt_state + 3 * PIC1DP_MT_N;
+  CK(cudaMemcpyAsync(d_src, B, sizeof(B), cudaMemcpyHostToDevice, h->stream));
+  h->h2d += sizeof(B);
+  if ((rc = mt_stream_device(h, d_src, p, d_a, na, d_b, pb, nb, T, d_fin, false))) return rc;
+  CK(cudaMemcpyAsync(B, d_fin, sizeof(B), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  h->d2h += sizeof(B);
+  memcpy(seeds, B, sizeof(B));
+  *iseed = (int32_t)(last - T + 1);
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_load_markers_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal, int64_t nparticle_init,
+                                       uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, double v_max,
+                                       int32_t init_nmode, const int32_t *init_mode, const double *init_mode_cos,
+                                       const double *init_mode_sin) {
+  int rc = load_check_args(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if (mt_bad_state(seeds, iseed) || nlocal < np) {
+    h->err = "load_markers_mt19937_64: bad stream argument (iseed in [0, 312], nlocal >= np)";
+    return PIC1DP_EINVAL;
+  }
+  CK(cudaSetDevice(h->p.device));
+  Species &S = h->sp[isp];
+  // multirand_real_array(pv) over the whole local array (:180), then multirand_real_array(px) (:222)
+  if ((rc = mt19937_64_fill_device(h, seeds, iseed, 2 * nlocal, S.v[0], np, S.x[0], nlocal, np))) return rc;
+  return load_markers_finish(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin, 2);
+}
+
+int pic1dp_gpu_mt19937_64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, int64_t n,
+                                   double *out) {
+  if (!h || mt_bad_state(seeds, iseed) || n < 0 || (n > 0 && !out)) {
+    if (h) h->err = "mt19937_64_uniforms: bad argument";
+    return PIC1DP_EINVAL;
+  }
+  if (n == 0) return PIC1DP_OK;
+  CK(cudaSetDevice(h->p.device));
+  double *d = nullptr;
+  CK(cudaMalloc(&d, (size_t)n * 8));
+  uint64_t s[PIC1DP_MT_N];
+  int32_t pos = *iseed;
+  memcpy(s, seeds, sizeof(s));
+  int rc = mt19937_64_fill_device(h, s, &pos, n, d, n, nullptr, 0, 0);
+  cudaError_t e = cudaSuccess;
+  if (!rc) {
+    e = cudaMemcpyAsync(out, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    h->d2h += n * 8;
+  }
+  cudaFree(d);
+  if (rc) return rc;
+  if (e != cudaSuccess) { h->err = std::string("mt19937_64_uniforms: ") + cudaGetErrorString(e); return PIC1DP_ECUDA; }
+  memcpy(seeds, s, sizeof(s));
+  *iseed = pos;
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_load_markers_maxwellian_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                                  int64_t nparticle_init, uint64_t seeds[PIC1DP_MT19937_64_NSEED],
+                                                  int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
+                                                  int32_t init_nmode, const int32_t *init_mode,
+                                                  const double *init_mode_cos, const double *init_mode_sin) {
+  int rc = maxwellian_check_args(h, "load_markers_maxwellian_mt19937_64", isp, np, nlocal, nparticle_init, seeds,
+                                 gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if (mt_bad_state(seeds, iseed)) {
+    h->err = "load_markers_maxwellian_mt19937_64: block position outside [0, 312]";
+    return PIC1DP_EINVAL;
+  }
+  CK(cudaSetDevice(h->p.device));
+  Species &S = h->sp[isp];
+  if (nlocal == 0) {   // no draw: the state stays as it is
+    h->gauss_draws = h->gauss_rounds = h->gauss_regenerated = 0;
+    return load_markers_finish(h, isp, 0, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1);
+  }
+  if ((rc = mt_alloc(h))) return rc;
+  uint64_t B[PIC1DP_MT_N];
+  int64_t p;
+  mt_start_block(seeds, *iseed, B, p);
+  // windows: [0] the caller's block (global word 0), [1] and [2] round start blocks in turn, [3] the final block
+  uint64_t *slot[4];
+  for (int k = 0; k < 4; k++) slot[k] = h->d_mt_state + k * PIC1DP_MT_N;
+  CK(cudaMemcpyAsync(slot[0], B, sizeof(B), cudaMemcpyHostToDevice, h->stream));
+  h->h2d += sizeof(B);
+  // Each round starts from the block that holds its first draw, which the round before saved; its chunk windows stay
+  // in h->d_mt_chunks, so the round that holds the cut also starts the x stream.
+  const int64_t R = PIC1DP_GAUSS_ROUND;
+  int cur = 0, next = 1;
+  int64_t g_cur = 0, g_next = 0;   // global word of the current round's start block, and of the next one's
+  bool any_round = false;
+  GaussResult g;
+  rc = gauss_stream_device(h, np, nlocal, *gauss_filled, *gauss_buf, S.v[0], g, [&](int64_t a, double *d) -> int {
+    if (a > 0) {
+      cur = next;
+      next = cur == 1 ? 2 : 1;
+      g_cur = g_next;
+    }
+    any_round = true;
+    g_next = mt_block_of(p + a + R);
+    return mt_stream_device(h, slot[cur], p + a - g_cur, d, R, nullptr, 0, 0, g_next - g_cur, slot[next], true);
+  });
+  if (rc) return rc;
+  // multirand_real_array(px) (:222): draws [cut, cut + nlocal), the first np kept.  It starts from the latest chunk
+  // window of the cut's round at or before both its first draw and the block of its last draw.
+  const int64_t x0 = p + g.cut, last = x0 + nlocal - 1, T = mt_block_of(last);
+  const uint64_t *src = slot[0];
+  int64_t base = 0;
+  if (any_round) {
+    const int64_t cc = (std::min(x0, T) - g_cur) >> PIC1DP_MT_LOG2_CHUNK;
+    src = h->d_mt_chunks + cc * PIC1DP_MT_N;
+    base = g_cur + (cc << PIC1DP_MT_LOG2_CHUNK);
+  }
+  if ((rc = mt_stream_device(h, src, x0 - base, S.x[0], np, nullptr, 0, 0, T - base, slot[3], false))) return rc;
+  CK(cudaMemcpyAsync(B, slot[3], sizeof(B), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
+    return rc;
+  h->d2h += sizeof(B);
+  memcpy(seeds, B, sizeof(B));
+  *iseed = (int32_t)(last - T + 1);
+  *gauss_filled = g.filled;
+  *gauss_buf = g.buf;
+  h->gauss_draws = g.cut;
+  h->gauss_regenerated = 0;
+  return PIC1DP_OK;
+}
+
+// the device's window-XOR jump run on the host: the state after n draws
+int pic1dp_host_mt19937_64_jump(uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, int64_t n) {
+  if (mt_bad_state(seeds, iseed) || n < 0) return PIC1DP_EINVAL;
+  if (n == 0) return PIC1DP_OK;
+  uint64_t B[PIC1DP_MT_N];
+  int64_t p;
+  mt_start_block(seeds, *iseed, B, p);
+  const int64_t last = p + n - 1, T = mt_block_of(last);
+  if ((uint64_t)T >> PIC1DP_MT_NK) return PIC1DP_EINVAL;
+  std::vector<uint64_t> w(PIC1DP_MT_JUMP_WORDS);
+  for (int k = 0; k < PIC1DP_MT_NK; k++) {
+    if (!((T >> k) & 1)) continue;
+    memcpy(w.data(), B, sizeof(B));
+    for (int m = 0; m + PIC1DP_MT_N < PIC1DP_MT_JUMP_WORDS; m++)
+      w[m + PIC1DP_MT_N] = mt64_next_word(w[m], w[m + 1], w[m + PIC1DP_MT_M]);
+    for (int j = 0; j < PIC1DP_MT_N; j++)
+      B[j] = mt64_window_xor(w.data(), mt_jump_poly[k], 0, PIC1DP_MT_POLY_WORDS, j);
+  }
+  memcpy(seeds, B, sizeof(B));
+  *iseed = (int32_t)(last - T + 1);
   return PIC1DP_OK;
 }
 

@@ -55,6 +55,13 @@ def _u64p(seeds: np.ndarray):
     return seeds.ctypes.data_as(C.POINTER(C.c_uint64))
 
 
+def _mt_u64p(seeds: np.ndarray):
+    """The MT19937-64 state multirand_seeds(0:311), passed for in-place update."""
+    assert seeds.dtype == np.uint64 and seeds.size == _capi.MT19937_64_NSEED and seeds.flags["C_CONTIGUOUS"], \
+        "MT19937-64 state: C-contiguous uint64 array of 312 words"
+    return seeds.ctypes.data_as(C.POINTER(C.c_uint64))
+
+
 def _ptr(addr: int):
     return C.cast(C.c_void_p(addr), C.POINTER(C.c_double))
 
@@ -198,6 +205,44 @@ class Pic1dGpu:
             self._h, isp, int(n), int(nlocal), int(nparticle_init), _u64p(seeds), C.byref(pos), C.byref(filled),
             C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_superkiss64")
         return pos.value, filled.value, buf.value
+
+    def load_markers_mt19937_64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, nparticle_init: int,
+                                v_max: float = 8.0, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)) -> int:
+        """Device-side particle_load with the device MT19937-64 stream (multirand_al_int = 2), bit-exact to multirand.
+        seeds: multirand_seeds(0:311) as a C-contiguous uint64 array, advanced IN PLACE past the 2 * nlocal draws;
+        iseed: the block position before them.  Returns the block position after them."""
+        nm = len(init_mode)
+        im = (C.c_int32 * nm)(*init_mode)
+        ic = (C.c_double * nm)(*init_cos)
+        isn = (C.c_double * nm)(*init_sin)
+        pos = C.c_int32(int(iseed))
+        self._ck(self.L.pic1dp_gpu_load_markers_mt19937_64(self._h, isp, int(n), int(nlocal), int(nparticle_init),
+                                                           _mt_u64p(seeds), C.byref(pos), float(v_max), nm, im, ic, isn),
+                 "load_markers_mt19937_64")
+        return pos.value
+
+    def load_markers_maxwellian_mt19937_64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, gauss_filled: int,
+                                           gauss_buf: float, nparticle_init: int, init_mode=(1,), init_cos=(0.0,),
+                                           init_sin=(1e-5,)):
+        """The Maxwellian loader with MT19937-64: seeds = multirand_seeds(0:311) (advanced in place), iseed = the block
+        position.  Returns (iseed, gauss_filled, gauss_buf) after the call."""
+        nm = len(init_mode)
+        im = (C.c_int32 * nm)(*init_mode)
+        ic = (C.c_double * nm)(*init_cos)
+        isn = (C.c_double * nm)(*init_sin)
+        pos, filled, buf = C.c_int32(int(iseed)), C.c_int32(int(gauss_filled)), C.c_double(float(gauss_buf))
+        self._ck(self.L.pic1dp_gpu_load_markers_maxwellian_mt19937_64(
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _mt_u64p(seeds), C.byref(pos), C.byref(filled),
+            C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_mt19937_64")
+        return pos.value, filled.value, buf.value
+
+    def mt19937_64_uniforms(self, seeds, iseed: int, n: int):
+        """(n uniforms of the device MT19937-64 stream, block position after them); seeds advanced in place."""
+        out = np.empty(n)
+        pos = C.c_int32(int(iseed))
+        self._ck(self.L.pic1dp_gpu_mt19937_64_uniforms(self._h, _mt_u64p(seeds), C.byref(pos), int(n), _dp(out)),
+                 "mt19937_64_uniforms")
+        return out, pos.value
 
     def last_gaussian_load(self):
         """(draws the Gaussian call consumed, rounds, SuperKISS64 draws regenerated) of the last Maxwellian load."""
@@ -654,3 +699,14 @@ def host_superkiss64_refill(seeds, nchunks: int):
     rc = _capi.load().pic1dp_host_superkiss64_refill(_u64p(seeds), int(nchunks))
     if rc:
         raise Pic1dpError(rc, "pic1dp_host_superkiss64_refill", "bad argument")
+
+
+
+def host_mt19937_64_jump(seeds, iseed: int, n: int) -> int:
+    """multirand_seeds(0:311) (uint64 array, in place) and the block position advanced by n draws with the device's
+    window-XOR jump run on the host.  Returns the block position after them."""
+    pos = C.c_int32(int(iseed))
+    rc = _capi.load().pic1dp_host_mt19937_64_jump(_mt_u64p(seeds), C.byref(pos), int(n))
+    if rc:
+        raise Pic1dpError(rc, "pic1dp_host_mt19937_64_jump", "bad argument")
+    return pos.value
