@@ -19,7 +19,6 @@
 #include <string.h>
 
 #include <algorithm>
-#include <functional>
 #include <string>
 #include <vector>
 
@@ -107,6 +106,22 @@ struct Species {
   SpeciesConst c;
 };
 
+// scratch of particle_load's device generators (each allocated on first use)
+struct RngScratch {
+  void *d_kiss_tab = nullptr;   // KissTables: jump-ahead tables of the device KISS64
+  uint64_t *d_sk_state = nullptr;   // SuperKISS64 table + carry advanced by k_superkiss64_table
+  uint64_t *d_sk_round = nullptr;   // copy of d_sk_state at the start of the current Gaussian round
+  uint64_t *d_mt_poly = nullptr;     // MT19937-64 jump polynomials P_k (mt_jump_tables.h)
+  uint64_t *d_mt_state = nullptr;    // MT19937-64 windows: the caller's block, two round states, the final block
+  uint64_t *d_mt_chunks = nullptr;   // MT19937-64 chunk start windows of the current stream (mt_chunks_cap windows)
+  int64_t mt_chunks_cap = 0;
+  // Gaussian marker stream: one round of raw words, per-CTA accept counts, GaussCtl
+  double *d_gauss_words = nullptr;
+  unsigned *d_gauss_bcount = nullptr;
+  void *d_gauss_ctl = nullptr;
+  int64_t gauss_draws = 0, gauss_rounds = 0, gauss_regenerated = 0;   // of the last Gaussian load
+};
+
 struct pic1dp_gpu {
   pic1dp_params p;
   cudaStream_t stream = nullptr;
@@ -121,18 +136,7 @@ struct pic1dp_gpu {
   double *d_E_start = nullptr;   // field of step()'s first substep, kept for the recomputed midpoint (ParticleArgs::E_start)
   double *d_Fre = nullptr, *d_Fim = nullptr, *d_ginv = nullptr;
   double *d_partial = nullptr, *d_red = nullptr, *d_energy = nullptr;
-  void *d_kiss_tab = nullptr;   // KissTables: jump-ahead tables of the device KISS64 (allocated on first use)
-  uint64_t *d_sk_state = nullptr;   // SuperKISS64 table + carry advanced by k_superkiss64_table (allocated on first use)
-  uint64_t *d_sk_round = nullptr;   // copy of d_sk_state at the start of the current Gaussian round
-  uint64_t *d_mt_poly = nullptr;     // MT19937-64 jump polynomials P_k (mt_jump_tables.h; allocated on first use)
-  uint64_t *d_mt_state = nullptr;    // MT19937-64 windows: the caller's block, two round states, the final block
-  uint64_t *d_mt_chunks = nullptr;   // MT19937-64 chunk start windows of the current stream (mt_chunks_cap windows)
-  int64_t mt_chunks_cap = 0;
-  // Gaussian marker stream (allocated on first use): one round of raw words, per-CTA accept counts, GaussCtl
-  double *d_gauss_words = nullptr;
-  unsigned *d_gauss_bcount = nullptr;
-  void *d_gauss_ctl = nullptr;
-  int64_t gauss_draws = 0, gauss_rounds = 0, gauss_regenerated = 0;   // of the last Gaussian load
+  RngScratch rng;
   unsigned long long *d_noob = nullptr;
   unsigned *d_wmax_hi = nullptr;              // [species] running max |deposit source| (high words), DEP_FIXED
   unsigned long long *d_dep_overflow = nullptr, *h_dep_overflow = nullptr;  // conversion overflows (+ pinned mirror)
@@ -384,15 +388,11 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
       else free(h->stage[q]);
     }
   if (h->d_noob) cudaFree(h->d_noob);
-  if (h->d_kiss_tab) cudaFree(h->d_kiss_tab);
-  if (h->d_sk_state) cudaFree(h->d_sk_state);
-  if (h->d_sk_round) cudaFree(h->d_sk_round);
-  if (h->d_mt_poly) cudaFree(h->d_mt_poly);
-  if (h->d_mt_state) cudaFree(h->d_mt_state);
-  if (h->d_mt_chunks) cudaFree(h->d_mt_chunks);
-  if (h->d_gauss_words) cudaFree(h->d_gauss_words);
-  if (h->d_gauss_bcount) cudaFree(h->d_gauss_bcount);
-  if (h->d_gauss_ctl) cudaFree(h->d_gauss_ctl);
+  RngScratch &R = h->rng;
+  void *rng_bufs[] = {R.d_kiss_tab, R.d_sk_state, R.d_sk_round, R.d_mt_poly, R.d_mt_state, R.d_mt_chunks,
+                      R.d_gauss_words, R.d_gauss_bcount, R.d_gauss_ctl};
+  for (void *b : rng_bufs)
+    if (b) cudaFree(b);
   if (h->d_wmax_hi) cudaFree(h->d_wmax_hi);
   if (h->d_dep_overflow) cudaFree(h->d_dep_overflow);
   if (h->d_hist_tab) cudaFree(h->d_hist_tab);
@@ -874,13 +874,13 @@ static int load_markers_impl(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t n
 
 // ---- device-side random streams (rng_kernels.cuh) ----
 static int kiss_tables(pic1dp_gpu_t *h) {
-  if (h->d_kiss_tab) return PIC1DP_OK;
+  if (h->rng.d_kiss_tab) return PIC1DP_OK;
   KissTables *t = new KissTables;
   memcpy(t->lcg, kiss_lcg_jump, sizeof(t->lcg));
   memcpy(t->mwc, kiss_mwc_jump, sizeof(t->mwc));
   memcpy(t->xs, kiss_xs_jump, sizeof(t->xs));
-  cudaError_t e = cudaMalloc(&h->d_kiss_tab, sizeof(KissTables));
-  if (e == cudaSuccess) e = cudaMemcpy(h->d_kiss_tab, t, sizeof(KissTables), cudaMemcpyHostToDevice);
+  cudaError_t e = cudaMalloc(&h->rng.d_kiss_tab, sizeof(KissTables));
+  if (e == cudaSuccess) e = cudaMemcpy(h->rng.d_kiss_tab, t, sizeof(KissTables), cudaMemcpyHostToDevice);
   delete t;
   if (e != cudaSuccess) { h->err = std::string("kiss tables: ") + cudaGetErrorString(e); return PIC1DP_ECUDA; }
   return PIC1DP_OK;
@@ -897,11 +897,11 @@ static int kiss64_fill_device(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t 
   const int64_t nchunks = (n + chunk - 1) / chunk;
   int blocks = (int)((nchunks + 127) / 128);
   if (blocks > h->nsm * 16) blocks = h->nsm * 16;
+  const KissTables *tab = (const KissTables *)h->rng.d_kiss_tab;
   if (raw)
-    k_kiss64_fill<true><<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, (const KissTables *)h->d_kiss_tab,
-                                                       d_out);
+    k_kiss64_fill<true><<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, tab, d_out);
   else
-    k_kiss64_fill<<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, (const KissTables *)h->d_kiss_tab, d_out);
+    k_kiss64_fill<<<blocks, 128, 0, h->stream>>>(s0, (uint64_t)offset, n, chunk, tab, d_out);
   CKL(h);
   return PIC1DP_OK;
 }
@@ -935,25 +935,6 @@ int pic1dp_gpu_load_markers_counter(pic1dp_gpu_t *h, int32_t isp, int64_t np, in
   return load_markers_finish(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin, 2);
 }
 
-int pic1dp_gpu_kiss64_uniforms(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t offset, int64_t n, double *out) {
-  if (!h || !seeds || offset < 0 || n < 0 || !out) { if (h) h->err = "kiss64_uniforms: bad argument"; return PIC1DP_EINVAL; }
-  if (n == 0) return PIC1DP_OK;
-  CK(cudaSetDevice(h->p.device));
-  double *d = nullptr;
-  CK(cudaMalloc(&d, (size_t)n * 8));
-  int rc = kiss64_fill_device(h, seeds, offset, n, d);
-  cudaError_t e = cudaSuccess;
-  if (!rc) {
-    e = cudaMemcpyAsync(out, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    h->d2h += n * 8;
-  }
-  cudaFree(d);
-  if (rc) return rc;
-  if (e != cudaSuccess) { h->err = std::string("kiss64_uniforms: ") + cudaGetErrorString(e); return PIC1DP_ECUDA; }
-  return PIC1DP_OK;
-}
-
 // the same generator on the host (no GPU): what a host does to keep its own multirand state in step with the numbers
 // the device consumed, and what the CPU tests use to check the jump tables
 int pic1dp_host_kiss64_jump(uint64_t seeds[4], int64_t n) {
@@ -977,11 +958,20 @@ static bool sk_bad_state(const uint64_t *seeds, const int32_t *iseed) {
   return !seeds || !iseed || *iseed < 0 || *iseed > PIC1DP_SK_N;
 }
 
+static const size_t SK_STATE_BYTES = (PIC1DP_SK_N + 1) * sizeof(uint64_t);   // the table and the carry
+
 // table position after ntot draws from position i0 (a refill happens lazily, at the draw that finds iseed = N)
 static int32_t sk_iseed_after(int32_t i0, int64_t ntot) {
   const int64_t rest = PIC1DP_SK_N - i0;
   if (ntot <= rest) return (int32_t)(i0 + ntot);
   return (int32_t)((ntot - rest - 1) % PIC1DP_SK_N + 1);
+}
+
+// the LCG, the xorshift and the table position of the host state after ntot draws (the table itself is the device's)
+static void sk_advance_host(uint64_t *seeds, int32_t *iseed, uint64_t lcg0, uint64_t xs0, int64_t ntot) {
+  seeds[PIC1DP_SK_N + 1] = sk_lcg_jump(lcg0, (uint64_t)ntot);
+  seeds[PIC1DP_SK_N + 2] = sk_xs_jump(xs0, (uint64_t)ntot, kiss_xs_jump);
+  *iseed = sk_iseed_after(*iseed, ntot);
 }
 
 // io[i] = the finished draw offset + i, i < n, from its raw table word (k_superkiss64_finish); (lcg0, xs0) = the LCG and
@@ -993,7 +983,7 @@ static int superkiss64_finish_device(pic1dp_gpu_t *h, uint64_t lcg0, uint64_t xs
   const int64_t nchunks = (n + chunk - 1) / chunk;
   int blocks = (int)((nchunks + 127) / 128);
   if (blocks > h->nsm * 16) blocks = h->nsm * 16;
-  const KissTables *tab = (const KissTables *)h->d_kiss_tab;
+  const KissTables *tab = (const KissTables *)h->rng.d_kiss_tab;
   if (raw)
     k_superkiss64_finish<true><<<blocks, 128, 0, h->stream>>>(lcg0, xs0, (uint64_t)offset, n, chunk, tab, io);
   else
@@ -1006,8 +996,16 @@ static int superkiss64_table_device(pic1dp_gpu_t *h, int32_t i0, int64_t ntot, d
                                     int64_t pb, int64_t nb) {
   const int smem = PIC1DP_SK_N * sizeof(uint64_t);
   CK(cudaFuncSetAttribute(k_superkiss64_table, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  k_superkiss64_table<<<1, PIC1DP_SK_THREADS, smem, h->stream>>>(h->d_sk_state, i0, ntot, d_a, na, d_b, pb, nb);
+  k_superkiss64_table<<<1, PIC1DP_SK_THREADS, smem, h->stream>>>(h->rng.d_sk_state, i0, ntot, d_a, na, d_b, pb, nb);
   CKL(h);
+  return PIC1DP_OK;
+}
+
+// the device table, loaded with the caller's table and carry
+static int sk_upload(pic1dp_gpu_t *h, const uint64_t *seeds) {
+  if (!h->rng.d_sk_state) CK(cudaMalloc(&h->rng.d_sk_state, SK_STATE_BYTES));
+  CK(cudaMemcpyAsync(h->rng.d_sk_state, seeds, SK_STATE_BYTES, cudaMemcpyHostToDevice, h->stream));
+  h->h2d += SK_STATE_BYTES;
   return PIC1DP_OK;
 }
 
@@ -1016,63 +1014,18 @@ static int superkiss64_table_device(pic1dp_gpu_t *h, int32_t i0, int64_t ntot, d
 // the table), so the host generator continues the same stream.
 static int superkiss64_fill_device(pic1dp_gpu_t *h, uint64_t *seeds, int32_t *iseed, int64_t ntot, double *d_a,
                                    int64_t na, double *d_b, int64_t pb, int64_t nb) {
-  int rc = kiss_tables(h);
+  int rc = kiss_tables(h);   // k_superkiss64_finish's jumps
   if (rc) return rc;
   if (ntot == 0) return PIC1DP_OK;
-  const size_t state_bytes = (PIC1DP_SK_N + 1) * sizeof(uint64_t);
-  if (!h->d_sk_state) CK(cudaMalloc(&h->d_sk_state, state_bytes));
   const uint64_t lcg0 = seeds[PIC1DP_SK_N + 1], xs0 = seeds[PIC1DP_SK_N + 2];
-  CK(cudaMemcpyAsync(h->d_sk_state, seeds, state_bytes, cudaMemcpyHostToDevice, h->stream));
-  h->h2d += state_bytes;
+  if ((rc = sk_upload(h, seeds))) return rc;
   if ((rc = superkiss64_table_device(h, *iseed, ntot, d_a, na, d_b, pb, nb))) return rc;
   if ((rc = superkiss64_finish_device(h, lcg0, xs0, 0, na, d_a))) return rc;
   if ((rc = superkiss64_finish_device(h, lcg0, xs0, pb, nb, d_b))) return rc;
-  CK(cudaMemcpyAsync(seeds, h->d_sk_state, state_bytes, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(seeds, h->rng.d_sk_state, SK_STATE_BYTES, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
-  h->d2h += state_bytes;
-  seeds[PIC1DP_SK_N + 1] = sk_lcg_jump(lcg0, (uint64_t)ntot);
-  seeds[PIC1DP_SK_N + 2] = sk_xs_jump(xs0, (uint64_t)ntot, kiss_xs_jump);
-  *iseed = sk_iseed_after(*iseed, ntot);
-  return PIC1DP_OK;
-}
-
-int pic1dp_gpu_load_markers_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
-                                        int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed,
-                                        double v_max, int32_t init_nmode, const int32_t *init_mode,
-                                        const double *init_mode_cos, const double *init_mode_sin) {
-  int rc = load_check_args(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
-  if (rc) return rc;
-  if (sk_bad_state(seeds, iseed) || nlocal < np) {
-    h->err = "load_markers_superkiss64: bad stream argument (iseed in [0, 20632], nlocal >= np)";
-    return PIC1DP_EINVAL;
-  }
-  CK(cudaSetDevice(h->p.device));
-  Species &S = h->sp[isp];
-  // multirand_real_array(pv) over the whole local array (:180), then multirand_real_array(px) (:222)
-  if ((rc = superkiss64_fill_device(h, seeds, iseed, 2 * nlocal, S.v[0], np, S.x[0], nlocal, np))) return rc;
-  return load_markers_finish(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin, 2);
-}
-
-int pic1dp_gpu_superkiss64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed, int64_t n,
-                                    double *out) {
-  if (!h || sk_bad_state(seeds, iseed) || n < 0 || (n > 0 && !out)) {
-    if (h) h->err = "superkiss64_uniforms: bad argument";
-    return PIC1DP_EINVAL;
-  }
-  if (n == 0) return PIC1DP_OK;
-  CK(cudaSetDevice(h->p.device));
-  double *d = nullptr;
-  CK(cudaMalloc(&d, (size_t)n * 8));
-  int rc = superkiss64_fill_device(h, seeds, iseed, n, d, n, nullptr, 0, 0);
-  cudaError_t e = cudaSuccess;
-  if (!rc) {
-    e = cudaMemcpyAsync(out, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    h->d2h += n * 8;
-  }
-  cudaFree(d);
-  if (rc) return rc;
-  if (e != cudaSuccess) { h->err = std::string("superkiss64_uniforms: ") + cudaGetErrorString(e); return PIC1DP_ECUDA; }
+  h->d2h += SK_STATE_BYTES;
+  sk_advance_host(seeds, iseed, lcg0, xs0, ntot);
   return PIC1DP_OK;
 }
 
@@ -1121,169 +1074,6 @@ int pic1dp_host_superkiss64_refill(uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int
   return PIC1DP_OK;
 }
 
-// ---- Maxwellian markers: multirand_gaussian_array(pv) on the device (rng_kernels.cuh) ----
-static_assert(PIC1DP_GAUSS_ROUND == PIC1DP_GAUSS_ROUND_DRAWS && PIC1DP_GAUSS_ROUND % 2 == 0, "Gaussian round size");
-struct GaussResult {
-  int64_t cut = 0;       // draws the Gaussian call consumed: the x stream starts here
-  int32_t filled = 0;    // the one-slot buffer after the call
-  double buf = 0.0;
-};
-
-// gaussian_array(pv, nlocal) from the raw-word stream that produce(a, d) writes (words [a, a + PIC1DP_GAUSS_ROUND) from
-// the call's first draw, into d), in rounds: words, accept counts, compaction into d_v (elements < np kept), then one
-// read of the running count.  The first round whose count reaches the attempts needed holds the cut.  (filled, buf) is
-// the caller's buffer on entry; the result carries it out, the caller's copy is left alone.
-static int gauss_stream_device(pic1dp_gpu_t *h, int64_t np, int64_t nlocal, int32_t filled, double buf, double *d_v,
-                               GaussResult &out, const std::function<int(int64_t, double *)> &produce) {
-  out = GaussResult();
-  out.filled = filled;
-  out.buf = buf;
-  h->gauss_rounds = 0;
-  if (nlocal == 0) return PIC1DP_OK;
-  int64_t lo = 0;
-  if (filled) {   // the buffered value is element 0; no draw for it
-    if (np > 0) {
-      CK(cudaMemcpyAsync(d_v, &buf, 8, cudaMemcpyHostToDevice, h->stream));
-      CK(cudaStreamSynchronize(h->stream));
-      h->h2d += 8;
-    }
-    lo = 1;
-  }
-  const int64_t need = (nlocal - lo + 1) / 2;   // accepted attempts
-  out.filled = (int32_t)((nlocal - lo) & 1);
-  if (need == 0) return PIC1DP_OK;
-  const int64_t R = PIC1DP_GAUSS_ROUND, npairs = R / 2, nblk = (npairs + PIC1DP_GAUSS_TILE - 1) / PIC1DP_GAUSS_TILE;
-  if (!h->d_gauss_words) CK(cudaMalloc(&h->d_gauss_words, (size_t)R * 8));
-  if (!h->d_gauss_bcount) CK(cudaMalloc(&h->d_gauss_bcount, (size_t)nblk * sizeof(unsigned)));
-  if (!h->d_gauss_ctl) CK(cudaMalloc(&h->d_gauss_ctl, sizeof(GaussCtl)));
-  GaussCtl *ctl = (GaussCtl *)h->d_gauss_ctl;
-  GaussCtl c = {0ULL, -1LL, 0.0};
-  CK(cudaMemcpyAsync(ctl, &c, sizeof(c), cudaMemcpyHostToDevice, h->stream));
-  h->h2d += sizeof(c);
-  const double2 *words = (const double2 *)h->d_gauss_words;
-  for (int64_t a = 0;; a += R) {
-    int rc = produce(a, h->d_gauss_words);
-    if (rc) return rc;
-    const int64_t base = (int64_t)c.total;
-    k_gauss_count<<<(unsigned)nblk, PIC1DP_GAUSS_THREADS, 0, h->stream>>>(words, npairs, h->d_gauss_bcount, ctl);
-    CKL(h);
-    k_gauss_scatter<<<(unsigned)nblk, PIC1DP_GAUSS_THREADS, 0, h->stream>>>(words, npairs, h->d_gauss_bcount, base, a, lo,
-                                                                          need, np, nlocal, d_v, ctl);
-    CKL(h);
-    CK(cudaMemcpyAsync(&c, ctl, sizeof(c), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    h->d2h += sizeof(c);
-    h->gauss_rounds++;
-    if ((int64_t)c.total >= need) break;
-  }
-  out.cut = c.cut;
-  if (out.filled) out.buf = c.spare;
-  return PIC1DP_OK;
-}
-
-static int maxwellian_check_args(pic1dp_gpu_t *h, const char *who, int32_t isp, int64_t np, int64_t nlocal,
-                                 int64_t nparticle_init, const void *seeds, const int32_t *gauss_filled,
-                                 const double *gauss_buf, int32_t init_nmode, const int32_t *init_mode,
-                                 const double *init_mode_cos, const double *init_mode_sin) {
-  int rc = load_check_args(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin);
-  if (rc) return rc;
-  if (h->p.iptcldist != 0) {  // input_init: "case of input_iptcldist >= 1 and input_imarker = 1 not implemented yet"
-    h->err = std::string(who) + ": input_imarker = 1 supports only iptcldist = 0 (src/pic1dp_input.F90:291-299)";
-    return PIC1DP_EINVAL;
-  }
-  if (!seeds || !gauss_filled || !gauss_buf || nlocal < np) {
-    h->err = std::string(who) + ": bad stream argument (NULL state or nlocal < np)";
-    return PIC1DP_EINVAL;
-  }
-  return PIC1DP_OK;
-}
-
-int pic1dp_gpu_load_markers_maxwellian_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
-                                              int64_t nparticle_init, uint64_t seeds[4], int32_t *gauss_filled,
-                                              double *gauss_buf, int32_t init_nmode, const int32_t *init_mode,
-                                              const double *init_mode_cos, const double *init_mode_sin) {
-  int rc = maxwellian_check_args(h, "load_markers_maxwellian_kiss64", isp, np, nlocal, nparticle_init, seeds,
-                                 gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
-  if (rc) return rc;
-  CK(cudaSetDevice(h->p.device));
-  Species &S = h->sp[isp];
-  GaussResult g;
-  rc = gauss_stream_device(h, np, nlocal, *gauss_filled, *gauss_buf, S.v[0], g, [&](int64_t a, double *d) -> int {
-    return kiss64_fill_device(h, seeds, a, PIC1DP_GAUSS_ROUND, d, true);
-  });
-  if (rc) return rc;
-  // multirand_real_array(px) (:222): from the first draw after the last attempt; its unloaded tail is not generated
-  if ((rc = kiss64_fill_device(h, seeds, g.cut, np, S.x[0]))) return rc;
-  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
-    return rc;
-  Kiss64 s = {seeds[0], seeds[1], seeds[2], seeds[3]};
-  kiss64_jump_host(s, (uint64_t)(g.cut + nlocal));
-  seeds[0] = s.x; seeds[1] = s.xs; seeds[2] = s.z; seeds[3] = s.c;
-  *gauss_filled = g.filled;
-  *gauss_buf = g.buf;
-  h->gauss_draws = g.cut;
-  h->gauss_regenerated = 0;
-  return PIC1DP_OK;
-}
-
-int pic1dp_gpu_load_markers_maxwellian_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
-                                                   int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED],
-                                                   int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
-                                                   int32_t init_nmode, const int32_t *init_mode,
-                                                   const double *init_mode_cos, const double *init_mode_sin) {
-  int rc = maxwellian_check_args(h, "load_markers_maxwellian_superkiss64", isp, np, nlocal, nparticle_init, seeds,
-                                 gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
-  if (rc) return rc;
-  if (sk_bad_state(seeds, iseed)) {
-    h->err = "load_markers_maxwellian_superkiss64: table position outside [0, 20632]";
-    return PIC1DP_EINVAL;
-  }
-  CK(cudaSetDevice(h->p.device));
-  if ((rc = kiss_tables(h))) return rc;
-  Species &S = h->sp[isp];
-  const size_t state_bytes = (PIC1DP_SK_N + 1) * sizeof(uint64_t);
-  if (!h->d_sk_state) CK(cudaMalloc(&h->d_sk_state, state_bytes));
-  if (!h->d_sk_round) CK(cudaMalloc(&h->d_sk_round, state_bytes));
-  const uint64_t lcg0 = seeds[PIC1DP_SK_N + 1], xs0 = seeds[PIC1DP_SK_N + 2];
-  CK(cudaMemcpyAsync(h->d_sk_state, seeds, state_bytes, cudaMemcpyHostToDevice, h->stream));
-  h->h2d += state_bytes;
-  // the table cannot be jumped back: each round starts from a copy of it, from which the x stream is regenerated
-  int64_t round_start = 0;
-  int32_t round_pos = *iseed;
-  bool saved = false;
-  GaussResult g;
-  rc = gauss_stream_device(h, np, nlocal, *gauss_filled, *gauss_buf, S.v[0], g, [&](int64_t a, double *d) -> int {
-    CK(cudaMemcpyAsync(h->d_sk_round, h->d_sk_state, state_bytes, cudaMemcpyDeviceToDevice, h->stream));
-    saved = true;
-    round_start = a;
-    round_pos = sk_iseed_after(*iseed, a);
-    int rc2 = superkiss64_table_device(h, round_pos, PIC1DP_GAUSS_ROUND, d, PIC1DP_GAUSS_ROUND, nullptr, 0, 0);
-    return rc2 ? rc2 : superkiss64_finish_device(h, lcg0, xs0, a, PIC1DP_GAUSS_ROUND, d, true);
-  });
-  if (rc) return rc;
-  // multirand_real_array(px) (:222): rerun the table from the start of the cut's round over the rest of that round's
-  // attempts and the nlocal draws of px, keeping the first np of them
-  if (saved) CK(cudaMemcpyAsync(h->d_sk_state, h->d_sk_round, state_bytes, cudaMemcpyDeviceToDevice, h->stream));
-  const int64_t skip = g.cut - round_start;
-  if (skip + nlocal > 0 && (rc = superkiss64_table_device(h, round_pos, skip + nlocal, nullptr, 0, S.x[0], skip, np)))
-    return rc;
-  if ((rc = superkiss64_finish_device(h, lcg0, xs0, g.cut, np, S.x[0]))) return rc;
-  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
-    return rc;
-  CK(cudaMemcpyAsync(seeds, h->d_sk_state, state_bytes, cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  h->d2h += state_bytes;
-  const int64_t ntot = g.cut + nlocal;
-  seeds[PIC1DP_SK_N + 1] = sk_lcg_jump(lcg0, (uint64_t)ntot);
-  seeds[PIC1DP_SK_N + 2] = sk_xs_jump(xs0, (uint64_t)ntot, kiss_xs_jump);
-  *iseed = sk_iseed_after(*iseed, ntot);
-  *gauss_filled = g.filled;
-  *gauss_buf = g.buf;
-  h->gauss_draws = g.cut;
-  h->gauss_regenerated = skip;
-  return PIC1DP_OK;
-}
-
 // ---- MT19937-64 on the device (rng_kernels.cuh) ----
 // Streams are addressed by "local words": word 0 is the first word of a window the caller holds on the device, and the
 // generated words follow it.  Every window a call starts from or hands back begins a reference block (a multiple of
@@ -1310,13 +1100,19 @@ static void mt_start_block(const uint64_t *seeds, int32_t iseed, uint64_t B[PIC1
 // mt_block_of(last), and iseed is the position after that draw (1 .. 312)
 static int64_t mt_block_of(int64_t last) { return last - last % PIC1DP_MT_N; }
 
-static int mt_alloc(pic1dp_gpu_t *h) {
-  if (!h->d_mt_poly) {
-    CK(cudaMalloc(&h->d_mt_poly, sizeof(mt_jump_poly)));
-    CK(cudaMemcpy(h->d_mt_poly, mt_jump_poly, sizeof(mt_jump_poly), cudaMemcpyHostToDevice));
+// the jump polynomials and the four windows of d_mt_state; then the caller's block at (seeds, iseed), made a window
+// (mt_start_block: B, *p), is uploaded to window 0
+static int mt_upload(pic1dp_gpu_t *h, const uint64_t *seeds, int32_t iseed, uint64_t B[PIC1DP_MT_N], int64_t *p) {
+  RngScratch &R = h->rng;
+  if (!R.d_mt_poly) {
+    CK(cudaMalloc(&R.d_mt_poly, sizeof(mt_jump_poly)));
+    CK(cudaMemcpy(R.d_mt_poly, mt_jump_poly, sizeof(mt_jump_poly), cudaMemcpyHostToDevice));
     h->h2d += sizeof(mt_jump_poly);
   }
-  if (!h->d_mt_state) CK(cudaMalloc(&h->d_mt_state, 4 * PIC1DP_MT_N * sizeof(uint64_t)));
+  if (!R.d_mt_state) CK(cudaMalloc(&R.d_mt_state, 4 * PIC1DP_MT_N * sizeof(uint64_t)));
+  mt_start_block(seeds, iseed, B, *p);
+  CK(cudaMemcpyAsync(R.d_mt_state, B, PIC1DP_MT_N * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+  h->h2d += PIC1DP_MT_N * sizeof(uint64_t);
   return PIC1DP_OK;
 }
 
@@ -1324,28 +1120,29 @@ static int mt_alloc(pic1dp_gpu_t *h) {
 // to d_a[q] (q < na) or d_b[q - pb] (0 <= q - pb < nb); save >= 0 also writes the window at local word save to
 // d_save.  Chunk c of 2^PIC1DP_MT_LOG2_CHUNK words starts from the window at word c * chunk: chunk 0 is src, and level
 // j of the doubling tree jumps chunks [0, 2^j) by P_{log2 chunk + j} to [2^j, 2^(j+1)).  The chunk windows stay in
-// h->d_mt_chunks until the next call (src may be one of them).
+// d_mt_chunks until the next call (src may be one of them).
 static int mt_stream_device(pic1dp_gpu_t *h, const uint64_t *src, int64_t first, double *d_a, int64_t na, double *d_b,
                             int64_t pb, int64_t nb, int64_t save, uint64_t *d_save, bool raw) {
+  RngScratch &R = h->rng;
   const int64_t chunk = (int64_t)1 << PIC1DP_MT_LOG2_CHUNK;
   int64_t last = first;   // the last local word the tree has to reach
   if (na > 0) last = std::max(last, first + na - 1);
   if (nb > 0) last = std::max(last, first + pb + nb - 1);
   if (save >= 0) last = std::max(last, save + PIC1DP_MT_N - 1);
   const int64_t nchunks = last / chunk + 1;
-  if (nchunks > h->mt_chunks_cap) {
+  if (nchunks > R.mt_chunks_cap) {
     // a window inside the old buffer (src) is copied out first
     uint64_t *fresh = nullptr;
     CK(cudaMalloc(&fresh, (size_t)nchunks * PIC1DP_MT_N * sizeof(uint64_t)));
     CK(cudaMemcpyAsync(fresh, src, PIC1DP_MT_N * sizeof(uint64_t), cudaMemcpyDeviceToDevice, h->stream));
-    if (h->d_mt_chunks) {
+    if (R.d_mt_chunks) {
       CK(cudaStreamSynchronize(h->stream));
-      cudaFree(h->d_mt_chunks);
+      cudaFree(R.d_mt_chunks);
     }
-    h->d_mt_chunks = fresh;
-    h->mt_chunks_cap = nchunks;
-  } else if (src != h->d_mt_chunks) {
-    CK(cudaMemcpyAsync(h->d_mt_chunks, src, PIC1DP_MT_N * sizeof(uint64_t), cudaMemcpyDeviceToDevice, h->stream));
+    R.d_mt_chunks = fresh;
+    R.mt_chunks_cap = nchunks;
+  } else if (src != R.d_mt_chunks) {
+    CK(cudaMemcpyAsync(R.d_mt_chunks, src, PIC1DP_MT_N * sizeof(uint64_t), cudaMemcpyDeviceToDevice, h->stream));
   }
   const int smem = PIC1DP_MT_JUMP_WORDS * sizeof(uint64_t);
   CK(cudaFuncSetAttribute(k_mt64_jump, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -1353,15 +1150,15 @@ static int mt_stream_device(pic1dp_gpu_t *h, const uint64_t *src, int64_t first,
     const int64_t half = (int64_t)1 << j;
     const int64_t m = std::min(half, nchunks - half);
     k_mt64_jump<<<(unsigned)m, PIC1DP_MT_JUMP_THREADS, smem, h->stream>>>(
-        h->d_mt_chunks, h->d_mt_chunks + half * PIC1DP_MT_N,
-        h->d_mt_poly + (size_t)(PIC1DP_MT_LOG2_CHUNK + j) * PIC1DP_MT_POLY_WORDS, 0);
+        R.d_mt_chunks, R.d_mt_chunks + half * PIC1DP_MT_N,
+        R.d_mt_poly + (size_t)(PIC1DP_MT_LOG2_CHUNK + j) * PIC1DP_MT_POLY_WORDS, 0);
     CKL(h);
   }
   if (raw)
-    k_mt64_fill<true><<<(unsigned)nchunks, PIC1DP_MT_FILL_THREADS, 0, h->stream>>>(h->d_mt_chunks, chunk, first, d_a, na,
+    k_mt64_fill<true><<<(unsigned)nchunks, PIC1DP_MT_FILL_THREADS, 0, h->stream>>>(R.d_mt_chunks, chunk, first, d_a, na,
                                                                                    d_b, pb, nb, save, d_save);
   else
-    k_mt64_fill<<<(unsigned)nchunks, PIC1DP_MT_FILL_THREADS, 0, h->stream>>>(h->d_mt_chunks, chunk, first, d_a, na, d_b,
+    k_mt64_fill<<<(unsigned)nchunks, PIC1DP_MT_FILL_THREADS, 0, h->stream>>>(R.d_mt_chunks, chunk, first, d_a, na, d_b,
                                                                              pb, nb, save, d_save);
   CKL(h);
   return PIC1DP_OK;
@@ -1372,135 +1169,18 @@ static int mt_stream_device(pic1dp_gpu_t *h, const uint64_t *src, int64_t first,
 static int mt19937_64_fill_device(pic1dp_gpu_t *h, uint64_t *seeds, int32_t *iseed, int64_t ntot, double *d_a,
                                   int64_t na, double *d_b, int64_t pb, int64_t nb) {
   if (ntot == 0) return PIC1DP_OK;
-  int rc = mt_alloc(h);
-  if (rc) return rc;
   uint64_t B[PIC1DP_MT_N];
   int64_t p;
-  mt_start_block(seeds, *iseed, B, p);
+  int rc = mt_upload(h, seeds, *iseed, B, &p);
+  if (rc) return rc;
   const int64_t last = p + ntot - 1, T = mt_block_of(last);
-  uint64_t *d_src = h->d_mt_state, *d_fin = h->d_mt_state + 3 * PIC1DP_MT_N;
-  CK(cudaMemcpyAsync(d_src, B, sizeof(B), cudaMemcpyHostToDevice, h->stream));
-  h->h2d += sizeof(B);
-  if ((rc = mt_stream_device(h, d_src, p, d_a, na, d_b, pb, nb, T, d_fin, false))) return rc;
+  uint64_t *d_fin = h->rng.d_mt_state + 3 * PIC1DP_MT_N;
+  if ((rc = mt_stream_device(h, h->rng.d_mt_state, p, d_a, na, d_b, pb, nb, T, d_fin, false))) return rc;
   CK(cudaMemcpyAsync(B, d_fin, sizeof(B), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   h->d2h += sizeof(B);
   memcpy(seeds, B, sizeof(B));
   *iseed = (int32_t)(last - T + 1);
-  return PIC1DP_OK;
-}
-
-int pic1dp_gpu_load_markers_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal, int64_t nparticle_init,
-                                       uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, double v_max,
-                                       int32_t init_nmode, const int32_t *init_mode, const double *init_mode_cos,
-                                       const double *init_mode_sin) {
-  int rc = load_check_args(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
-  if (rc) return rc;
-  if (mt_bad_state(seeds, iseed) || nlocal < np) {
-    h->err = "load_markers_mt19937_64: bad stream argument (iseed in [0, 312], nlocal >= np)";
-    return PIC1DP_EINVAL;
-  }
-  CK(cudaSetDevice(h->p.device));
-  Species &S = h->sp[isp];
-  // multirand_real_array(pv) over the whole local array (:180), then multirand_real_array(px) (:222)
-  if ((rc = mt19937_64_fill_device(h, seeds, iseed, 2 * nlocal, S.v[0], np, S.x[0], nlocal, np))) return rc;
-  return load_markers_finish(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin, 2);
-}
-
-int pic1dp_gpu_mt19937_64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, int64_t n,
-                                   double *out) {
-  if (!h || mt_bad_state(seeds, iseed) || n < 0 || (n > 0 && !out)) {
-    if (h) h->err = "mt19937_64_uniforms: bad argument";
-    return PIC1DP_EINVAL;
-  }
-  if (n == 0) return PIC1DP_OK;
-  CK(cudaSetDevice(h->p.device));
-  double *d = nullptr;
-  CK(cudaMalloc(&d, (size_t)n * 8));
-  uint64_t s[PIC1DP_MT_N];
-  int32_t pos = *iseed;
-  memcpy(s, seeds, sizeof(s));
-  int rc = mt19937_64_fill_device(h, s, &pos, n, d, n, nullptr, 0, 0);
-  cudaError_t e = cudaSuccess;
-  if (!rc) {
-    e = cudaMemcpyAsync(out, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    h->d2h += n * 8;
-  }
-  cudaFree(d);
-  if (rc) return rc;
-  if (e != cudaSuccess) { h->err = std::string("mt19937_64_uniforms: ") + cudaGetErrorString(e); return PIC1DP_ECUDA; }
-  memcpy(seeds, s, sizeof(s));
-  *iseed = pos;
-  return PIC1DP_OK;
-}
-
-int pic1dp_gpu_load_markers_maxwellian_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
-                                                  int64_t nparticle_init, uint64_t seeds[PIC1DP_MT19937_64_NSEED],
-                                                  int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
-                                                  int32_t init_nmode, const int32_t *init_mode,
-                                                  const double *init_mode_cos, const double *init_mode_sin) {
-  int rc = maxwellian_check_args(h, "load_markers_maxwellian_mt19937_64", isp, np, nlocal, nparticle_init, seeds,
-                                 gauss_filled, gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
-  if (rc) return rc;
-  if (mt_bad_state(seeds, iseed)) {
-    h->err = "load_markers_maxwellian_mt19937_64: block position outside [0, 312]";
-    return PIC1DP_EINVAL;
-  }
-  CK(cudaSetDevice(h->p.device));
-  Species &S = h->sp[isp];
-  if (nlocal == 0) {   // no draw: the state stays as it is
-    h->gauss_draws = h->gauss_rounds = h->gauss_regenerated = 0;
-    return load_markers_finish(h, isp, 0, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1);
-  }
-  if ((rc = mt_alloc(h))) return rc;
-  uint64_t B[PIC1DP_MT_N];
-  int64_t p;
-  mt_start_block(seeds, *iseed, B, p);
-  // windows: [0] the caller's block (global word 0), [1] and [2] round start blocks in turn, [3] the final block
-  uint64_t *slot[4];
-  for (int k = 0; k < 4; k++) slot[k] = h->d_mt_state + k * PIC1DP_MT_N;
-  CK(cudaMemcpyAsync(slot[0], B, sizeof(B), cudaMemcpyHostToDevice, h->stream));
-  h->h2d += sizeof(B);
-  // Each round starts from the block that holds its first draw, which the round before saved; its chunk windows stay
-  // in h->d_mt_chunks, so the round that holds the cut also starts the x stream.
-  const int64_t R = PIC1DP_GAUSS_ROUND;
-  int cur = 0, next = 1;
-  int64_t g_cur = 0, g_next = 0;   // global word of the current round's start block, and of the next one's
-  bool any_round = false;
-  GaussResult g;
-  rc = gauss_stream_device(h, np, nlocal, *gauss_filled, *gauss_buf, S.v[0], g, [&](int64_t a, double *d) -> int {
-    if (a > 0) {
-      cur = next;
-      next = cur == 1 ? 2 : 1;
-      g_cur = g_next;
-    }
-    any_round = true;
-    g_next = mt_block_of(p + a + R);
-    return mt_stream_device(h, slot[cur], p + a - g_cur, d, R, nullptr, 0, 0, g_next - g_cur, slot[next], true);
-  });
-  if (rc) return rc;
-  // multirand_real_array(px) (:222): draws [cut, cut + nlocal), the first np kept.  It starts from the latest chunk
-  // window of the cut's round at or before both its first draw and the block of its last draw.
-  const int64_t x0 = p + g.cut, last = x0 + nlocal - 1, T = mt_block_of(last);
-  const uint64_t *src = slot[0];
-  int64_t base = 0;
-  if (any_round) {
-    const int64_t cc = (std::min(x0, T) - g_cur) >> PIC1DP_MT_LOG2_CHUNK;
-    src = h->d_mt_chunks + cc * PIC1DP_MT_N;
-    base = g_cur + (cc << PIC1DP_MT_LOG2_CHUNK);
-  }
-  if ((rc = mt_stream_device(h, src, x0 - base, S.x[0], np, nullptr, 0, 0, T - base, slot[3], false))) return rc;
-  CK(cudaMemcpyAsync(B, slot[3], sizeof(B), cudaMemcpyDeviceToHost, h->stream));
-  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
-    return rc;
-  h->d2h += sizeof(B);
-  memcpy(seeds, B, sizeof(B));
-  *iseed = (int32_t)(last - T + 1);
-  *gauss_filled = g.filled;
-  *gauss_buf = g.buf;
-  h->gauss_draws = g.cut;
-  h->gauss_regenerated = 0;
   return PIC1DP_OK;
 }
 
@@ -1527,12 +1207,345 @@ int pic1dp_host_mt19937_64_jump(uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t
   return PIC1DP_OK;
 }
 
+// ---- particle_load's uniform streams from the table generators (SuperKISS64, MT19937-64) ----
+// Their state is multirand_seeds plus a table / block position; bad_state refuses a NULL or out-of-range one, and fill
+// (superkiss64_fill_device / mt19937_64_fill_device) places the draws and advances the state.
+typedef bool (*TableBadState)(const uint64_t *seeds, const int32_t *iseed);
+typedef int (*TableFill)(pic1dp_gpu_t *h, uint64_t *seeds, int32_t *iseed, int64_t ntot, double *d_a, int64_t na,
+                         double *d_b, int64_t pb, int64_t nb);
+
+static int load_markers_table(pic1dp_gpu_t *h, const char *who, TableBadState bad_state, TableFill fill, int32_t isp,
+                              int64_t np, int64_t nlocal, int64_t nparticle_init, uint64_t *seeds, int32_t *iseed,
+                              double v_max, int32_t init_nmode, const int32_t *init_mode, const double *init_mode_cos,
+                              const double *init_mode_sin) {
+  int rc = load_check_args(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if (bad_state(seeds, iseed) || nlocal < np) {
+    h->err = std::string(who) + ": bad stream argument (NULL state, position out of range or nlocal < np)";
+    return PIC1DP_EINVAL;
+  }
+  CK(cudaSetDevice(h->p.device));
+  Species &S = h->sp[isp];
+  // multirand_real_array(pv) over the whole local array (:180), then multirand_real_array(px) (:222)
+  if ((rc = fill(h, seeds, iseed, 2 * nlocal, S.v[0], np, S.x[0], nlocal, np))) return rc;
+  return load_markers_finish(h, isp, np, nparticle_init, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin, 2);
+}
+
+int pic1dp_gpu_load_markers_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                        int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed,
+                                        double v_max, int32_t init_nmode, const int32_t *init_mode,
+                                        const double *init_mode_cos, const double *init_mode_sin) {
+  return load_markers_table(h, "load_markers_superkiss64", sk_bad_state, superkiss64_fill_device, isp, np, nlocal,
+                            nparticle_init, seeds, iseed, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+}
+
+int pic1dp_gpu_load_markers_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal, int64_t nparticle_init,
+                                       uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, double v_max,
+                                       int32_t init_nmode, const int32_t *init_mode, const double *init_mode_cos,
+                                       const double *init_mode_sin) {
+  return load_markers_table(h, "load_markers_mt19937_64", mt_bad_state, mt19937_64_fill_device, isp, np, nlocal,
+                            nparticle_init, seeds, iseed, v_max, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+}
+
+// ---- Maxwellian markers: multirand_gaussian_array(pv) on the device (rng_kernels.cuh) ----
+static_assert(PIC1DP_GAUSS_ROUND == PIC1DP_GAUSS_ROUND_DRAWS && PIC1DP_GAUSS_ROUND % 2 == 0, "Gaussian round size");
+
+// input_init: "case of input_iptcldist >= 1 and input_imarker = 1 not implemented yet"
+static int maxwellian_check_dist(pic1dp_gpu_t *h, const char *who) {
+  if (!h || h->p.iptcldist == 0) return PIC1DP_OK;
+  h->err = std::string(who) + ": input_imarker = 1 supports only iptcldist = 0 (src/pic1dp_input.F90:291-299)";
+  return PIC1DP_EINVAL;
+}
+
+extern "C++" {   // templates need C++ linkage
+
+// The Maxwellian loader: gaussian_array(pv, nlocal), then real_array(px, nlocal), from the stream of Gen (KissGauss,
+// SkGauss, MtGauss), which supplies for a call with nlocal > 0:
+//   bad_state()      the caller's state is NULL or out of range;
+//   begin(h)         the state on the device;
+//   round(h, a, d)   raw words [a, a + PIC1DP_GAUSS_ROUND) from the call's first draw into d;
+//   x_stream(h, cut, np, nlocal, d_x)   uniforms of draws [cut, cut + nlocal), the first np kept, and a D2H of the
+//                    state after them into its own copy;
+//   hand_back(ntot)  the caller's state after ntot draws;  regenerated: the draws generated twice.
+// The Gaussian call runs in rounds: words, accept counts, compaction into v (elements < np kept), then one read of the
+// running count.  The first round whose count reaches the attempts needed holds the cut, the draw after the last
+// needed attempt.  The caller's state and Gaussian buffer are written back only when every device step has succeeded.
+template <class Gen>
+static int load_maxwellian(pic1dp_gpu_t *h, const char *who, Gen &gen, int32_t isp, int64_t np, int64_t nlocal,
+                           int64_t nparticle_init, int32_t *gauss_filled, double *gauss_buf, int32_t init_nmode,
+                           const int32_t *init_mode, const double *init_mode_cos, const double *init_mode_sin) {
+  int rc = load_check_args(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+  if (rc) return rc;
+  if ((rc = maxwellian_check_dist(h, who))) return rc;
+  if (gen.bad_state() || !gauss_filled || !gauss_buf || nlocal < np) {
+    h->err = std::string(who) + ": bad stream argument (NULL state, position out of range or nlocal < np)";
+    return PIC1DP_EINVAL;
+  }
+  CK(cudaSetDevice(h->p.device));
+  RngScratch &R = h->rng;
+  if (nlocal == 0) {   // no draw: the state and the buffer stay as they are
+    R.gauss_draws = R.gauss_rounds = R.gauss_regenerated = 0;
+    return load_markers_finish(h, isp, 0, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1);
+  }
+  if ((rc = gen.begin(h))) return rc;
+  double *d_v = h->sp[isp].v[0];
+  R.gauss_rounds = 0;
+  int64_t lo = 0;
+  if (*gauss_filled) {   // the buffered value is element 0; no draw for it
+    if (np > 0) {
+      CK(cudaMemcpyAsync(d_v, gauss_buf, 8, cudaMemcpyHostToDevice, h->stream));
+      CK(cudaStreamSynchronize(h->stream));
+      h->h2d += 8;
+    }
+    lo = 1;
+  }
+  const int64_t need = (nlocal - lo + 1) / 2;   // accepted attempts
+  const int32_t filled = (int32_t)((nlocal - lo) & 1);   // the one-slot buffer after the call
+  GaussCtl c = {0ULL, 0LL, 0.0};   // what the device reports; need = 0 takes no draw
+  if (need > 0) {
+    const int64_t npairs = PIC1DP_GAUSS_ROUND / 2, nblk = (npairs + PIC1DP_GAUSS_TILE - 1) / PIC1DP_GAUSS_TILE;
+    if (!R.d_gauss_words) CK(cudaMalloc(&R.d_gauss_words, (size_t)PIC1DP_GAUSS_ROUND * 8));
+    if (!R.d_gauss_bcount) CK(cudaMalloc(&R.d_gauss_bcount, (size_t)nblk * sizeof(unsigned)));
+    if (!R.d_gauss_ctl) CK(cudaMalloc(&R.d_gauss_ctl, sizeof(GaussCtl)));
+    GaussCtl *ctl = (GaussCtl *)R.d_gauss_ctl;
+    const GaussCtl c0 = {0ULL, -1LL, 0.0};
+    CK(cudaMemcpyAsync(ctl, &c0, sizeof(c0), cudaMemcpyHostToDevice, h->stream));
+    h->h2d += sizeof(c0);
+    const double2 *words = (const double2 *)R.d_gauss_words;
+    for (int64_t a = 0; (int64_t)c.total < need; a += PIC1DP_GAUSS_ROUND) {
+      if ((rc = gen.round(h, a, R.d_gauss_words))) return rc;
+      const int64_t base = (int64_t)c.total;
+      k_gauss_count<<<(unsigned)nblk, PIC1DP_GAUSS_THREADS, 0, h->stream>>>(words, npairs, R.d_gauss_bcount, ctl);
+      CKL(h);
+      k_gauss_scatter<<<(unsigned)nblk, PIC1DP_GAUSS_THREADS, 0, h->stream>>>(words, npairs, R.d_gauss_bcount, base, a,
+                                                                            lo, need, np, nlocal, d_v, ctl);
+      CKL(h);
+      CK(cudaMemcpyAsync(&c, ctl, sizeof(c), cudaMemcpyDeviceToHost, h->stream));
+      CK(cudaStreamSynchronize(h->stream));
+      h->d2h += sizeof(c);
+      R.gauss_rounds++;
+    }
+  }
+  const int64_t cut = c.cut;
+  if ((rc = gen.x_stream(h, cut, np, nlocal, h->sp[isp].x[0]))) return rc;
+  if ((rc = load_markers_finish(h, isp, np, nparticle_init, 1.0, init_nmode, init_mode, init_mode_cos, init_mode_sin, 1)))
+    return rc;
+  gen.hand_back(cut + nlocal);
+  *gauss_filled = filled;
+  if (filled) *gauss_buf = c.spare;
+  R.gauss_draws = cut;
+  R.gauss_regenerated = gen.regenerated;
+  return PIC1DP_OK;
+}
+
+// n uniforms of a device stream, written by fill into a scratch buffer, copied to out (the parity calls)
+template <class Fill>
+static int uniforms_to_host(pic1dp_gpu_t *h, const char *who, int64_t n, double *out, Fill fill) {
+  CK(cudaSetDevice(h->p.device));
+  double *d = nullptr;
+  CK(cudaMalloc(&d, (size_t)n * 8));
+  int rc = fill(d);
+  cudaError_t e = cudaSuccess;
+  if (!rc) {
+    e = cudaMemcpyAsync(out, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    h->d2h += n * 8;
+  }
+  cudaFree(d);
+  if (rc) return rc;
+  if (e != cudaSuccess) { h->err = std::string(who) + ": " + cudaGetErrorString(e); return PIC1DP_ECUDA; }
+  return PIC1DP_OK;
+}
+
+}  // extern "C++"
+
+// KISS64 jumps: each round and the x stream start where they are; the state is handed back by a host jump
+struct KissGauss {
+  uint64_t *seeds;
+  int64_t regenerated = 0;
+  bool bad_state() const { return !seeds; }
+  int begin(pic1dp_gpu_t *) { return PIC1DP_OK; }
+  int round(pic1dp_gpu_t *h, int64_t a, double *d) { return kiss64_fill_device(h, seeds, a, PIC1DP_GAUSS_ROUND, d, true); }
+  int x_stream(pic1dp_gpu_t *h, int64_t cut, int64_t np, int64_t, double *d_x) {
+    return kiss64_fill_device(h, seeds, cut, np, d_x);   // the unloaded tail is not generated
+  }
+  void hand_back(int64_t ntot) {
+    Kiss64 s = {seeds[0], seeds[1], seeds[2], seeds[3]};
+    kiss64_jump_host(s, (uint64_t)ntot);
+    seeds[0] = s.x; seeds[1] = s.xs; seeds[2] = s.z; seeds[3] = s.c;
+  }
+};
+
+// SuperKISS64's table cannot be jumped back: each round starts from a copy of it (d_sk_round), from which the x stream
+// is regenerated over the rest of the cut's round
+struct SkGauss {
+  uint64_t *seeds;
+  int32_t *iseed;
+  uint64_t lcg0 = 0, xs0 = 0;
+  int64_t round_start = 0;
+  int32_t round_pos = 0;
+  bool saved = false;
+  int64_t regenerated = 0;
+  std::vector<uint64_t> table;   // the device table and carry after the call
+  bool bad_state() const { return sk_bad_state(seeds, iseed); }
+  int begin(pic1dp_gpu_t *h) {
+    lcg0 = seeds[PIC1DP_SK_N + 1];
+    xs0 = seeds[PIC1DP_SK_N + 2];
+    round_pos = *iseed;
+    int rc = kiss_tables(h);
+    if (rc) return rc;
+    if (!h->rng.d_sk_round) CK(cudaMalloc(&h->rng.d_sk_round, SK_STATE_BYTES));
+    return sk_upload(h, seeds);
+  }
+  int round(pic1dp_gpu_t *h, int64_t a, double *d) {
+    CK(cudaMemcpyAsync(h->rng.d_sk_round, h->rng.d_sk_state, SK_STATE_BYTES, cudaMemcpyDeviceToDevice, h->stream));
+    saved = true;
+    round_start = a;
+    round_pos = sk_iseed_after(*iseed, a);
+    int rc = superkiss64_table_device(h, round_pos, PIC1DP_GAUSS_ROUND, d, PIC1DP_GAUSS_ROUND, nullptr, 0, 0);
+    return rc ? rc : superkiss64_finish_device(h, lcg0, xs0, a, PIC1DP_GAUSS_ROUND, d, true);
+  }
+  int x_stream(pic1dp_gpu_t *h, int64_t cut, int64_t np, int64_t nlocal, double *d_x) {
+    if (saved)
+      CK(cudaMemcpyAsync(h->rng.d_sk_state, h->rng.d_sk_round, SK_STATE_BYTES, cudaMemcpyDeviceToDevice, h->stream));
+    regenerated = cut - round_start;
+    int rc = superkiss64_table_device(h, round_pos, regenerated + nlocal, nullptr, 0, d_x, regenerated, np);
+    if (rc || (rc = superkiss64_finish_device(h, lcg0, xs0, cut, np, d_x))) return rc;
+    table.resize(PIC1DP_SK_N + 1);
+    CK(cudaMemcpyAsync(table.data(), h->rng.d_sk_state, SK_STATE_BYTES, cudaMemcpyDeviceToHost, h->stream));
+    h->d2h += SK_STATE_BYTES;
+    return PIC1DP_OK;
+  }
+  void hand_back(int64_t ntot) {
+    std::copy(table.begin(), table.end(), seeds);
+    sk_advance_host(seeds, iseed, lcg0, xs0, ntot);
+  }
+};
+
+// MT19937-64: each round starts from the block that holds its first draw, which the round before saved; its chunk
+// windows stay in d_mt_chunks, so the round that holds the cut also starts the x stream
+struct MtGauss {
+  uint64_t *seeds;
+  int32_t *iseed;
+  uint64_t B[PIC1DP_MT_N];
+  int64_t p = 0;
+  int cur = 0, next = 1;
+  int64_t g_cur = 0, g_next = 0;   // global word of the current round's start block, and of the next one's
+  bool any_round = false;
+  int64_t last = 0, T = 0;   // the x stream's last draw and the start of its block
+  int64_t regenerated = 0;
+  // windows of d_mt_state: [0] the caller's block (global word 0), [1] and [2] round start blocks in turn, [3] the final
+  // block
+  static uint64_t *slot(pic1dp_gpu_t *h, int k) { return h->rng.d_mt_state + k * PIC1DP_MT_N; }
+  bool bad_state() const { return mt_bad_state(seeds, iseed); }
+  int begin(pic1dp_gpu_t *h) { return mt_upload(h, seeds, *iseed, B, &p); }
+  int round(pic1dp_gpu_t *h, int64_t a, double *d) {
+    if (a > 0) {
+      cur = next;
+      next = cur == 1 ? 2 : 1;
+      g_cur = g_next;
+    }
+    any_round = true;
+    g_next = mt_block_of(p + a + PIC1DP_GAUSS_ROUND);
+    return mt_stream_device(h, slot(h, cur), p + a - g_cur, d, PIC1DP_GAUSS_ROUND, nullptr, 0, 0, g_next - g_cur,
+                            slot(h, next), true);
+  }
+  // the x stream starts from the latest chunk window of the cut's round at or before both its first draw and the
+  // block of its last draw
+  int x_stream(pic1dp_gpu_t *h, int64_t cut, int64_t np, int64_t nlocal, double *d_x) {
+    const int64_t x0 = p + cut;
+    last = x0 + nlocal - 1;
+    T = mt_block_of(last);
+    const uint64_t *src = slot(h, 0);
+    int64_t base = 0;
+    if (any_round) {
+      const int64_t cc = (std::min(x0, T) - g_cur) >> PIC1DP_MT_LOG2_CHUNK;
+      src = h->rng.d_mt_chunks + cc * PIC1DP_MT_N;
+      base = g_cur + (cc << PIC1DP_MT_LOG2_CHUNK);
+    }
+    int rc = mt_stream_device(h, src, x0 - base, d_x, np, nullptr, 0, 0, T - base, slot(h, 3), false);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(B, slot(h, 3), sizeof(B), cudaMemcpyDeviceToHost, h->stream));
+    h->d2h += sizeof(B);
+    return PIC1DP_OK;
+  }
+  void hand_back(int64_t) {
+    memcpy(seeds, B, sizeof(B));
+    *iseed = (int32_t)(last - T + 1);
+  }
+};
+
+int pic1dp_gpu_load_markers_maxwellian_kiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                              int64_t nparticle_init, uint64_t seeds[4], int32_t *gauss_filled,
+                                              double *gauss_buf, int32_t init_nmode, const int32_t *init_mode,
+                                              const double *init_mode_cos, const double *init_mode_sin) {
+  KissGauss gen{seeds};
+  return load_maxwellian(h, "load_markers_maxwellian_kiss64", gen, isp, np, nlocal, nparticle_init, gauss_filled,
+                         gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+}
+
+int pic1dp_gpu_load_markers_maxwellian_superkiss64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                                   int64_t nparticle_init, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED],
+                                                   int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
+                                                   int32_t init_nmode, const int32_t *init_mode,
+                                                   const double *init_mode_cos, const double *init_mode_sin) {
+  SkGauss gen{seeds, iseed};
+  return load_maxwellian(h, "load_markers_maxwellian_superkiss64", gen, isp, np, nlocal, nparticle_init, gauss_filled,
+                         gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+}
+
+int pic1dp_gpu_load_markers_maxwellian_mt19937_64(pic1dp_gpu_t *h, int32_t isp, int64_t np, int64_t nlocal,
+                                                  int64_t nparticle_init, uint64_t seeds[PIC1DP_MT19937_64_NSEED],
+                                                  int32_t *iseed, int32_t *gauss_filled, double *gauss_buf,
+                                                  int32_t init_nmode, const int32_t *init_mode,
+                                                  const double *init_mode_cos, const double *init_mode_sin) {
+  MtGauss gen{seeds, iseed};
+  return load_maxwellian(h, "load_markers_maxwellian_mt19937_64", gen, isp, np, nlocal, nparticle_init, gauss_filled,
+                         gauss_buf, init_nmode, init_mode, init_mode_cos, init_mode_sin);
+}
+
 int pic1dp_gpu_last_gaussian_load(pic1dp_gpu_t *h, int64_t *draws, int64_t *rounds, int64_t *regenerated) {
   if (!h || !draws || !rounds || !regenerated) return PIC1DP_EINVAL;
-  *draws = h->gauss_draws;
-  *rounds = h->gauss_rounds;
-  *regenerated = h->gauss_regenerated;
+  *draws = h->rng.gauss_draws;
+  *rounds = h->rng.gauss_rounds;
+  *regenerated = h->rng.gauss_regenerated;
   return PIC1DP_OK;
+}
+
+// ---- parity checks: n uniforms of a device stream copied to the host ----
+int pic1dp_gpu_kiss64_uniforms(pic1dp_gpu_t *h, const uint64_t seeds[4], int64_t offset, int64_t n, double *out) {
+  if (!h || !seeds || offset < 0 || n < 0 || !out) { if (h) h->err = "kiss64_uniforms: bad argument"; return PIC1DP_EINVAL; }
+  if (n == 0) return PIC1DP_OK;
+  return uniforms_to_host(h, "kiss64_uniforms", n, out, [&](double *d) { return kiss64_fill_device(h, seeds, offset, n, d); });
+}
+
+// a table generator's stream: the caller's state is staged and written back only when every device step has succeeded
+static int table_uniforms(pic1dp_gpu_t *h, const char *who, TableBadState bad_state, TableFill fill, size_t nseed,
+                          uint64_t *seeds, int32_t *iseed, int64_t n, double *out) {
+  if (!h || bad_state(seeds, iseed) || n < 0 || (n > 0 && !out)) {
+    if (h) h->err = std::string(who) + ": bad argument";
+    return PIC1DP_EINVAL;
+  }
+  if (n == 0) return PIC1DP_OK;
+  std::vector<uint64_t> s(seeds, seeds + nseed);
+  int32_t pos = *iseed;
+  int rc = uniforms_to_host(h, who, n, out, [&](double *d) { return fill(h, s.data(), &pos, n, d, n, nullptr, 0, 0); });
+  if (rc) return rc;
+  std::copy(s.begin(), s.end(), seeds);
+  *iseed = pos;
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_superkiss64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_SUPERKISS64_NSEED], int32_t *iseed, int64_t n,
+                                    double *out) {
+  return table_uniforms(h, "superkiss64_uniforms", sk_bad_state, superkiss64_fill_device, PIC1DP_SUPERKISS64_NSEED,
+                        seeds, iseed, n, out);
+}
+
+int pic1dp_gpu_mt19937_64_uniforms(pic1dp_gpu_t *h, uint64_t seeds[PIC1DP_MT19937_64_NSEED], int32_t *iseed, int64_t n,
+                                   double *out) {
+  return table_uniforms(h, "mt19937_64_uniforms", mt_bad_state, mt19937_64_fill_device, PIC1DP_MT19937_64_NSEED, seeds,
+                        iseed, n, out);
 }
 
 void pic1dp_host_counter_uniforms(uint64_t seed, int32_t stream, int64_t first_index, int64_t n, double *u_v, double *u_x) {
@@ -1550,10 +1563,8 @@ int pic1dp_gpu_load_markers_maxwellian(pic1dp_gpu_t *h, int32_t isp, int64_t np,
                                        const double *gauss_v, const double *rand_x, int32_t init_nmode,
                                        const int32_t *init_mode, const double *init_mode_cos,
                                        const double *init_mode_sin) {
-  if (h && h->p.iptcldist != 0) {  // input_init: "case of input_iptcldist >= 1 and input_imarker = 1 not implemented yet"
-    h->err = "load_markers_maxwellian: input_imarker = 1 supports only iptcldist = 0 (src/pic1dp_input.F90:291-299)";
-    return PIC1DP_EINVAL;
-  }
+  int rc = maxwellian_check_dist(h, "load_markers_maxwellian");
+  if (rc) return rc;
   return load_markers_impl(h, isp, np, nparticle_init, gauss_v, rand_x, 1.0, init_nmode, init_mode, init_mode_cos,
                            init_mode_sin, 1);
 }

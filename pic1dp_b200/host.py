@@ -48,18 +48,20 @@ def _dp(a: Optional[np.ndarray]):
     return a.ctypes.data_as(C.POINTER(C.c_double))
 
 
-def _u64p(seeds: np.ndarray):
-    """The SuperKISS64 state multirand_seeds(0:20634), passed for in-place update."""
-    assert seeds.dtype == np.uint64 and seeds.size == _capi.SUPERKISS64_NSEED and seeds.flags["C_CONTIGUOUS"], \
-        "SuperKISS64 state: C-contiguous uint64 array of 20635 words"
+_KISS, _SK, _MT = (4, "KISS64"), (_capi.SUPERKISS64_NSEED, "SuperKISS64"), (_capi.MT19937_64_NSEED, "MT19937-64")
+
+
+def _state_ptr(seeds: np.ndarray, nwords: int, name: str):
+    """A generator state multirand_seeds(0:nwords-1), passed for in-place update (_state_ptr(seeds, *_SK))."""
+    assert seeds.dtype == np.uint64 and seeds.size == nwords and seeds.flags["C_CONTIGUOUS"], \
+        f"{name} state: C-contiguous uint64 array of {nwords} words"
     return seeds.ctypes.data_as(C.POINTER(C.c_uint64))
 
 
-def _mt_u64p(seeds: np.ndarray):
-    """The MT19937-64 state multirand_seeds(0:311), passed for in-place update."""
-    assert seeds.dtype == np.uint64 and seeds.size == _capi.MT19937_64_NSEED and seeds.flags["C_CONTIGUOUS"], \
-        "MT19937-64 state: C-contiguous uint64 array of 312 words"
-    return seeds.ctypes.data_as(C.POINTER(C.c_uint64))
+def _modes(init_mode, init_cos, init_sin):
+    """The initial perturbation's mode numbers and cos / sin amplitudes as ctypes arrays of init_nmode elements."""
+    nm = len(init_mode)
+    return (C.c_int32 * nm)(*init_mode), (C.c_double * nm)(*init_cos), (C.c_double * nm)(*init_sin)
 
 
 def _ptr(addr: int):
@@ -135,42 +137,34 @@ class Pic1dGpu:
     def load_markers(self, isp: int, rand_v, rand_x, nparticle_init: int, v_max: float = 8.0, init_mode=(1,),
                      init_cos=(0.0,), init_sin=(1e-5,)):
         """Device-side particle_load from the two uniform streams (arrays or raw host addresses)."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         if isinstance(rand_v, np.ndarray):
             n, pv, px = rand_v.size, _dp(rand_v), _dp(rand_x)
         else:
             n, pv, px = rand_v[1], _ptr(rand_v[0]), _ptr(rand_x[0])
-        self._ck(self.L.pic1dp_gpu_load_markers(self._h, isp, n, int(nparticle_init), pv, px, float(v_max), nm, im, ic, isn),
-                 "load_markers")
+        self._ck(self.L.pic1dp_gpu_load_markers(self._h, isp, n, int(nparticle_init), pv, px, float(v_max), len(im), im,
+                                                ic, isn), "load_markers")
 
     def load_markers_kiss64(self, isp: int, n: int, seeds, offset_v: int, offset_x: int, nparticle_init: int,
                             v_max: float = 8.0, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)):
         """Device-side particle_load with the device KISS64 stream (multirand_al_int = 1), bit-exact to multirand.
         seeds: multirand_seeds(0:3) after multirand_init; offsets: outputs consumed before pv / px of this rank."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         sd = (C.c_uint64 * 4)(*[int(v) & 0xFFFFFFFFFFFFFFFF for v in seeds])
         self._ck(self.L.pic1dp_gpu_load_markers_kiss64(self._h, isp, int(n), int(nparticle_init), sd, int(offset_v),
-                                                       int(offset_x), float(v_max), nm, im, ic, isn), "load_markers_kiss64")
+                                                       int(offset_x), float(v_max), len(im), im, ic, isn),
+                 "load_markers_kiss64")
 
     def load_markers_superkiss64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, nparticle_init: int,
                                  v_max: float = 8.0, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)) -> int:
         """Device-side particle_load with the device SuperKISS64 stream (multirand_al_int = 3), bit-exact to multirand.
         seeds: multirand_seeds(0:20634) as a uint64 array, advanced IN PLACE past the 2 * nlocal draws; iseed: the
         table position before them.  Returns the table position after them."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         pos = C.c_int32(int(iseed))
-        self._ck(self.L.pic1dp_gpu_load_markers_superkiss64(self._h, isp, int(n), int(nlocal), int(nparticle_init),
-                                                            _u64p(seeds), C.byref(pos), float(v_max), nm, im, ic, isn),
-                 "load_markers_superkiss64")
+        self._ck(self.L.pic1dp_gpu_load_markers_superkiss64(
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _state_ptr(seeds, *_SK), C.byref(pos),
+            float(v_max), len(im), im, ic, isn), "load_markers_superkiss64")
         return pos.value
 
     def load_markers_maxwellian_kiss64(self, isp: int, n: int, nlocal: int, seeds, gauss_filled: int, gauss_buf: float,
@@ -179,16 +173,11 @@ class Pic1dGpu:
         real_array(px, nlocal)) generated on the device by KISS64.  seeds: multirand_seeds(0:3) as a C-contiguous uint64
         array, advanced IN PLACE past every draw; (gauss_filled, gauss_buf): the Gaussian one-slot buffer before the
         call.  Returns the buffer after it."""
-        assert seeds.dtype == np.uint64 and seeds.size == 4 and seeds.flags["C_CONTIGUOUS"], \
-            "KISS64 state: C-contiguous uint64 array of 4 words"
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         filled, buf = C.c_int32(int(gauss_filled)), C.c_double(float(gauss_buf))
         self._ck(self.L.pic1dp_gpu_load_markers_maxwellian_kiss64(
-            self._h, isp, int(n), int(nlocal), int(nparticle_init), seeds.ctypes.data_as(C.POINTER(C.c_uint64)),
-            C.byref(filled), C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_kiss64")
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _state_ptr(seeds, *_KISS),
+            C.byref(filled), C.byref(buf), len(im), im, ic, isn), "load_markers_maxwellian_kiss64")
         return filled.value, buf.value
 
     def load_markers_maxwellian_superkiss64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, gauss_filled: int,
@@ -196,14 +185,11 @@ class Pic1dGpu:
                                             init_sin=(1e-5,)):
         """The same with SuperKISS64: seeds = multirand_seeds(0:20634) (advanced in place), iseed = the table position.
         Returns (iseed, gauss_filled, gauss_buf) after the call."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         pos, filled, buf = C.c_int32(int(iseed)), C.c_int32(int(gauss_filled)), C.c_double(float(gauss_buf))
         self._ck(self.L.pic1dp_gpu_load_markers_maxwellian_superkiss64(
-            self._h, isp, int(n), int(nlocal), int(nparticle_init), _u64p(seeds), C.byref(pos), C.byref(filled),
-            C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_superkiss64")
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _state_ptr(seeds, *_SK), C.byref(pos),
+            C.byref(filled), C.byref(buf), len(im), im, ic, isn), "load_markers_maxwellian_superkiss64")
         return pos.value, filled.value, buf.value
 
     def load_markers_mt19937_64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, nparticle_init: int,
@@ -211,14 +197,11 @@ class Pic1dGpu:
         """Device-side particle_load with the device MT19937-64 stream (multirand_al_int = 2), bit-exact to multirand.
         seeds: multirand_seeds(0:311) as a C-contiguous uint64 array, advanced IN PLACE past the 2 * nlocal draws;
         iseed: the block position before them.  Returns the block position after them."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         pos = C.c_int32(int(iseed))
-        self._ck(self.L.pic1dp_gpu_load_markers_mt19937_64(self._h, isp, int(n), int(nlocal), int(nparticle_init),
-                                                           _mt_u64p(seeds), C.byref(pos), float(v_max), nm, im, ic, isn),
-                 "load_markers_mt19937_64")
+        self._ck(self.L.pic1dp_gpu_load_markers_mt19937_64(
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _state_ptr(seeds, *_MT), C.byref(pos),
+            float(v_max), len(im), im, ic, isn), "load_markers_mt19937_64")
         return pos.value
 
     def load_markers_maxwellian_mt19937_64(self, isp: int, n: int, nlocal: int, seeds, iseed: int, gauss_filled: int,
@@ -226,21 +209,18 @@ class Pic1dGpu:
                                            init_sin=(1e-5,)):
         """The Maxwellian loader with MT19937-64: seeds = multirand_seeds(0:311) (advanced in place), iseed = the block
         position.  Returns (iseed, gauss_filled, gauss_buf) after the call."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         pos, filled, buf = C.c_int32(int(iseed)), C.c_int32(int(gauss_filled)), C.c_double(float(gauss_buf))
         self._ck(self.L.pic1dp_gpu_load_markers_maxwellian_mt19937_64(
-            self._h, isp, int(n), int(nlocal), int(nparticle_init), _mt_u64p(seeds), C.byref(pos), C.byref(filled),
-            C.byref(buf), nm, im, ic, isn), "load_markers_maxwellian_mt19937_64")
+            self._h, isp, int(n), int(nlocal), int(nparticle_init), _state_ptr(seeds, *_MT), C.byref(pos),
+            C.byref(filled), C.byref(buf), len(im), im, ic, isn), "load_markers_maxwellian_mt19937_64")
         return pos.value, filled.value, buf.value
 
     def mt19937_64_uniforms(self, seeds, iseed: int, n: int):
         """(n uniforms of the device MT19937-64 stream, block position after them); seeds advanced in place."""
         out = np.empty(n)
         pos = C.c_int32(int(iseed))
-        self._ck(self.L.pic1dp_gpu_mt19937_64_uniforms(self._h, _mt_u64p(seeds), C.byref(pos), int(n), _dp(out)),
+        self._ck(self.L.pic1dp_gpu_mt19937_64_uniforms(self._h, _state_ptr(seeds, *_MT), C.byref(pos), int(n), _dp(out)),
                  "mt19937_64_uniforms")
         return out, pos.value
 
@@ -254,19 +234,16 @@ class Pic1dGpu:
         """(n uniforms of the device SuperKISS64 stream, table position after them); seeds advanced in place."""
         out = np.empty(n)
         pos = C.c_int32(int(iseed))
-        self._ck(self.L.pic1dp_gpu_superkiss64_uniforms(self._h, _u64p(seeds), C.byref(pos), int(n), _dp(out)),
-                 "superkiss64_uniforms")
+        self._ck(self.L.pic1dp_gpu_superkiss64_uniforms(self._h, _state_ptr(seeds, *_SK), C.byref(pos), int(n),
+                                                        _dp(out)), "superkiss64_uniforms")
         return out, pos.value
 
     def load_markers_counter(self, isp: int, n: int, seed: int, first_index: int, nparticle_init: int,
                              v_max: float = 8.0, init_mode=(1,), init_cos=(0.0,), init_sin=(1e-5,)):
         """Device-side particle_load with the counter-based generator (synthetic markers, no reference stream)."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         self._ck(self.L.pic1dp_gpu_load_markers_counter(self._h, isp, int(n), int(nparticle_init), int(seed),
-                                                        int(first_index), float(v_max), nm, im, ic, isn),
+                                                        int(first_index), float(v_max), len(im), im, ic, isn),
                  "load_markers_counter")
 
     def kiss64_uniforms(self, seeds, offset: int, n: int) -> np.ndarray:
@@ -288,12 +265,10 @@ class Pic1dGpu:
     def load_markers_maxwellian(self, isp: int, gauss_v, rand_x, nparticle_init: int, init_mode=(1,), init_cos=(0.0,),
                                 init_sin=(1e-5,)):
         """Device-side particle_load for input_imarker = 1 (Gaussian v stream, iptcldist = 0)."""
-        nm = len(init_mode)
-        im = (C.c_int32 * nm)(*init_mode)
-        ic = (C.c_double * nm)(*init_cos)
-        isn = (C.c_double * nm)(*init_sin)
+        im, ic, isn = _modes(init_mode, init_cos, init_sin)
         self._ck(self.L.pic1dp_gpu_load_markers_maxwellian(self._h, isp, gauss_v.size, int(nparticle_init), _dp(gauss_v),
-                                                           _dp(rand_x), nm, im, ic, isn), "load_markers_maxwellian")
+                                                           _dp(rand_x), len(im), im, ic, isn),
+                 "load_markers_maxwellian")
 
     def get_markers(self, isp: int, want=("x", "v", "p", "w")):
         n = C.c_int64()
@@ -688,7 +663,7 @@ def host_superkiss64_fill(seeds, iseed: int, n: int):
     20635 words) advanced in place."""
     out = np.empty(n)
     pos = C.c_int32(int(iseed))
-    rc = _capi.load().pic1dp_host_superkiss64_fill(_u64p(seeds), C.byref(pos), int(n), _dp(out))
+    rc = _capi.load().pic1dp_host_superkiss64_fill(_state_ptr(seeds, *_SK), C.byref(pos), int(n), _dp(out))
     if rc:
         raise Pic1dpError(rc, "pic1dp_host_superkiss64_fill", "bad argument")
     return out, pos.value
@@ -696,7 +671,7 @@ def host_superkiss64_fill(seeds, iseed: int, n: int):
 
 def host_superkiss64_refill(seeds, nchunks: int):
     """One table refill of seeds (in place) by the device's chunked carry-map scan, run on the host."""
-    rc = _capi.load().pic1dp_host_superkiss64_refill(_u64p(seeds), int(nchunks))
+    rc = _capi.load().pic1dp_host_superkiss64_refill(_state_ptr(seeds, *_SK), int(nchunks))
     if rc:
         raise Pic1dpError(rc, "pic1dp_host_superkiss64_refill", "bad argument")
 
@@ -706,7 +681,7 @@ def host_mt19937_64_jump(seeds, iseed: int, n: int) -> int:
     """multirand_seeds(0:311) (uint64 array, in place) and the block position advanced by n draws with the device's
     window-XOR jump run on the host.  Returns the block position after them."""
     pos = C.c_int32(int(iseed))
-    rc = _capi.load().pic1dp_host_mt19937_64_jump(_mt_u64p(seeds), C.byref(pos), int(n))
+    rc = _capi.load().pic1dp_host_mt19937_64_jump(_state_ptr(seeds, *_MT), C.byref(pos), int(n))
     if rc:
         raise Pic1dpError(rc, "pic1dp_host_mt19937_64_jump", "bad argument")
     return pos.value

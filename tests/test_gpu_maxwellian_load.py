@@ -4,7 +4,6 @@ KISS64 (multirand_al_int = 1) and SuperKISS64 (al_int = 3).  Checked against the
 returned generator state exactly, the Gaussian values to a few ulp (the device log is not glibc's), the one-slot
 Gaussian buffer across calls and species, refusals, and the C++ host driver with and without the device streams."""
 import ctypes as C
-import subprocess
 
 import numpy as np
 import pytest
@@ -12,53 +11,11 @@ import pytest
 import pic1dp_b200 as P
 from pic1dp_b200 import _capi
 from helpers import make_params
-from multirand_state import NSEED, get_state
+from multirand_state import get_spare, get_state, run_host, ulps
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 N_TABLE = 20632
-
-# struct orc_multirand (oracle/multirand_oracle.c): uint64_t seeds[20635]; int iseed; int al_int; int gauss_filled;
-# double gauss_buf -- the one-slot buffer of orc_multirand_gaussian_array
-_AL_OFFSET = NSEED * 8 + 4
-_FILLED_OFFSET = NSEED * 8 + 8
-_BUF_OFFSET = NSEED * 8 + 16
-_spare_layout_checked = False
-
-
-def _check_spare_layout():
-    global _spare_layout_checked
-    if _spare_layout_checked:
-        return
-    for al in (1, 3):
-        g = O.MultiRand()
-        g.seed_default(al)
-        addr = g.g.value
-        assert C.c_int.from_address(addr + _AL_OFFSET).value == al, "orc_multirand.al_int moved"
-        assert C.c_int.from_address(addr + _FILLED_OFFSET).value == 0
-        ref = O.MultiRand()
-        ref.seed_default(al)
-        pair = ref.gaussian_array(2)
-        g.gaussian_array(1)   # odd length: the second value of the pair stays buffered
-        assert C.c_int.from_address(addr + _FILLED_OFFSET).value == 1, "orc_multirand.gauss_filled moved"
-        assert C.c_double.from_address(addr + _BUF_OFFSET).value == pair[1], "orc_multirand.gauss_buf moved"
-    _spare_layout_checked = True
-
-
-def get_spare(g):
-    """(gauss_filled, gauss_buf) of the oracle generator."""
-    _check_spare_layout()
-    addr = g.g.value
-    return C.c_int.from_address(addr + _FILLED_OFFSET).value, C.c_double.from_address(addr + _BUF_OFFSET).value
-
-
-def ulps(a, b):
-    """Elementwise distance in units in the last place (as ordered integers)."""
-    def key(x):
-        i = np.asarray(x, dtype=np.float64).view(np.int64)
-        return np.where(i < 0, np.int64(-0x8000000000000000) - i, i)
-    return np.abs(key(a) - key(b))
-
 
 class Stream:
     """The device loader of one generator with its state threaded through, in the oracle's representation."""
@@ -183,7 +140,7 @@ def test_refusals_leave_the_state_alone(al):
         else:
             rc = L.pic1dp_gpu_load_markers_maxwellian_kiss64(g._h, 0, np_, nlocal, 1000, sp, C.byref(filled),
                                                              C.byref(buf), 1, im, ic, isn)
-            assert np.array_equal(seeds, ref) and pos.value == iseed and filled.value == filled0 and buf.value == buf0
+        assert np.array_equal(seeds, ref) and pos.value == iseed and filled.value == filled0 and buf.value == buf0
         return rc
 
     _, gp3 = make_params(capacity=1000, iptcldist=3)
@@ -199,16 +156,6 @@ def test_refusals_leave_the_state_alone(al):
         assert call(g, 1001, 2000) == _capi.ECAPACITY
 
 
-def _run_host(exe, tmp_path, tag, args):
-    mk = tmp_path / f"markers_{tag}.bin"
-    r = subprocess.run([exe, *args, f"out={tmp_path / f'energy_{tag}.txt'}", f"markers_out={mk}"],
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout + r.stderr
-    raw = np.fromfile(mk, dtype=np.float64)
-    n = int(np.frombuffer(raw[:1].tobytes(), dtype=np.int64)[0])
-    return r.stdout, n, dict(zip(("x", "v", "p", "w"), raw[1:].reshape(4, n)))
-
-
 @pytest.mark.parametrize("al", [1, 3])
 def test_cpp_host_driver_maxwellian_device_streams(tmp_path, al):
     """host/pic1dp_host, imarker=1, seed_type 1, an unloaded tail: the markers right after particle_load with the device
@@ -220,15 +167,15 @@ def test_cpp_host_driver_maxwellian_device_streams(tmp_path, al):
             f"al_int={al}", "v0=0.5", "temperature=1.2"]
     load = {}
     for dev in (1, 0):
-        _, n, load[dev] = _run_host(exe, tmp_path, f"load{dev}", base + ["ntime_max=0", f"device_rng={dev}"])
+        _, n, load[dev] = run_host(exe, tmp_path, f"load{dev}", base + ["ntime_max=0", f"device_rng={dev}"])
         assert n == 200_001
     for k in ("x", "p", "w"):
         assert np.array_equal(load[1][k], load[0][k]), k
     assert np.max(np.abs(load[1]["v"] - load[0]["v"])) <= 1e-15 * np.max(np.abs(load[0]["v"]))
     run = {}
     for dev in (1, 0):
-        out, n, run[dev] = _run_host(exe, tmp_path, f"run{dev}", base + ["ntime_max=4", "nsplit=1", "opt_t0=0.0",
-                                                                        "opt_dt=0.1", f"device_rng={dev}"])
+        out, n, run[dev] = run_host(exe, tmp_path, f"run{dev}", base + ["ntime_max=4", "nsplit=1", "opt_t0=0.0",
+                                                                       "opt_dt=0.1", f"device_rng={dev}"])
         assert "marker optimisation" in out
         run[dev]["n"] = n
     assert run[1]["n"] == run[0]["n"] > 200_001
@@ -245,9 +192,9 @@ def test_cpp_host_driver_kiss64_uniform_device_stream(tmp_path):
     exe = build.build_host()
     outs = {}
     for dev in (1, 0):
-        out, n, m = _run_host(exe, tmp_path, f"k{dev}", ["nparticle_max=300000", "nparticle_init=200000", "nx=192",
-                                                         "ntime_max=4", "seed_type=1", "al_int=1", "nremove=1",
-                                                         "nsplit=1", "opt_t0=0.0", "opt_dt=0.1", f"device_rng={dev}"])
+        out, n, m = run_host(exe, tmp_path, f"k{dev}", ["nparticle_max=300000", "nparticle_init=200000", "nx=192",
+                                                        "ntime_max=4", "seed_type=1", "al_int=1", "nremove=1",
+                                                        "nsplit=1", "opt_t0=0.0", "opt_dt=0.1", f"device_rng={dev}"])
         assert "marker optimisation" in out
         outs[dev] = (n, m)
     assert outs[1][0] == outs[0][0] > 100_000

@@ -5,7 +5,6 @@ streams."""
 import ctypes as C
 import json
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -13,39 +12,11 @@ import pytest
 import pic1dp_b200 as P
 from pic1dp_b200 import _capi
 from helpers import make_params
-from multirand_state import NSEED, get_state
+from multirand_state import get_spare, get_state, run_host, to_real, ulps
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 NN = 312
-
-
-# struct orc_multirand (oracle/multirand_oracle.c): uint64_t seeds[20635]; int iseed; int al_int; int gauss_filled;
-# double gauss_buf -- the one-slot buffer of orc_multirand_gaussian_array
-_FILLED_OFFSET = NSEED * 8 + 8
-_BUF_OFFSET = NSEED * 8 + 16
-_spare_layout_checked = False
-
-
-def get_spare(g):
-    """(gauss_filled, gauss_buf) of the oracle generator; the layout is checked against gaussian_array first."""
-    global _spare_layout_checked
-    if not _spare_layout_checked:
-        a, b = O.MultiRand(), O.MultiRand()
-        a.seed_default(2)
-        b.seed_default(2)
-        assert C.c_int.from_address(a.g.value + _FILLED_OFFSET).value == 0
-        pair = b.gaussian_array(2)
-        a.gaussian_array(1)   # odd length: the second value of the pair stays buffered
-        assert C.c_int.from_address(a.g.value + _FILLED_OFFSET).value == 1, "orc_multirand.gauss_filled moved"
-        assert C.c_double.from_address(a.g.value + _BUF_OFFSET).value == pair[1], "orc_multirand.gauss_buf moved"
-        _spare_layout_checked = True
-    addr = g.g.value
-    return C.c_int.from_address(addr + _FILLED_OFFSET).value, C.c_double.from_address(addr + _BUF_OFFSET).value
-
-
-def _to_real(i):
-    return float(np.int64(i)) / 18446744073709551615.0 + 0.5
 
 
 def _mt_state(r):
@@ -56,13 +27,6 @@ def _mt_state(r):
 def _assert_state(r, seeds, iseed, what):
     want, want_iseed = _mt_state(r)
     assert iseed == want_iseed and np.array_equal(seeds, want), what
-
-
-def ulps(a, b):
-    def key(x):
-        i = np.asarray(x, dtype=np.float64).view(np.int64)
-        return np.where(i < 0, np.int64(-0x8000000000000000) - i, i)
-    return np.abs(key(a) - key(b))
 
 
 def test_device_mt19937_64_known_answer_head_and_tail():
@@ -76,8 +40,8 @@ def test_device_mt19937_64_known_answer_head_and_tail():
     _, gp = make_params(capacity=16)
     with P.Pic1dGpu(gp) as g:
         u, pos = g.mt19937_64_uniforms(seeds, iseed, NN + 5)
-    assert [float(t) for t in u[:10]] == [_to_real(i) for i in gold["mt19937_64_head"]]
-    assert [float(t) for t in u[NN - 5:NN + 5]] == [_to_real(i) for i in gold["mt19937_64_tail"]]
+    assert [float(t) for t in u[:10]] == [to_real(i) for i in gold["mt19937_64_head"]]
+    assert [float(t) for t in u[NN - 5:NN + 5]] == [to_real(i) for i in gold["mt19937_64_tail"]]
     g0.skip(NN + 5)
     _assert_state(g0, seeds, pos, "after the KAT")
 
@@ -217,16 +181,6 @@ def test_refusals_leave_the_state_alone():
         assert np.array_equal(seeds, ref) and pos.value == NN + 1
 
 
-def _run_host(exe, tmp_path, tag, args):
-    mk = tmp_path / f"markers_{tag}.bin"
-    r = subprocess.run([exe, *args, f"out={tmp_path / f'energy_{tag}.txt'}", f"markers_out={mk}"],
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout + r.stderr
-    raw = np.fromfile(mk, dtype=np.float64)
-    n = int(np.frombuffer(raw[:1].tobytes(), dtype=np.int64)[0])
-    return r.stdout, n, dict(zip(("x", "v", "p", "w"), raw[1:].reshape(4, n)))
-
-
 def test_cpp_host_driver_uniform_device_stream(tmp_path):
     """host/pic1dp_host, al_int=2, imarker=2: the device stream (device_rng=1) against the host stream (device_rng=0),
     bit for bit, right after the load and after remove / split events that draw from the generator afterwards."""
@@ -236,7 +190,7 @@ def test_cpp_host_driver_uniform_device_stream(tmp_path):
     for extra in (["ntime_max=0"], ["ntime_max=4", "nremove=1", "nsplit=1", "opt_t0=0.0", "opt_dt=0.1"]):
         outs = {}
         for dev in (1, 0):
-            _, n, m = _run_host(exe, tmp_path, f"u{dev}", base + extra + [f"device_rng={dev}"])
+            _, n, m = run_host(exe, tmp_path, f"u{dev}", base + extra + [f"device_rng={dev}"])
             outs[dev] = (n, m)
         assert outs[1][0] == outs[0][0] > 100_000
         for k in ("x", "v", "p", "w"):
@@ -252,15 +206,15 @@ def test_cpp_host_driver_maxwellian_device_streams(tmp_path):
             "al_int=2", "v0=0.5", "temperature=1.2"]
     load = {}
     for dev in (1, 0):
-        _, n, load[dev] = _run_host(exe, tmp_path, f"load{dev}", base + ["ntime_max=0", f"device_rng={dev}"])
+        _, n, load[dev] = run_host(exe, tmp_path, f"load{dev}", base + ["ntime_max=0", f"device_rng={dev}"])
         assert n == 200_001
     for k in ("x", "p", "w"):
         assert np.array_equal(load[1][k], load[0][k]), k
     assert np.max(np.abs(load[1]["v"] - load[0]["v"])) <= 1e-15 * np.max(np.abs(load[0]["v"]))
     run = {}
     for dev in (1, 0):
-        out, n, run[dev] = _run_host(exe, tmp_path, f"run{dev}", base + ["ntime_max=4", "nsplit=1", "opt_t0=0.0",
-                                                                        "opt_dt=0.1", f"device_rng={dev}"])
+        out, n, run[dev] = run_host(exe, tmp_path, f"run{dev}", base + ["ntime_max=4", "nsplit=1", "opt_t0=0.0",
+                                                                       "opt_dt=0.1", f"device_rng={dev}"])
         assert "marker optimisation" in out
         run[dev]["n"] = n
     assert run[1]["n"] == run[0]["n"] > 200_001

@@ -11,15 +11,11 @@ import pytest
 import pic1dp_b200 as P
 from pic1dp_b200 import _capi
 from helpers import make_params
-from multirand_state import get_state
+from multirand_state import get_state, to_real
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 N = 20632
-
-
-def _to_real(i):
-    return float(np.int64(i)) / 18446744073709551615.0 + 0.5
 
 
 def test_device_superkiss64_known_answer_head_and_tail():
@@ -30,8 +26,8 @@ def test_device_superkiss64_known_answer_head_and_tail():
     _, gp = make_params(capacity=16)
     with P.Pic1dGpu(gp) as g:
         u, pos = g.superkiss64_uniforms(seeds, iseed, N + 5)
-    assert [float(t) for t in u[:10]] == [_to_real(i) for i in gold["superkiss64_head"]]
-    assert [float(t) for t in u[N - 5:N + 5]] == [_to_real(i) for i in gold["superkiss64_tail"]]
+    assert [float(t) for t in u[:10]] == [to_real(i) for i in gold["superkiss64_head"]]
+    assert [float(t) for t in u[N - 5:N + 5]] == [to_real(i) for i in gold["superkiss64_tail"]]
     g0.skip(N + 5)
     want_seeds, want_iseed = get_state(g0)
     assert pos == want_iseed and np.array_equal(seeds, want_seeds)

@@ -99,7 +99,7 @@ def main():
         u = np.zeros(ndraw)        # pre-faulted
         pos_h = C.c_int32(iseed0)
         t0 = time.perf_counter()
-        rc = _capi.load().pic1dp_host_superkiss64_fill(H._u64p(s), C.byref(pos_h), ndraw, H._dp(u))
+        rc = _capi.load().pic1dp_host_superkiss64_fill(H._state_ptr(s, *H._SK), C.byref(pos_h), ndraw, H._dp(u))
         t1 = time.perf_counter()
         assert rc == 0
         p2 = pos_h.value
