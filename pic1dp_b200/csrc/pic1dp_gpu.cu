@@ -166,8 +166,9 @@ struct pic1dp_gpu {
   int tma_smem[2] = {0, 0};  // dynamic shared memory of the TMA kernels, irk = 1, 2
   bool use_cpa[2] = {false, false};  // cp.async-staged kernel per substep
   int cpa_smem[2] = {0, 0};
-  // step() runs the recomputed-midpoint kernel pair (k_push with RC = true): substep 1 stores only w', substep 2 rebuilds
-  // x' and v' from the start-of-step state and E_start.  40 + 64 instead of 56 + 80 bytes per marker and step.
+  // step() runs the recomputed-midpoint kernel pair (k_push with RC = true): substep 1 stores only d' = p - w' (nonlinear
+  // delta-f; nothing otherwise), substep 2 reads it in place of w' and p and rebuilds x' and v' from the start-of-step
+  // state and E_start.  40 + 56 instead of 56 + 80 bytes per marker and step.
   bool recompute = false;
   int smem_rc = 0;   // dynamic shared memory of the RC irk = 2 kernel (second field table)
   bool partial_valid = false;  // a fused push has already deposited into d_partial
@@ -1797,8 +1798,9 @@ int pic1dp_gpu_solve_field(pic1dp_gpu_t *h) {
   return solve_field_impl(h, false);
 }
 
-// recompute: the RC kernel pair of step() (h->recompute).  Its irk = 1 leaves the midpoint set's x and v unwritten, so
-// it must be followed by the RC irk = 2 before anything reads the markers; the public per-substep push stores them.
+// recompute: the RC kernel pair of step() (h->recompute).  Its irk = 1 leaves the midpoint set's x and v unwritten and
+// its w buffer holding p - w' (nonlinear delta-f) or unwritten, so it must be followed by the RC irk = 2 before anything
+// reads the markers; the public per-substep push stores the midpoint.
 static int push_impl(pic1dp_gpu_t *h, int32_t irk, bool recompute) {
   int rc = check_loaded(h, "push");
   if (rc) return rc;
