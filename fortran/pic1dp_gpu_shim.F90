@@ -218,6 +218,12 @@ interface
     type(c_ptr), value :: handle
     real(c_double), intent(out) :: electric(*), chargeden(*), mode_re(*), mode_im(*)
   end function
+  integer(c_int) function pic1dp_gpu_set_modes(handle, nmode, modes) bind(c, name = 'pic1dp_gpu_set_modes')
+    import :: c_ptr, c_int, c_int32_t
+    type(c_ptr), value :: handle
+    integer(c_int32_t), value :: nmode
+    integer(c_int32_t), intent(in) :: modes(*)
+  end function
   integer(c_int) function pic1dp_gpu_set_field(handle, electric, chargeden) bind(c, name = 'pic1dp_gpu_set_field')
     import :: c_ptr, c_int
     type(c_ptr), value :: handle
@@ -294,7 +300,7 @@ public :: pic1dp_gpu_comm_unique_id, pic1dp_gpu_comm_init
 public :: pic1dp_gpu_set_markers, pic1dp_gpu_load_markers, pic1dp_gpu_load_markers_maxwellian
 public :: pic1dp_gpu_get_markers, pic1dp_gpu_compute_shape_x
 public :: pic1dp_gpu_collect_charge, pic1dp_gpu_solve_field, pic1dp_gpu_push
-public :: pic1dp_gpu_get_field, pic1dp_gpu_set_field, pic1dp_gpu_sync
+public :: pic1dp_gpu_get_field, pic1dp_gpu_set_field, pic1dp_gpu_set_modes, pic1dp_gpu_sync
 public :: pic1dp_gpu_p2p_export, pic1dp_gpu_p2p_import, pic1dp_gpu_output_field, pic1dp_gpu_output_ptcldist
 public :: pic1dp_gpu_compute_dist_pertb_abs_v, pic1dp_gpu_particle_merge, pic1dp_gpu_particle_remove
 public :: pic1dp_gpu_particle_split
@@ -333,8 +339,9 @@ integer :: imode
 
 call pic1dp_gpu_params_default(p)
 p%nx = input_nx
-p%nmode = input_nmode
-do imode = 0, input_nmode - 1
+! params holds up to PIC1DP_MAX_MODES kept modes; a longer input_modes list is installed with set_modes below
+p%nmode = min(input_nmode, PIC1DP_MAX_MODES)
+do imode = 0, p%nmode - 1
   p%modes(imode + 1) = input_modes(imode)
 end do
 p%lx = input_lx
@@ -357,6 +364,12 @@ p%nranks = global_npe
 
 global_ierr = pic1dp_gpu_create(p, gpu_handle)
 CHKERRQ(global_ierr)
+if (input_nmode > PIC1DP_MAX_MODES) then
+  ! field_init builds the operators for any input_nmode (src/pic1dp_field.F90:158-210)
+  global_ierr = pic1dp_gpu_set_modes(gpu_handle, int(input_nmode, c_int32_t), &
+                                     int(input_modes(0 : input_nmode - 1), c_int32_t))
+  CHKERRQ(global_ierr)
+end if
 
 if (global_npe > 1) then
   ! replaces MPI_COMM_WORLD for the density all-reduce (src/pic1dp_interaction.F90:132-133)

@@ -19,6 +19,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <condition_variable>
 #include <mutex>
@@ -63,8 +64,7 @@ struct Input {
   int input_nspecies = 1;
   double input_species_charge = -1.0, input_species_mass = 1.0, input_species_temperature = 1.0,
          input_species_temperature2 = 1.0, input_species_density = 0.9, input_species_v0 = 5.0;
-  int input_nmode = 1;
-  int input_modes[PIC1DP_MAX_MODES] = {1};
+  std::vector<int> input_modes = {1};   // input_modes(0:input_nmode-1), any count (modes=1,3,5 or modes=1:96)
   int input_init_nmode = 1;
   int input_init_mode[PIC1DP_MAX_MODES] = {1};
   double input_init_mode_cos[PIC1DP_MAX_MODES] = {0.0}, input_init_mode_sin[PIC1DP_MAX_MODES] = {1e-5};
@@ -102,6 +102,30 @@ struct Input {
   double input_tsplit(int i) const { return opt_t0 + i * opt_dt; }                                      // :192
   double input_thshsplit(int i) const { return 1.0 - 0.9 / (input_nsplit > 1 ? input_nsplit : 1) * (double)i; }  // :199
 };
+
+// modes=: comma-separated mode numbers and inclusive ranges a:b, e.g. 1:96 (every mode of nx = 192) or 1,2,10:20
+static bool parse_modes(const std::string &v, std::vector<int> &out) {
+  out.clear();
+  size_t pos = 0;
+  while (pos <= v.size()) {
+    const size_t end = std::min(v.find(',', pos), v.size());
+    const std::string item = v.substr(pos, end - pos);
+    char *e1 = nullptr, *e2 = nullptr;
+    const long a = strtol(item.c_str(), &e1, 10);
+    long b = a;
+    if (e1 == item.c_str()) return false;
+    if (*e1 == ':') {
+      b = strtol(e1 + 1, &e2, 10);
+      if (e2 == e1 + 1 || *e2) return false;
+    } else if (*e1) {
+      return false;
+    }
+    if (b < a || b - a > (1L << 24)) return false;
+    for (long m = a; m <= b; m++) out.push_back((int)m);
+    pos = end + 1;
+  }
+  return !out.empty();
+}
 
 static bool parse(Input &in, int argc, char **argv) {
   for (int i = 1; i < argc; i++) {
@@ -152,6 +176,7 @@ static bool parse(Input &in, int argc, char **argv) {
     else if (k == "markers_out") in.markers_out = v;
     else if (k == "imarker") in.input_imarker = (int)d;
     else if (k == "device_rng") in.device_rng = (int)d;
+    else if (k == "modes") { if (!parse_modes(v, in.input_modes)) return false; }
     else return false;
   }
   return true;
@@ -391,8 +416,9 @@ static void particle_init(Rank &r, const uint8_t *uid) {
   pic1dp_params p;
   pic1dp_gpu_params_default(&p);
   p.nx = in.input_nx;
-  p.nmode = in.input_nmode;
-  for (int m = 0; m < in.input_nmode; m++) p.modes[m] = in.input_modes[m];
+  const int nmode = (int)in.input_modes.size();
+  p.nmode = std::min(nmode, PIC1DP_MAX_MODES);   // params holds up to 64 modes; set_modes below takes any count
+  for (int m = 0; m < p.nmode; m++) p.modes[m] = in.input_modes[m];
   p.lx = in.input_lx;
   p.dt = in.input_dt;
   p.nspecies = 1;
@@ -415,6 +441,10 @@ static void particle_init(Rank &r, const uint8_t *uid) {
   p.fuse = in.fuse;
   r.g.global_ierr = pic1dp_gpu_create(&p, &r.h);
   CHKERRQ(r.g, (pic1dp_gpu_t *)nullptr);
+  if (nmode > PIC1DP_MAX_MODES) {
+    r.g.global_ierr = pic1dp_gpu_set_modes(r.h, nmode, in.input_modes.data());
+    CHKERRQ(r.g, r.h);
+  }
   if (npe > 1) {
     r.g.global_ierr = pic1dp_gpu_comm_init(r.h, uid);
     CHKERRQ(r.g, r.h);
@@ -424,8 +454,8 @@ static void particle_init(Rank &r, const uint8_t *uid) {
   r.particle_isplit = in.input_nsplit > 0 ? 1 : 0;    // :83-87
   r.field_electric.resize(in.input_nx);
   r.field_chargeden.resize(in.input_nx);
-  r.field_mode_re.resize(in.input_nmode);
-  r.field_mode_im.resize(in.input_nmode);
+  r.field_mode_re.resize(nmode);
+  r.field_mode_im.resize(nmode);
 }
 
 // particle_load (src/pic1dp_particle.F90:145-269): the RNG (multirand, a sequential generator) keeps the reference's
@@ -606,12 +636,12 @@ static void put_vec(FILE *f, const std::vector<double> &v) {  // VecView: VEC_FI
 // output_init header (src/pic1dp_output.F90:74-92)
 static void output_init(const pic1dp_input::Input &in, FILE *f) {
   put_i32(f, in.input_nspecies);
-  put_i32(f, in.input_nmode);
+  put_i32(f, (int32_t)in.input_modes.size());
   put_i32(f, in.input_nx);
   put_i32(f, in.input_nv);
   put_i32(f, in.input_nx_opd);
   put_i32(f, in.input_nv_opd);
-  for (int m = 0; m < in.input_nmode; m++) put_i32(f, in.input_modes[m]);
+  for (int m : in.input_modes) put_i32(f, m);
   put_f64(f, in.input_lx);
   put_f64(f, in.input_v_max);
 }

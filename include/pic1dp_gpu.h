@@ -33,7 +33,8 @@ extern "C" {
 
 #define PIC1DP_ABI_VERSION 2
 #define PIC1DP_MAX_SPECIES 4
-#define PIC1DP_MAX_MODES 64
+#define PIC1DP_MAX_MODES 64                             /* kept modes params.modes holds; pic1dp_gpu_set_modes takes more */
+#define PIC1DP_MAX_FIELD_TABLE_BYTES ((int64_t)1 << 32) /* 32 * nx * nmode bytes of field tables at most (set_modes) */
 #define PIC1DP_UNIQUE_ID_BYTES 128
 
 /* error codes */
@@ -408,16 +409,31 @@ int pic1dp_gpu_push(pic1dp_gpu_t *h, int32_t irk);
  */
 int pic1dp_gpu_step(pic1dp_gpu_t *h, int32_t nsteps);
 
-/* field access: field_electric, field_chargeden, field_mode_re, field_mode_im (src/pic1dp_field.F90:27-31);
- * any pointer may be NULL.  get synchronises. */
+/* field access: field_electric, field_chargeden, field_mode_re, field_mode_im (src/pic1dp_field.F90:27-31), the mode
+ * arrays sized by the handle's current nmode (set_modes); any pointer may be NULL.  get synchronises. */
 int pic1dp_gpu_get_field(pic1dp_gpu_t *h, double *electric, double *chargeden, double *mode_re, double *mode_im);
 /* set field_chargeden / field_electric from the host (what field_test does with VecSetValues,
  * src/pic1dp_field.F90:286-297); either may be NULL */
 int pic1dp_gpu_set_field(pic1dp_gpu_t *h, const double *electric, const double *chargeden);
 
-/* the partial-DFT operators built at create (src/pic1dp_field.F90:158-210): F_re, F_im row-major [j*nmode+m],
- * grad_inv[nmode]; any may be NULL */
+/* the partial-DFT operators of the current mode set (src/pic1dp_field.F90:158-210): F_re, F_im row-major
+ * [j*nmode+m], grad_inv[nmode]; any may be NULL */
 int pic1dp_gpu_get_operators(pic1dp_gpu_t *h, double *F_re, double *F_im, double *grad_inv);
+
+/*
+ * set_modes: replaces the kept-mode set that create took from params.nmode / params.modes, i.e. input_nmode and
+ * input_modes(1:input_nmode) (src/pic1dp_input.F90:75-80), with any count: field_init builds the nx x nmode cos / -sin
+ * operators and grad_inv for any input_nmode (src/pic1dp_field.F90:158-210).  Keeping every mode 1 .. nx/2 the grid
+ * resolves is the unfiltered spectral Poisson solve.  The tables are rebuilt on the host with libm by create's code and
+ * expression order (bit-identical to the reference's), the mode buffers are resized (mode_re / mode_im read 0 until the
+ * next solve) and the captured step graph is dropped.  May be called at any time, also between steps; get_field,
+ * get_operators and everything else sized by nmode follow the new set.  Above 64 modes the solve runs multi-CTA kernels
+ * whose sums keep the sequential order: PIC1DP_FIELD_TREE and PIC1DP_FIELD_SEQUENTIAL give the same, bit-identical
+ * results there.  PIC1DP_EINVAL for nmode < 1, a mode number 0 or modes == NULL; PIC1DP_EUNSUPPORTED when
+ * 32 * nx * nmode bytes (F_re, F_im and the column-major copies the solve reads) exceed PIC1DP_MAX_FIELD_TABLE_BYTES.
+ * A refused call leaves the previous mode set in place.
+ */
+int pic1dp_gpu_set_modes(pic1dp_gpu_t *h, int32_t nmode, const int32_t *modes);
 
 /* field energy |E|_2^2 * lx / nx (src/pic1dp_output.F90:120-123), reduced on the device */
 int pic1dp_gpu_field_energy(pic1dp_gpu_t *h, double *energy);

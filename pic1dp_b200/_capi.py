@@ -9,7 +9,8 @@ import ctypes as C
 import os
 
 MAX_SPECIES = 4
-MAX_MODES = 64
+MAX_MODES = 64                     # kept modes Params.modes holds; pic1dp_gpu_set_modes takes any count
+MAX_FIELD_TABLE_BYTES = 1 << 32    # PIC1DP_MAX_FIELD_TABLE_BYTES: 32 * nx * nmode bytes of field tables at most
 UNIQUE_ID_BYTES = 128
 IPC_HANDLE_BYTES = 64
 SUPERKISS64_NSEED = 20635
@@ -100,7 +101,7 @@ EXPORTS = [
     "pic1dp_gpu_load_markers_maxwellian_superkiss64", "pic1dp_gpu_last_gaussian_load",
     "pic1dp_gpu_load_markers_mt19937_64", "pic1dp_gpu_load_markers_maxwellian_mt19937_64",
     "pic1dp_gpu_mt19937_64_uniforms", "pic1dp_host_mt19937_64_jump",
-    "pic1dp_gpu_p2p_trace", "pic1dp_gpu_p2p_trace_read", "pic1dp_gpu_output_all",
+    "pic1dp_gpu_p2p_trace", "pic1dp_gpu_p2p_trace_read", "pic1dp_gpu_output_all", "pic1dp_gpu_set_modes",
 ]
 
 # RNG call-backs of particle_remove / particle_split (pic1dp_real64_fn, pic1dp_gaussian_array_fn)
@@ -152,6 +153,7 @@ def load() -> C.CDLL:
     L.pic1dp_gpu_get_field.argtypes = [vp, dp, dp, dp, dp]
     L.pic1dp_gpu_set_field.argtypes = [vp, dp, dp]
     L.pic1dp_gpu_get_operators.argtypes = [vp, dp, dp, dp]
+    L.pic1dp_gpu_set_modes.argtypes = [vp, i32, C.POINTER(i32)]
     L.pic1dp_gpu_field_energy.argtypes = [vp, dp]
     L.pic1dp_gpu_output_field.argtypes = [vp, dp]
     L.pic1dp_gpu_output_ptcldist.argtypes = [vp, i32, i32, i32, C.c_double, dp, dp, dp, dp, dp, dp]

@@ -85,6 +85,45 @@ __global__ void __launch_bounds__(1024) k_field_solve(const GridArgs g) {
   field_solve_body<SEQ, FINALIZE>(g, smem);
 }
 
+// ---- many-mode field solve (nmode > PIC1DP_FIELD_CTA_MODES): the same arithmetic as k_field_solve<true, *> spread
+// over CTAs.  rho is formed beforehand (k_finalize_rho, or set_field / collect_charge).  Both passes keep the
+// sequential order of the reference's SeqAIJ products, so TREE and SEQUENTIAL coincide here.  One warp per CTA, so a
+// few hundred modes or cells still spread over as many SMs as there are warps.
+constexpr int FIELD_MC_THREADS = 32;
+
+// projection: thread m walks j = 0..nx-1 in order (MatMultTranspose, src/pic1dp_field.F90:231, :236); the warp reads
+// 32 consecutive entries of a table row per j (coalesced), rho[j] is a broadcast
+__global__ void __launch_bounds__(FIELD_MC_THREADS) k_field_project(const GridArgs g) {
+  const int m = blockIdx.x * FIELD_MC_THREADS + threadIdx.x;
+  if (m >= g.nmode) return;
+  const size_t M = (size_t)g.nmode;
+  const double *fr = g.F_re + m, *fi = g.F_im + m, *rho = g.rho;
+  double sim = 0.0, sre = 0.0;
+#pragma unroll 8
+  for (int j = 0; j < g.nx; j++) {
+    const double r = __ldg(rho + j);
+    sim = dadd(sim, dmul(__ldg(fr + j * M), r));
+    sre = dadd(sre, dmul(__ldg(fi + j * M), r));
+  }
+  g.mode_im[m] = dmul(dmul(sim, g.a_im), g.ginv[m]);  // :234, :246
+  g.mode_re[m] = dmul(dmul(sre, g.a_re), g.ginv[m]);  // :239, :243
+}
+
+// synthesis: thread j sums its row left to right (MatMult then MatMultAdd, :251-256) from the column-major copies, so
+// the warp's reads of one column are coalesced; mode_re[m] / mode_im[m] are broadcasts
+__global__ void __launch_bounds__(FIELD_MC_THREADS) k_field_synth(const GridArgs g) {
+  const int j = blockIdx.x * FIELD_MC_THREADS + threadIdx.x;
+  if (j >= g.nx) return;
+  const size_t nx = (size_t)g.nx;
+  const double *fr = g.F_reT + j, *fi = g.F_imT + j;
+  double sum = 0.0;
+#pragma unroll 8
+  for (int m = 0; m < g.nmode; m++) sum = dadd(sum, dmul(__ldg(fr + m * nx), __ldg(g.mode_re + m)));
+#pragma unroll 8
+  for (int m = 0; m < g.nmode; m++) sum = dadd(sum, dmul(__ldg(fi + m * nx), __ldg(g.mode_im + m)));
+  g.E[j] = dmul(sum, 2.0);
+}
+
 // single CTA of 1024 threads
 __global__ void __launch_bounds__(1024) k_field_energy(const GridArgs g) {
   __shared__ double s_part[32];

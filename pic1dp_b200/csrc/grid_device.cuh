@@ -19,6 +19,7 @@ struct GridArgs {
   double *red;            // [nred][nx], nred = matrix_path ? nspecies : 1
   double *rho, *E, *mode_re, *mode_im;
   const double *F_re, *F_im, *ginv;  // [nx*nmode] row-major, [nmode]
+  const double *F_reT, *F_imT;       // [nmode*nx]: column-major copies read by k_field_synth (many-mode path only)
   double a_im, a_re;      // -1.0/nx, 1.0/nx  (src/pic1dp_field.F90:234, :239)
   double nx_over_lx;      // input_nx / input_lx (src/pic1dp_interaction.F90:77)
   double *energy;

@@ -135,13 +135,15 @@ struct pic1dp_gpu {
   double *d_E = nullptr, *d_rho = nullptr, *d_mre = nullptr, *d_mim = nullptr;
   double *d_E_start = nullptr;   // field of step()'s first substep, kept for the recomputed midpoint (ParticleArgs::E_start)
   double *d_Fre = nullptr, *d_Fim = nullptr, *d_ginv = nullptr;
+  double *d_FreT = nullptr, *d_FimT = nullptr;   // column-major copies of the tables (many-mode solve only)
+  std::vector<int32_t> modes;   // the kept-mode set: params.modes at create, replaced by pic1dp_gpu_set_modes
+  bool field_multi = false;     // solve with the many-mode kernels (k_field_project / k_field_synth)
   double *d_partial = nullptr, *d_red = nullptr, *d_energy = nullptr;
   RngScratch rng;
   unsigned long long *d_noob = nullptr;
   unsigned *d_wmax_hi = nullptr;              // [species] running max |deposit source| (high words), DEP_FIXED
   unsigned long long *d_dep_overflow = nullptr, *h_dep_overflow = nullptr;  // conversion overflows (+ pinned mirror)
 
-  std::vector<double> h_Fre, h_Fim, h_ginv;
   // diagnostics scratch (allocated on first use)
   double *d_diag_part = nullptr, *d_diag_sums = nullptr, *d_hist = nullptr, *d_hist_out = nullptr;
   int diag_grid = 0, hist_cells = 0, hist_copies = 16, hist_smem_set = -1;
@@ -379,7 +381,7 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
     }
     if (S.p) cudaFree(S.p);
   }
-  double *bufs[] = {h->d_E, h->d_E_start, h->d_rho, h->d_mre, h->d_mim, h->d_Fre, h->d_Fim, h->d_ginv, h->d_partial, h->d_red, h->d_energy,
+  double *bufs[] = {h->d_E, h->d_E_start, h->d_rho, h->d_mre, h->d_mim, h->d_Fre, h->d_Fim, h->d_ginv, h->d_FreT, h->d_FimT, h->d_partial, h->d_red, h->d_energy,
                     h->d_diag_part, h->d_diag_sums, h->d_hist, h->d_hist_out, h->d_dist_part, h->d_hist_all};
   for (double *b : bufs)
     if (b) cudaFree(b);
@@ -419,6 +421,86 @@ int pic1dp_gpu_destroy(pic1dp_gpu_t *h) {
   return PIC1DP_OK;
 }
 
+// ---- the kept-mode set (input_nmode, input_modes) and its operators: field_init, src/pic1dp_field.F90:158-210 ----
+// The field solve runs the single-CTA k_field_solve up to PIC1DP_FIELD_CTA_MODES kept modes and the many-mode kernels
+// (k_field_project / k_field_synth) above.  PIC1DP_EXP_FIELD=single|multi forces one path (measurement aid; the
+// single CTA needs nx + 2 nmode doubles of shared memory).
+static constexpr int PIC1DP_FIELD_CTA_MODES = 64;
+
+// Builds F_re, F_im and grad_inv for `modes` on the host with libm, in field_init's expression order, and replaces the
+// handle's mode buffers.  On failure the handle keeps its previous mode set.
+static int install_modes(pic1dp_gpu_t *h, int32_t nmode, const int32_t *modes) {
+  const pic1dp_params &p = h->p;
+  const size_t nx = (size_t)p.nx, M = (size_t)nmode, tb = nx * M * 8;
+  if (4 * tb > (size_t)PIC1DP_MAX_FIELD_TABLE_BYTES) {
+    h->err = "nx * nmode = " + std::to_string(nx * M) + ": the field tables (32 bytes per entry) exceed "
+             "PIC1DP_MAX_FIELD_TABLE_BYTES";
+    return PIC1DP_EUNSUPPORTED;
+  }
+  bool multi = nmode > PIC1DP_FIELD_CTA_MODES;
+  if (const char *e = getenv("PIC1DP_EXP_FIELD")) {
+    if (!strcmp(e, "single")) multi = false;
+    if (!strcmp(e, "multi")) multi = true;
+  }
+  const size_t single_smem = (nx + 2 * M) * 8;
+  if (!multi && single_smem > h->max_smem) {
+    h->err = "PIC1DP_EXP_FIELD=single: nx + 2 nmode doubles do not fit in shared memory";
+    return PIC1DP_EUNSUPPORTED;
+  }
+  const double PETSC_PI = 3.14159265358979323846264338327950288419716939937510582;
+  std::vector<double> Fre(nx * M), Fim(nx * M), ginv(M), FreT, FimT;
+  for (size_t m = 0; m < M; m++) ginv[m] = 1.0 / (2.0 * PETSC_PI / p.lx * (double)modes[m]);  // :166
+  for (size_t j = 0; j < nx; j++)
+    for (size_t m = 0; m < M; m++) {
+      const double arg = 2.0 * PETSC_PI / (double)p.nx * (double)modes[m] * (double)j;  // :188, :196
+      Fre[j * M + m] = cos(arg);
+      Fim[j * M + m] = -sin(arg);
+    }
+  if (multi) {
+    FreT.resize(nx * M);
+    FimT.resize(nx * M);
+    for (size_t j = 0; j < nx; j++)
+      for (size_t m = 0; m < M; m++) {
+        FreT[m * nx + j] = Fre[j * M + m];
+        FimT[m * nx + j] = Fim[j * M + m];
+      }
+  }
+  // new buffers: mode_re, mode_im, F_re, F_im, grad_inv, F_re^T, F_im^T
+  double *nb[7] = {};
+  const size_t bytes[7] = {M * 8, M * 8, tb, tb, M * 8, multi ? tb : 0, multi ? tb : 0};
+  const double *src[7] = {nullptr, nullptr, Fre.data(), Fim.data(), ginv.data(), FreT.data(), FimT.data()};
+  cudaError_t e = cudaSuccess;
+  for (int i = 0; i < 7 && e == cudaSuccess; i++) {
+    if (!bytes[i]) continue;
+    e = cudaMalloc(&nb[i], bytes[i]);
+    if (e == cudaSuccess)
+      e = src[i] ? cudaMemcpyAsync(nb[i], src[i], bytes[i], cudaMemcpyHostToDevice, h->stream)
+                 : cudaMemsetAsync(nb[i], 0, bytes[i], h->stream);
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);   // also: no queued kernel reads the old buffers
+  if (e == cudaSuccess && !multi) {
+    const void *ks[4] = {(const void *)k_field_solve<true, true>, (const void *)k_field_solve<false, true>,
+                         (const void *)k_field_solve<true, false>, (const void *)k_field_solve<false, false>};
+    for (int i = 0; i < 4 && e == cudaSuccess; i++)
+      e = cudaFuncSetAttribute(ks[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)single_smem);
+  }
+  if (e != cudaSuccess) {
+    for (double *b : nb)
+      if (b) cudaFree(b);
+    cudaGetLastError();
+    h->err = std::string("field operators for ") + std::to_string(M) + " modes: " + cudaGetErrorString(e);
+    return e == cudaErrorMemoryAllocation ? PIC1DP_ENOMEM : PIC1DP_ECUDA;
+  }
+  double **cur[7] = {&h->d_mre, &h->d_mim, &h->d_Fre, &h->d_Fim, &h->d_ginv, &h->d_FreT, &h->d_FimT};
+  for (int i = 0; i < 7; i++) {
+    if (*cur[i]) cudaFree(*cur[i]);
+    *cur[i] = nb[i];
+  }
+  h->modes.assign(modes, modes + nmode);
+  h->field_multi = multi;
+  return PIC1DP_OK;
+}
+
 static int create_impl(pic1dp_gpu_t *h) {
   const pic1dp_params &p = h->p;
   int ndev = 0;
@@ -443,7 +525,7 @@ static int create_impl(pic1dp_gpu_t *h) {
   CK(cudaEventCreate(&h->ev1));
   for (int i = 0; i < 7; i++) CK(cudaEventCreate(&h->pev[i]));
 
-  const int nx = p.nx, M = p.nmode;
+  const int nx = p.nx;
   const size_t max_smem = prop.sharedMemPerBlockOptin;
   h->max_smem = max_smem;
   // ---- deposit strategy and launch geometry ----
@@ -594,10 +676,6 @@ static int create_impl(pic1dp_gpu_t *h) {
   }
   CK(cudaFuncSetAttribute(pick_deposit(dep, true), cudaFuncAttributeMaxDynamicSharedMemorySize,
                           h->smem_dep > 0 ? h->smem_dep : 8));
-  CK(cudaFuncSetAttribute(k_field_solve<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (nx + 2 * M) * 8));
-  CK(cudaFuncSetAttribute(k_field_solve<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (nx + 2 * M) * 8));
-  CK(cudaFuncSetAttribute(k_field_solve<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (nx + 2 * M) * 8));
-  CK(cudaFuncSetAttribute(k_field_solve<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (nx + 2 * M) * 8));
 
   // ---- markers ----
   const size_t cap = ((size_t)p.capacity + 1) & ~(size_t)1;  // even, for 128-bit accesses
@@ -617,11 +695,6 @@ static int create_impl(pic1dp_gpu_t *h) {
   CK(cudaMalloc(&h->d_E, (size_t)nx * 8));
   CK(cudaMalloc(&h->d_E_start, (size_t)nx * 8));
   CK(cudaMalloc(&h->d_rho, (size_t)nx * 8));
-  CK(cudaMalloc(&h->d_mre, (size_t)M * 8));
-  CK(cudaMalloc(&h->d_mim, (size_t)M * 8));
-  CK(cudaMalloc(&h->d_Fre, (size_t)nx * M * 8));
-  CK(cudaMalloc(&h->d_Fim, (size_t)nx * M * 8));
-  CK(cudaMalloc(&h->d_ginv, (size_t)M * 8));
   CK(cudaMalloc(&h->d_partial, (size_t)p.nspecies * h->grid * nx * 8));
   CK(cudaMalloc(&h->d_red, (size_t)h->nred * nx * 8));
   CK(cudaMalloc(&h->d_energy, 8));
@@ -633,23 +706,7 @@ static int create_impl(pic1dp_gpu_t *h) {
   CK(cudaMallocHost(&h->h_dep_overflow, 8));
   *h->h_dep_overflow = 0;
 
-  // ---- field operators (src/pic1dp_field.F90:158-210), evaluated on the host with libm exactly as written ----
-  const double PETSC_PI = 3.14159265358979323846264338327950288419716939937510582;
-  h->h_Fre.resize((size_t)nx * M);
-  h->h_Fim.resize((size_t)nx * M);
-  h->h_ginv.resize(M);
-  for (int m = 0; m < M; m++) h->h_ginv[m] = 1.0 / (2.0 * PETSC_PI / p.lx * (double)p.modes[m]);  // :166
-  for (int j = 0; j < nx; j++)
-    for (int m = 0; m < M; m++) {
-      const double arg = 2.0 * PETSC_PI / (double)nx * (double)p.modes[m] * (double)j;  // :188, :196
-      h->h_Fre[(size_t)j * M + m] = cos(arg);
-      h->h_Fim[(size_t)j * M + m] = -sin(arg);
-    }
-  CK(cudaMemcpyAsync(h->d_Fre, h->h_Fre.data(), (size_t)nx * M * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(cudaMemcpyAsync(h->d_Fim, h->h_Fim.data(), (size_t)nx * M * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(cudaMemcpyAsync(h->d_ginv, h->h_ginv.data(), (size_t)M * 8, cudaMemcpyHostToDevice, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  return PIC1DP_OK;
+  return install_modes(h, p.nmode, p.modes);   // field operators (src/pic1dp_field.F90:158-210)
 }
 
 int pic1dp_gpu_create(const pic1dp_params *p, pic1dp_gpu_t **out) {
@@ -1589,7 +1646,7 @@ static void fill_grid_args(pic1dp_gpu_t *h, GridArgs &g) {
   const pic1dp_params &p = h->p;
   memset(&g, 0, sizeof(g));
   g.nx = p.nx;
-  g.nmode = p.nmode;
+  g.nmode = (int)h->modes.size();
   g.nspecies = p.nspecies;
   g.ngrids = h->grid;
   g.deltaf = p.deltaf;
@@ -1610,6 +1667,8 @@ static void fill_grid_args(pic1dp_gpu_t *h, GridArgs &g) {
   g.F_re = h->d_Fre;
   g.F_im = h->d_Fim;
   g.ginv = h->d_ginv;
+  g.F_reT = h->d_FreT;
+  g.F_imT = h->d_FimT;
   g.a_im = -1.0 / (double)p.nx;
   g.a_re = 1.0 / (double)p.nx;
   g.nx_over_lx = (double)p.nx / p.lx;
@@ -1783,7 +1842,18 @@ static int solve_field_impl(pic1dp_gpu_t *h, bool finalize_first) {
   CK(cudaSetDevice(h->p.device));
   GridArgs g;
   fill_grid_args(h, g);
-  const int smem = (h->p.nx + 2 * h->p.nmode) * 8;
+  if (h->field_multi) {
+    if (finalize_first) {
+      k_finalize_rho<<<(g.nx + 127) / 128, 128, 0, h->stream>>>(g);
+      CKL(h);
+    }
+    k_field_project<<<(g.nmode + FIELD_MC_THREADS - 1) / FIELD_MC_THREADS, FIELD_MC_THREADS, 0, h->stream>>>(g);
+    CKL(h);
+    k_field_synth<<<(g.nx + FIELD_MC_THREADS - 1) / FIELD_MC_THREADS, FIELD_MC_THREADS, 0, h->stream>>>(g);
+    CKL(h);
+    return PIC1DP_OK;
+  }
+  const int smem = (g.nx + 2 * g.nmode) * 8;
   const bool seq = h->p.field_mode == PIC1DP_FIELD_SEQUENTIAL;
   if (seq && finalize_first) k_field_solve<true, true><<<1, 1024, smem, h->stream>>>(g);
   else if (seq) k_field_solve<true, false><<<1, 1024, smem, h->stream>>>(g);
@@ -2021,7 +2091,7 @@ int pic1dp_gpu_profile_step(pic1dp_gpu_t *h, float ms[6]) {
 int pic1dp_gpu_get_field(pic1dp_gpu_t *h, double *electric, double *chargeden, double *mode_re, double *mode_im) {
   if (!h) return PIC1DP_EINVAL;
   CK(cudaSetDevice(h->p.device));
-  const size_t nb = (size_t)h->p.nx * 8, mb = (size_t)h->p.nmode * 8;
+  const size_t nb = (size_t)h->p.nx * 8, mb = h->modes.size() * 8;
   if (electric) { CK(cudaMemcpyAsync(electric, h->d_E, nb, cudaMemcpyDeviceToHost, h->stream)); h->d2h += nb; }
   if (chargeden) { CK(cudaMemcpyAsync(chargeden, h->d_rho, nb, cudaMemcpyDeviceToHost, h->stream)); h->d2h += nb; }
   if (mode_re) { CK(cudaMemcpyAsync(mode_re, h->d_mre, mb, cudaMemcpyDeviceToHost, h->stream)); h->d2h += mb; }
@@ -2044,10 +2114,26 @@ int pic1dp_gpu_set_field(pic1dp_gpu_t *h, const double *electric, const double *
 int pic1dp_gpu_get_operators(pic1dp_gpu_t *h, double *F_re, double *F_im, double *grad_inv) {
   if (!h) return PIC1DP_EINVAL;
   CK(cudaSetDevice(h->p.device));
-  const size_t fb = (size_t)h->p.nx * h->p.nmode * 8;
+  const size_t fb = (size_t)h->p.nx * h->modes.size() * 8;
   if (F_re) CK(cudaMemcpy(F_re, h->d_Fre, fb, cudaMemcpyDeviceToHost));
   if (F_im) CK(cudaMemcpy(F_im, h->d_Fim, fb, cudaMemcpyDeviceToHost));
-  if (grad_inv) CK(cudaMemcpy(grad_inv, h->d_ginv, (size_t)h->p.nmode * 8, cudaMemcpyDeviceToHost));
+  if (grad_inv) CK(cudaMemcpy(grad_inv, h->d_ginv, h->modes.size() * 8, cudaMemcpyDeviceToHost));
+  return PIC1DP_OK;
+}
+
+int pic1dp_gpu_set_modes(pic1dp_gpu_t *h, int32_t nmode, const int32_t *modes) {
+  if (!h) return PIC1DP_EINVAL;
+  if (nmode < 1) { h->err = "set_modes: nmode must be >= 1"; return PIC1DP_EINVAL; }
+  if (!modes) { h->err = "set_modes: modes is NULL"; return PIC1DP_EINVAL; }
+  for (int m = 0; m < nmode; m++)
+    if (modes[m] == 0) { h->err = "set_modes: mode number 0 has no 1/k"; return PIC1DP_EINVAL; }
+  CK(cudaSetDevice(h->p.device));
+  const int rc = install_modes(h, nmode, modes);
+  if (rc) return rc;
+  if (h->step_graph) {   // the captured solve holds the old tables and mode count
+    cudaGraphExecDestroy(h->step_graph);
+    h->step_graph = nullptr;
+  }
   return PIC1DP_OK;
 }
 

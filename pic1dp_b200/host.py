@@ -79,6 +79,7 @@ class Pic1dGpu:
         if rc:
             self._h = C.c_void_p()
             raise Pic1dpError(rc, "pic1dp_gpu_create", self.L.pic1dp_gpu_last_error(None).decode())
+        self.modes = [params.modes[m] for m in range(params.nmode)]   # the handle's kept-mode set
 
     def _ck(self, rc: int, where: str):
         if rc:
@@ -311,8 +312,16 @@ class Pic1dGpu:
         self._ck(self.L.pic1dp_gpu_step(self._h, nsteps), "step")
 
     # ---- fields ----
+    def set_modes(self, modes):
+        """Replace the kept-mode set (input_modes(1:input_nmode), any count, e.g. range(1, nx // 2 + 1) for the
+        unfiltered solve): rebuilds the field operators; takes effect from the next solve."""
+        ms = [int(m) for m in modes]
+        arr = (C.c_int32 * len(ms))(*ms) if ms else None
+        self._ck(self.L.pic1dp_gpu_set_modes(self._h, len(ms), arr), "set_modes")
+        self.modes = ms
+
     def get_field(self):
-        nx, M = self.params.nx, self.params.nmode
+        nx, M = self.params.nx, len(self.modes)
         E, rho, mre, mim = np.empty(nx), np.empty(nx), np.empty(M), np.empty(M)
         self._ck(self.L.pic1dp_gpu_get_field(self._h, _dp(E), _dp(rho), _dp(mre), _dp(mim)), "get_field")
         return dict(electric=E, chargeden=rho, mode_re=mre, mode_im=mim)
@@ -327,7 +336,7 @@ class Pic1dGpu:
         self._ck(self.L.pic1dp_gpu_set_field(self._h, _dp(e), _dp(r)), "set_field")
 
     def get_operators(self):
-        nx, M = self.params.nx, self.params.nmode
+        nx, M = self.params.nx, len(self.modes)
         Fre, Fim, g = np.empty(nx * M), np.empty(nx * M), np.empty(M)
         self._ck(self.L.pic1dp_gpu_get_operators(self._h, _dp(Fre), _dp(Fim), _dp(g)), "get_operators")
         return Fre.reshape(nx, M), Fim.reshape(nx, M), g

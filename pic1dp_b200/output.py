@@ -25,7 +25,7 @@ class OutputWriter:
         self.nx_opd, self.nv_opd, self.v_max = nx_opd, nv_opd, float(v_max)
         self.f = open(path, "wb")
         p = self.p
-        ints = [p.nspecies, p.nmode, p.nx, nv, nx_opd, nv_opd] + [p.modes[m] for m in range(p.nmode)]
+        ints = [p.nspecies, len(gpu.modes), p.nx, nv, nx_opd, nv_opd] + list(gpu.modes)   # the handle's kept modes
         np.asarray(ints, dtype=">i4").tofile(self.f)
         np.asarray([p.lx, self.v_max], dtype=">f8").tofile(self.f)
 
